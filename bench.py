@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ELBO forward+backward throughput of the gridded variational GP hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (BASELINE.json configs[4], the configuration the metric is quoted on; it fits one GPU): 2-D
@@ -25,6 +25,7 @@ import tempfile
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -337,6 +338,22 @@ def tensor_roofline(vg, plan, device, reps=20):
                     "instruction is the warp-level DMMA"}
 
 
+DUMP_NAMES = ("out", "dtheta", "dm", "dL")       # what plan.step returns; out = [ELBO, scaled log-likelihood, KL, n]
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, tensors):
+    """Write the arrays of one step as <path>/<name>.npy (float64), so that two builds can be compared output for output:
+    the data and the parameters are functions of the arguments alone (make_tracks, make_params)."""
+    arrays = {name: t.numpy() for name, t in zip(DUMP_NAMES, tensors)}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def measured_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     try:
@@ -485,7 +502,14 @@ def main():
     ap.add_argument("--spatial-reshard", action="store_true",
                     help="multi-GPU: exchange the acquisition-order shards by grid-cell range at setup "
                          "(dist.spatial_reshard; measured slower at 8 x B200 in round 1, off by default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (ELBO terms, dtheta, dm, dL) "
+                         "as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -633,6 +657,7 @@ def main():
         out = step(i)
     t_end.record()
     barrier()
+    dumped = [t.cpu() for t in out] if (args.dump_outputs and rank == 0) else None
     launches = lib.vggp_launch_count() - launches0
     if plan.peer_allreduce_failed():
         raise SystemExit("a barrier of the peer-memory all-reduce timed out (a rank went missing)")
@@ -809,6 +834,8 @@ def main():
             line["e2e"] = e2e
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"] = time_cpu_baseline(workload=args.workload)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

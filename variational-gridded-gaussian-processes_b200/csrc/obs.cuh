@@ -748,7 +748,8 @@ struct B0Args {
     const double* P[D];
     const double* Q[D];
     T* galpha;
-    T* gfac;                 // per dim [bP (n_d^2) | bQ (n_d^2)]
+    double* gfac;            // per dim [bP (n_d^2) | bQ (n_d^2)], float64 whatever T: the gbuf block itself for float64
+                             // observations, a plan-owned buffer rounded once into the gbuf for float32 ones
     i64 gfac_off[D];
     double* gs;              // [E, n, -, G_l[0..1], G_s[0..1]]
 };
@@ -931,14 +932,16 @@ __global__ void __launch_bounds__(256) k_obs_b0(const __grid_constant__ B0Args<T
             accGl[d] += gl;
             accGs[d] += gsv;
             const int nn = a.nd[d];
-            T* gP = a.gfac + a.gfac_off[d];
-            T* gQ = gP + (i64)nn * nn;
+            // float64 sums: the l / s2 gradients go through P bP P and Q bQ Q, which amplify a relative error of bQ by about four
+            // orders of magnitude; float32 atomics over the tiles put the 1-D s2 gradient ~ 1 % off the oracle, varying with their order
+            double* gP = a.gfac + a.gfac_off[d];
+            double* gQ = gP + (i64)nn * nn;
             for (int e = tid; e < nn * nn; e += blockDim.x) {
                 const int i = e / nn, j = e % nn;
-                T vp = (T)0, vq = (T)0;
+                double vp = 0.0, vq = 0.0;
 #pragma unroll
                 for (int t = 0; t < B0_TN; ++t) {
-                    const T ff = phi[(size_t)(off[d] + i) * B0_TN + t] * phi[(size_t)(off[d] + j) * B0_TN + t];
+                    const double ff = (double)phi[(size_t)(off[d] + i) * B0_TN + t] * phi[(size_t)(off[d] + j) * B0_TN + t];
                     vp += s_op[d][t] * ff;
                     vq += s_oq[d][t] * ff;
                 }

@@ -95,6 +95,7 @@ struct vggp_plan {
     int band_off[VGGP_MAX_D], band_total, knot_off[VGGP_MAX_D], knot_total;
     int tab_off[VGGP_MAX_D], tab_total;
     i64 gfac_off[VGGP_MAX_D], gfac_total;   // B0 family: full factor-gradient blocks [bP | bQ] per dim
+    double* gfac_f64 = nullptr;            // dense-feature families, float32 observations: [bP | bQ] of k_obs_b0 in float64
     unsigned char* tables;                 // [band tables (obs dtype) | pad16 | knots (float32) | pad16]
     int table_bytes, knots_byte_off;
     int sm_count, obs_blocks_per_sm;
@@ -1026,19 +1027,25 @@ int launch_obs_b0(vggp_plan* p, const void* const* x, const void* y, i64 n, void
     a.alpha = reinterpret_cast<const T*>(p->alphaT);
     T* gb = reinterpret_cast<T*>(gbuf);
     a.galpha = gb;
-    a.gfac = gb + p->M;
+    constexpr bool f32 = sizeof(T) == 4;
+    a.gfac = f32 ? p->gfac_f64 : reinterpret_cast<double*>(gb + p->M);
     i64 n_elems, soff, nsc, total;
     vggp_gbuf_layout(p, &n_elems, &soff, &nsc, &total);
     a.gs = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(gbuf) + soff);
     const size_t smem = (size_t)5 * ntot * B0_TN * sizeof(T);
     if (smem > 200 * 1024) return fail(VGGP_E_UNSUPPORTED, "B0 feature tiles do not fit in shared memory");
     if (int rc = raise_dyn_smem(k_obs_b0<T, D>, smem)) return rc;
+    if (f32) VGGP_CUDA(cudaMemsetAsync(p->gfac_f64, 0, sizeof(double) * p->gfac_total, st));
     const i64 tiles = (n + B0_TN - 1) / B0_TN;
     const int blocks = (int)std::min<i64>(tiles, (i64)p->sm_count * 2);
     k1_mark(p, 0, st);
     k_obs_b0<T, D><<<blocks, 256, smem, st>>>(a);
     k1_mark(p, 1, st);
     VGGP_LAUNCH_CHECK();
+    if (f32) {      // the caller cleared the gbuf (vggp_obs_fwd_bwd): the float64 sums replace its [bP | bQ] blocks
+        k_b0s_from_double<T><<<ceil_div(p->gfac_total, 256), 256, 0, st>>>(p->gfac_f64, gb + p->M, p->gfac_total);
+        VGGP_LAUNCH_CHECK();
+    }
     return 0;
 }
 
@@ -2100,6 +2107,8 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
         unsigned char* br = nullptr;
         TRY(dev_alloc(p, &br, (i64)BAND_REPLICAS * p->band_total * (i64)tsz));
         p->band_rep = br;
+    } else if (obs_dtype == VGGP_F32) {
+        TRY(dev_alloc(p, &p->gfac_f64, p->gfac_total));
     }
     TRY(dev_alloc(p, &p->theta_dev, 2 * VGGP_MAX_D + 1));
     TRY(dev_alloc(p, &p->obs_counter, 4));
