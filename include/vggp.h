@@ -57,6 +57,12 @@ extern "C" {
                              * per dimension M + 1 cosines and M sines of w_k = 2 pi k / (b - a) on the domain [a, b), exp(-r / l) outside,
                              * Kuu_d = diag(alpha) + beta beta^T.  The mesh of a dimension has 2 M + 1 knots spanning [a, b]: only its end
                              * points and its size are used (M_d = n_knots[d], odd).  Dense-feature kernel, D <= 2. */
+#define VGGP_SVGP_MARKOV 4  /* the model of VGGP_SVGP_GRID (same knots-as-Z, theta layout and ELBO) in its O(1)-per-observation Markov
+                             * form: K_d^-1 is tridiagonal and psi_d = K_d^-1 k_d(Z, x) has two non-zeros per dimension, so the
+                             * per-observation kernel streams the binned layout (extended cells: observations outside the points
+                             * contribute) and the grid side is O(M + sum M_d^2) elementwise work.  D = 1..3, Z fixed.  Takes the binned
+                             * layout only: vggp_obs_fwd_bwd, vggp_obs_fwd_bwd_packed and vggp_elbo_host return VGGP_E_UNSUPPORTED, as do
+                             * vggp_set_deterministic(plan, 1) and vggp_workspace_ptr; vggp_features_dense returns the dense k_d(Z, x). */
 
 /* observation dtype */
 #define VGGP_F32 0
@@ -81,7 +87,7 @@ uint64_t vggp_launch_count(void);
 
 /*
  * Plan = grid descriptor + workspace, one per (model, device).
- *   family      VGGP_B1_ASVGP | VGGP_B0_GRIDDED | VGGP_SVGP_GRID | VGGP_VFF_GRID
+ *   family      VGGP_B1_ASVGP | VGGP_B0_GRIDDED | VGGP_SVGP_GRID | VGGP_VFF_GRID | VGGP_SVGP_MARKOV
  *   D           number of input dimensions, 1..VGGP_MAX_D
  *   n_knots     [D] number of knots of each per-dimension mesh (B1: M_d = n_knots, B0: M_d = n_knots-1)
  *   knots_host  [D] host pointers to the float32 knot arrays, exactly as the reference builds them
@@ -109,6 +115,9 @@ int vggp_plan_dims(const vggp_plan* plan, int* D, int* m_per_dim /*[D]*/, int64_
  *     [ n_obs_elems values of obs_dtype | pad to 8 bytes | n_scalars float64 ]
  *   n_obs_elems = M (d alpha) + per-dimension band / factor-gradient blocks
  *   scalars     = { sum_n (r_n^2 - prod p + prod q), n_local, n_inside, reserved... }
+ *   VGGP_SVGP_MARKOV: n_obs_elems = M (d m corner sums) + the band block [bp_d | bp_o | bq_d | bq_o] of every dimension (sums of
+ *   prod_{e != d} p_e resp. q_e times wlo^2, wlo whi, whi^2 per node / node pair); scalars 3 + d hold
+ *   sum_n d/dl_d [(y - mu)^2 + var] through the weights (bands held fixed).
  * `scalar_offset_bytes` is the byte offset of the float64 block, `total_bytes` the size to allocate.
  */
 int vggp_gbuf_layout(const vggp_plan* plan, int64_t* n_obs_elems, int64_t* scalar_offset_bytes,
@@ -167,6 +176,8 @@ int vggp_obs_fwd_bwd(vggp_plan* plan, const void* const* x, const void* y, int64
  *   vggp_obs_bin_pack      fills `binned` (desc->bytes) from x[D], y; synchronises, frees the temporaries.
  *   vggp_obs_fwd_bwd_binned  the fused forward+backward over a binned buffer (asynchronous, allocation-free);
  *                          gbuf is zeroed by the call, exactly as vggp_obs_fwd_bwd_packed.
+ * VGGP_SVGP_MARKOV (D = 1..3): the same three calls with extended cells as for the B0 family below; the per-observation kernel is
+ * k_obs_svgpm_binned (csrc/svgpm.cuh).  This is the only observation path of that family.
  * B0 family (D <= 2): the same three calls select the SCAN form of the cell-integrated features (csrc/b0scan.cuh,
  * DESIGN.md section 4): cells are extended by one virtual cell on each side (observations outside the mesh do
  * contribute in this family, n_inside == n), the per-observation kernel does O(1) work against per-cell tables built by
@@ -295,6 +306,7 @@ int vggp_features_dense(const vggp_plan* plan, int dim, const void* x, int64_t n
  *   mean = <kron_d phi_d(x*), alpha>,   var = prod_d s2_d - prod_d phi_d^T P_d phi_d + prod_d phi_d^T Q_d phi_d.
  *   x [D] HOST array of device pointers (n values of obs_dtype each); mean, var: n values of obs_dtype.
  * B1 family: test points outside the mesh get mean 0 and the prior variance (their feature column is zero).
+ * VGGP_SVGP_MARKOV: two weights per dimension against the per-cell tables of the last forward, O(1) per point.
  * B0 family (D <= 2): the cell-integrated features are non-zero everywhere; they are evaluated in their scan form
  *   (three local features per dimension against per-cell tables built by first-order recurrences on the grid side,
  *   csrc/b0scan.cuh),
@@ -309,7 +321,7 @@ int vggp_predict(vggp_plan* plan, const void* const* x, int64_t n, void* mean, v
  * from which MSE = out0/n, MAE = out1/n, RMSE = sqrt(MSE), R^2 = 1 - out0 / (out3 - out2^2/n).
  *   vggp_metrics          truth, pred: n values of `dtype` (VGGP_F32 | VGGP_F64) each
  *   vggp_predict_metrics  the same sums for pred = posterior mean at the test points x[D] (state of the last
- *                         vggp_grid_forward, B1 family), without writing the predictions to memory
+ *                         vggp_grid_forward, B1 and VGGP_SVGP_MARKOV families), without writing the predictions to memory
  */
 int vggp_metrics(int dtype, const void* truth, const void* pred, int64_t n, double* out, void* stream);
 int vggp_predict_metrics(vggp_plan* plan, const void* const* x, const void* y, int64_t n, double* out, void* stream);

@@ -17,3 +17,4 @@ B1_ASVGP = _lib.B1_ASVGP
 B0_GRIDDED = _lib.B0_GRIDDED
 SVGP_GRID = _lib.SVGP_GRID
 VFF_GRID = _lib.VFF_GRID
+SVGP_MARKOV = _lib.SVGP_MARKOV

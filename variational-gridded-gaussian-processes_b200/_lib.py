@@ -6,7 +6,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libvggp.so")
 
-B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID = 0, 1, 2, 3
+B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID, SVGP_MARKOV = 0, 1, 2, 3, 4
 F32, F64 = 0, 1
 ABI_VERSION = 1
 

@@ -16,6 +16,7 @@
 #include "obs_binned.cuh"
 #include "metrics.cuh"
 #include "b0scan.cuh"
+#include "svgpm.cuh"
 #include "collective.cuh"
 
 // Every plan-taking entry point runs with the plan's device current and restores the caller's device on return
@@ -126,6 +127,10 @@ struct vggp_plan {
     bool k1_timing = false; std::vector<cudaEvent_t> k1_ev; int k1_count = 0;
     cudaEvent_t k1_gev[2] = {nullptr, nullptr};      // the pair recorded by event nodes of a captured graph (vggp_k1_graph_time_read)
     bool k1_gev_captured = false;
+    // product-grid SVGP, Markov form (svgpm.cuh): per-cell tables (obs dtype), float64 bands per dimension, scalars
+    void* svm_tab = nullptr; int svm_tab_off[VGGP_MAX_D] = {0, 0, 0};
+    double* svm_W[VGGP_MAX_D] = {}; double* svm_sc = nullptr;
+    int svm_blocks_per_sm = 0;
     double* b1_acc = nullptr; int b1_acc_total = 0;      // structured == 3: band accumulators of dK_d, [3][n_d] per dimension
     cudaStream_t last_stream = nullptr;                  // stream of the last grid forward (on-demand workspace fills)
     // deterministic mode (vggp_set_deterministic): run records + sort scratch of the per-observation kernel, per-CTA partials
@@ -1137,7 +1142,9 @@ int pack_dispatch(vggp_plan* p, const void* const* x, const void* y, i64 n, int 
 template <typename T, int D>
 int bin_prepare_impl(vggp_plan* p, const void* const* x, i64 n, int run_cap, vggp_binned_desc* desc, cudaStream_t st) {
     i64 ncells = 1;
-    for (int d = 0; d < D; ++d) ncells *= (p->family == VGGP_B0_GRIDDED ? p->K[d] + 1 : p->K[d] - 1);
+    // B0 and Markov-SVGP families: extended cells (observations outside the mesh contribute)
+    const bool ext = p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV;
+    for (int d = 0; d < D; ++d) ncells *= (ext ? p->K[d] + 1 : p->K[d] - 1);
     if (ncells >= ((i64)1 << 32) - 1) return fail(VGGP_E_UNSUPPORTED, "too many cells for 32-bit keys");
     std::vector<uint32_t> count((size_t)ncells + 1, 0u);
     if (n > 0) {
@@ -1157,13 +1164,11 @@ int bin_prepare_impl(vggp_plan* p, const void* const* x, i64 n, int run_cap, vgg
         VGGP_CUDA(tmp.alloc(&d_count, sizeof(uint32_t) * (ncells + 1)));
         VGGP_CUDA(cudaMemsetAsync(d_count, 0, sizeof(uint32_t) * (ncells + 1), st));
         const int blocks = (int)std::min<i64>((n + 255) / 256, 148 * 16);
-        if (p->family == VGGP_B0_GRIDDED) {       // extended cells: every observation has one (b0scan.cuh)
-            if constexpr (D <= 2) {
-                B0sKeyArgs<T, D> kb;
-                kb.n = n;
-                for (int d = 0; d < D; ++d) { kb.x[d] = ka.x[d]; kb.mesh[d] = p->mesh[d]; }
-                k_b0s_keys<T, D><<<blocks, 256, 0, st>>>(kb, keys_in, idx_in);
-            }
+        if (ext) {       // extended cells: every observation has one (b0scan.cuh)
+            B0sKeyArgs<T, D> kb;
+            kb.n = n;
+            for (int d = 0; d < D; ++d) { kb.x[d] = ka.x[d]; kb.mesh[d] = p->mesh[d]; }
+            k_b0s_keys<T, D><<<blocks, 256, 0, st>>>(kb, keys_in, idx_in);
         } else {
             k_cell_keys<T, D><<<blocks, 256, 0, st>>>(ka, (uint32_t)ncells, keys_in, idx_in);
         }
@@ -1207,22 +1212,20 @@ int bin_pack_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* const*
         VGGP_CUDA(cudaMemcpyAsync(buf + desc->off_run_n, L.run_n.data(), sizeof(int32_t) * 32 * L.n_tasks, cudaMemcpyHostToDevice, st));
         VGGP_CUDA(cudaMemcpyAsync(buf + desc->off_run_start, L.run_start.data(), sizeof(uint32_t) * 32 * L.n_tasks, cudaMemcpyHostToDevice, st));
         const int blocks = (int)std::min<i64>(L.n_tasks, (i64)p->sm_count * 8);
-        if (p->family == VGGP_B0_GRIDDED) {
-            if constexpr (D <= 2) {
-                B0sGatherArgs<T, D> gb0;
-                for (int d = 0; d < D; ++d) {
-                    gb0.x[d] = reinterpret_cast<const T*>(x[d]);
-                    gb0.knots[d] = p->d_knots[d];
-                    gb0.K[d] = p->K[d];
-                }
-                gb0.y = reinterpret_cast<const T*>(y);
-                gb0.perm = p->bin_perm;
-                gb0.buf = buf;
-                gb0.off_task_off = desc->off_task_off; gb0.off_task_R = desc->off_task_R; gb0.off_run_cell = desc->off_run_cell;
-                gb0.off_run_n = desc->off_run_n; gb0.off_run_start = desc->off_run_start; gb0.off_data = desc->off_data;
-                gb0.n_tasks = (int)L.n_tasks;
-                k_b0s_gather<T, D><<<blocks, 256, 0, st>>>(gb0);
+        if (p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV) {
+            B0sGatherArgs<T, D> gb0;
+            for (int d = 0; d < D; ++d) {
+                gb0.x[d] = reinterpret_cast<const T*>(x[d]);
+                gb0.knots[d] = p->d_knots[d];
+                gb0.K[d] = p->K[d];
             }
+            gb0.y = reinterpret_cast<const T*>(y);
+            gb0.perm = p->bin_perm;
+            gb0.buf = buf;
+            gb0.off_task_off = desc->off_task_off; gb0.off_task_R = desc->off_task_R; gb0.off_run_cell = desc->off_run_cell;
+            gb0.off_run_n = desc->off_run_n; gb0.off_run_start = desc->off_run_start; gb0.off_data = desc->off_data;
+            gb0.n_tasks = (int)L.n_tasks;
+            k_b0s_gather<T, D><<<blocks, 256, 0, st>>>(gb0);
         } else {
             BinGatherArgs<T, D> ga;
             for (int d = 0; d < D; ++d) {
@@ -1921,6 +1924,165 @@ int launch_tracks(void* const* x, void* y, i64 lo, i64 hi, i64 n_total, i64 seed
     return 0;
 }
 
+// ---- product-grid SVGP, Markov form (svgpm.cuh) -------------------------------------------------------------
+template <int D>
+SvgpmGeom<D> svgpm_geom(const vggp_plan* p) {
+    SvgpmGeom<D> g;
+    for (int d = 0; d < D; ++d) {
+        g.M[d] = p->n[d];
+        g.stride[d] = (int)p->stride[d];
+        g.band_off[d] = p->band_off[d];
+        g.tab_off[d] = p->svm_tab_off[d];
+    }
+    return g;
+}
+
+SvgpmBwd svgpm_bwd(const vggp_plan* p) {
+    SvgpmBwd g;
+    memset(&g, 0, sizeof(g));
+    g.D = p->D;
+    g.Mtot = p->M;
+    for (int d = 0; d < p->D; ++d) {
+        g.M[d] = p->n[d];
+        g.stride[d] = (int)p->stride[d];
+        g.band_off[d] = p->band_off[d];
+        g.Loff[d] = p->g.Loff[d];
+        g.W[d] = p->svm_W[d];
+    }
+    g.sc = p->svm_sc;
+    return g;
+}
+
+// K_d band and K_d^-1 band in closed form, S_d band from tril(L_d), per-cell tables, log-dets and traces, m in the
+// observation dtype.  Four launches, no allocation, no synchronisation.
+int svgpm_forward(vggp_plan* p, const double* theta, const double* m, const double* L, cudaStream_t st) {
+    const int D = p->D;
+    VGGP_CUDA(cudaMemsetAsync(p->svm_sc, 0, sizeof(double) * SVS_MKM, st));
+    VGGP_CUDA(cudaMemsetAsync(p->g.info, 0, sizeof(int), st));
+    VGGP_CUDA(cudaMemcpyAsync(p->theta_dev, theta, sizeof(double) * (2 * D + 1), cudaMemcpyDeviceToDevice, st));
+    SvgpmGrid g;
+    memset(&g, 0, sizeof(g));
+    g.D = D;
+    for (int d = 0; d < D; ++d) {
+        g.M[d] = p->n[d];
+        g.z[d] = p->d_knots[d];
+        g.Loff[d] = p->g.Loff[d];
+        g.W[d] = p->svm_W[d];
+        g.tab_off[d] = p->svm_tab_off[d];
+    }
+    g.tab = p->svm_tab;
+    g.sc = p->svm_sc;
+    g.info = p->g.info;
+    const dim3 grid(ceil_div(p->nmax, 8), D);
+    const int cblocks = (int)std::min<i64>((p->M + 255) / 256, 148 * 4);
+    if (p->obs_dtype == VGGP_F32) {
+        k_svgpm_fwd<float><<<grid, 256, 0, st>>>(g, theta, L);
+        VGGP_LAUNCH_CHECK();
+        k_b0s_from_double<float><<<cblocks, 256, 0, st>>>(m, reinterpret_cast<float*>(p->alphaT), p->M);
+    } else {
+        k_svgpm_fwd<double><<<grid, 256, 0, st>>>(g, theta, L);
+        VGGP_LAUNCH_CHECK();
+        k_b0s_from_double<double><<<cblocks, 256, 0, st>>>(m, reinterpret_cast<double*>(p->alphaT), p->M);
+    }
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+
+template <typename T, int D>
+int svgpm_backward_impl(vggp_plan* p, const double* theta, const double* m, const double* L, const void* gbuf,
+                        double ell_scale, double* out, double* dtheta, double* dm, double* dL, cudaStream_t st) {
+    i64 n_elems, soff, nsc, total;
+    vggp_gbuf_layout(p, &n_elems, &soff, &nsc, &total);
+    const double* gs = reinterpret_cast<const double*>(reinterpret_cast<const unsigned char*>(gbuf) + soff);
+    const T* gm = reinterpret_cast<const T*>(gbuf);
+    const T* gband = gm + p->M;
+    const SvgpmBwd g = svgpm_bwd(p);
+    VGGP_CUDA(cudaMemsetAsync(p->svm_sc + SVS_MKM, 0, sizeof(double) * (SVS_COUNT - SVS_MKM), st));
+    const int mblocks = (int)std::min<i64>((p->M + 255) / 256, (i64)p->sm_count * 4);
+    k_svgpm_dm<T, D><<<mblocks, 256, 0, st>>>(g, gm, m, theta, ell_scale, dm);
+    VGGP_LAUNCH_CHECK();
+    k_svgpm_dL<T><<<dim3(ceil_div((i64)p->nmax * p->nmax, 256), D), 256, 0, st>>>(g, gband, L, theta, ell_scale, dL);
+    VGGP_LAUNCH_CHECK();
+    k_svgpm_theta<T><<<1, 256, 0, st>>>(g, gband, gs, theta, ell_scale, out, dtheta);
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+int svgpm_backward(vggp_plan* p, const double* theta, const double* m, const double* L, const void* gbuf, double ell_scale,
+                   double* out, double* dtheta, double* dm, double* dL, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, svgpm_backward_impl, p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
+}
+
+template <typename T, int D>
+int launch_obs_svgpm(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, void* gbuf, cudaStream_t st) {
+    if (p->svm_blocks_per_sm == 0) {
+        int nb = 0;
+        VGGP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_obs_svgpm_binned<T, D>, BIN_THREADS, 0));
+        p->svm_blocks_per_sm = nb < 1 ? 1 : nb;
+    }
+    SvgpmArgs<T, D> a;
+    memset(&a, 0, sizeof(a));
+    a.bin.buf = reinterpret_cast<const unsigned char*>(binned);
+    a.bin.off_task_off = desc->off_task_off; a.bin.off_task_R = desc->off_task_R; a.bin.off_run_cell = desc->off_run_cell;
+    a.bin.off_run_n = desc->off_run_n; a.bin.off_data = desc->off_data;
+    a.bin.n_tasks = (int)desc->n_tasks;
+    T* gb = reinterpret_cast<T*>(gbuf);
+    a.bin.galpha = gb;
+    a.bin.gband = reinterpret_cast<T*>(p->band_rep);
+    a.bin.n_rep = BAND_REPLICAS;
+    a.bin.band_rep_stride = p->band_total;
+    i64 n_elems, soff, nsc, total;
+    vggp_gbuf_layout(p, &n_elems, &soff, &nsc, &total);
+    a.bin.gs = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(gbuf) + soff);
+    a.bin.n_real = (double)desc->n;
+    a.bin.counter = p->obs_counter + 1;          // reset by k_band_reduce after every launch
+    a.geo = svgpm_geom<D>(p);
+    a.tab = reinterpret_cast<const T*>(p->svm_tab);
+    a.m = reinterpret_cast<const T*>(p->alphaT);
+    a.theta = p->theta_dev;
+    i64 blocks = (desc->n_tasks + BIN_WARPS - 1) / BIN_WARPS;
+    blocks = std::max<i64>(1, std::min<i64>(blocks, (i64)p->sm_count * p->svm_blocks_per_sm));
+    k1_mark(p, 0, st);
+    k_obs_svgpm_binned<T, D><<<(unsigned)blocks, BIN_THREADS, 0, st>>>(a);
+    k1_mark(p, 1, st);
+    VGGP_LAUNCH_CHECK();
+    k_band_reduce<T><<<ceil_div(p->band_total, 16), 256, 0, st>>>(a.bin.gband, BAND_REPLICAS, p->band_total, p->band_total, gb + p->M,
+                                                                  a.bin.counter);
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+int obs_svgpm_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, void* gbuf, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, launch_obs_svgpm, p, desc, binned, gbuf, st);
+}
+
+template <typename T, int D>
+int launch_predict_svgpm(vggp_plan* p, const void* const* x, const void* y, i64 n, void* mean, void* var, double* out,
+                         cudaStream_t st) {
+    SvgpmPredictArgs<T, D> a;
+    memset(&a, 0, sizeof(a));
+    a.geo = svgpm_geom<D>(p);
+    for (int d = 0; d < D; ++d) {
+        a.z[d] = p->d_knots[d];
+        a.x[d] = reinterpret_cast<const T*>(x[d]);
+    }
+    a.y = reinterpret_cast<const T*>(y);
+    a.n = n;
+    a.tab = reinterpret_cast<const T*>(p->svm_tab);
+    a.m = reinterpret_cast<const T*>(p->alphaT);
+    a.theta = p->theta_dev;
+    a.mean = reinterpret_cast<T*>(mean);
+    a.var = reinterpret_cast<T*>(var);
+    a.out = out;
+    const int blocks = (int)std::min<i64>((n + 255) / 256, (i64)p->sm_count * 8);
+    if (out) k_predict_svgpm<T, D, true><<<blocks, 256, 0, st>>>(a);
+    else k_predict_svgpm<T, D, false><<<blocks, 256, 0, st>>>(a);
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+int predict_svgpm_dispatch(vggp_plan* p, const void* const* x, const void* y, i64 n, void* mean, void* var, double* out,
+                           cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, launch_predict_svgpm, p, x, y, n, mean, var, out, st);
+}
+
 extern "C" {
 
 int vggp_abi_version(void) { return VGGP_ABI_VERSION; }
@@ -1971,7 +2133,8 @@ int vggp_set_b1_structured(int on) {
 int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, const float* const* knots_host,
                      int obs_dtype, int device) {
     if (!out || !n_knots || !knots_host) return fail(VGGP_E_ARG, "null argument");
-    if (family != VGGP_B1_ASVGP && family != VGGP_B0_GRIDDED && family != VGGP_SVGP_GRID && family != VGGP_VFF_GRID)
+    if (family != VGGP_B1_ASVGP && family != VGGP_B0_GRIDDED && family != VGGP_SVGP_GRID && family != VGGP_VFF_GRID &&
+        family != VGGP_SVGP_MARKOV)
         return fail(VGGP_E_FAMILY, "unknown feature family");
     if ((family == VGGP_SVGP_GRID || family == VGGP_VFF_GRID) && D > 2)
         return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families are built for D <= 2, as in the reference");
@@ -1996,6 +2159,7 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
     vggp_plan* p = new (std::nothrow) vggp_plan();
     if (!p) return fail(VGGP_E_NOMEM, "out of host memory");
     p->family = family; p->D = D; p->obs_dtype = obs_dtype; p->device = device;
+    const bool markov = family == VGGP_SVGP_MARKOV;     // O(M + sum M_d^2) grid side: no factor arrays, no GEMM schedules
     p->M = 1; p->Lsize = 0; p->nmax = 0;
     int rc = 0;
     GridDims& g = p->g;
@@ -2049,6 +2213,7 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
             const float gf = (knots_host[d][k] - mv.t0) * mv.inv_h;
             if (fabsf(gf - (float)k) > 1.25f) mv.nearly_uniform = 0;
         }
+        if (markov) continue;
         const i64 nn = (i64)p->n[d] * p->n[d];
         TRY(dev_alloc(p, &g.Kraw[d], nn)); TRY(dev_alloc(p, &g.Kc[d], nn)); TRY(dev_alloc(p, &g.W[d], nn));
         TRY(dev_alloc(p, &g.cdiag[d], (i64)NB * NB));
@@ -2067,6 +2232,32 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
     TRY(dev_alloc(p, &g.sc, SC_COUNT));
     TRY(dev_alloc(p, &g.info, 1));
     const size_t tsz = obs_dtype == VGGP_F32 ? 4 : 8;
+    if (markov) {
+        int toff2 = 0;
+        for (int d = 0; d < D; ++d) {
+            p->svm_tab_off[d] = toff2;
+            toff2 += SVM_TAB * (p->n[d] + 1);
+            TRY(dev_alloc(p, &p->svm_W[d], (i64)SVM_W * p->n[d]));
+        }
+        unsigned char* t = nullptr;
+        TRY(dev_alloc(p, &t, (i64)toff2 * (i64)tsz));
+        p->svm_tab = t;
+        TRY(dev_alloc(p, &p->svm_sc, SVS_COUNT));
+        unsigned char* a = nullptr;
+        TRY(dev_alloc(p, &a, p->M * (i64)tsz));
+        p->alphaT = a;
+        unsigned char* br = nullptr;
+        TRY(dev_alloc(p, &br, (i64)BAND_REPLICAS * p->band_total * (i64)tsz));
+        p->band_rep = br;
+        TRY(dev_alloc(p, &p->theta_dev, 2 * VGGP_MAX_D + 1));
+        TRY(dev_alloc(p, &p->obs_counter, 4));
+        cudaDeviceProp prop;
+        rc = (int)cudaGetDeviceProperties(&prop, device);
+        if (rc) { vggp_plan_destroy(p); return fail(rc, "cudaGetDeviceProperties failed"); }
+        p->sm_count = prop.multiProcessorCount;
+        *out = p;
+        return 0;
+    }
     {
         const int band_bytes = (int)(((size_t)p->tab_total * tsz + 15) / 16 * 16);
         const int knot_bytes = (int)(((size_t)p->knot_total * 4 + 15) / 16 * 16);
@@ -2179,7 +2370,8 @@ int vggp_gbuf_layout(const vggp_plan* p, int64_t* n_obs_elems, int64_t* scalar_o
                      int64_t* total_bytes) {
     if (!p) return fail(VGGP_E_ARG, "null plan");
     const i64 tsz = p->obs_dtype == VGGP_F32 ? 4 : 8;
-    const i64 ne = p->M + (p->family != VGGP_B1_ASVGP ? p->gfac_total : (i64)p->band_total);
+    const bool band = p->family == VGGP_B1_ASVGP || p->family == VGGP_SVGP_MARKOV;
+    const i64 ne = p->M + (band ? (i64)p->band_total : p->gfac_total);
     const i64 soff = (ne * tsz + 7) / 8 * 8;
     if (n_obs_elems) *n_obs_elems = ne;
     if (scalar_offset_bytes) *scalar_offset_bytes = soff;
@@ -2195,6 +2387,7 @@ int vggp_grid_forward(vggp_plan* p, const double* theta, const double* m, const 
     const int D = p->D;
     int rc;
     p->last_stream = st;
+    if (p->family == VGGP_SVGP_MARKOV) return svgpm_forward(p, theta, m, L, st);
     if (p->g.structured == 3) return b1f_forward(p, theta, m, L, st);
     VGGP_CUDA(cudaMemcpyAsync(p->mws, m, sizeof(double) * p->M, cudaMemcpyDeviceToDevice, st));
     VGGP_CUDA(cudaMemcpyAsync(p->theta_dev, theta, sizeof(double) * (2 * D + 1), cudaMemcpyDeviceToDevice, st));
@@ -2286,6 +2479,7 @@ int vggp_obs_fwd_bwd_packed(vggp_plan* p, const void* const* xp, const void* yp,
     DeviceGuard dev_guard(p ? p->device : -1);
     if (p && p->det) return fail(VGGP_E_UNSUPPORTED, "deterministic mode takes the binned layout (vggp_obs_fwd_bwd_binned)");
     if (!p || !gbuf || n < 0) return fail(VGGP_E_ARG, "bad argument");
+    if (p->family == VGGP_SVGP_MARKOV) return fail(VGGP_E_UNSUPPORTED, "the Markov SVGP family takes the binned layout (vggp_obs_bin_prepare / _pack, vggp_obs_fwd_bwd_binned)");
     if (n > 0 && (!xp || !yp)) return fail(VGGP_E_ARG, "null observation pointers");
     cudaStream_t st = (cudaStream_t)stream;
     i64 n_elems, soff, nsc, total;
@@ -2303,6 +2497,7 @@ int vggp_obs_fwd_bwd(vggp_plan* p, const void* const* x, const void* y, int64_t 
     DeviceGuard dev_guard(p ? p->device : -1);
     if (p && p->det) return fail(VGGP_E_UNSUPPORTED, "deterministic mode takes the binned layout (vggp_obs_fwd_bwd_binned)");
     if (!p || !gbuf || n < 0) return fail(VGGP_E_ARG, "bad argument");
+    if (p->family == VGGP_SVGP_MARKOV) return fail(VGGP_E_UNSUPPORTED, "the Markov SVGP family takes the binned layout (vggp_obs_bin_prepare / _pack, vggp_obs_fwd_bwd_binned)");
     if (n > 0 && (!x || !y)) return fail(VGGP_E_ARG, "null observation pointers");
     if (n == 0 || p->family != VGGP_B1_ASVGP) {
         cudaStream_t st0 = (cudaStream_t)stream;
@@ -2339,7 +2534,8 @@ int vggp_obs_bin_prepare(vggp_plan* p, const void* const* x, int64_t n, int run_
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !desc || n < 0) return fail(VGGP_E_ARG, "bad argument");
     if (p->family == VGGP_B0_GRIDDED && p->D > 2) return fail(VGGP_E_UNSUPPORTED, "the B0 (cell-integrated) family is built for D <= 2, as in the reference");
-    if (p->family >= VGGP_SVGP_GRID) return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families take plain observation arrays (vggp_obs_fwd_bwd)");
+    if (p->family == VGGP_SVGP_GRID || p->family == VGGP_VFF_GRID)
+        return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families take plain observation arrays (vggp_obs_fwd_bwd)");
     if (run_cap == 0) {
         // automatic: about two tasks (of 32 runs) per resident warp, so that thin shards and cell-range shards (few, full cells)
         // still spread over the whole GPU; 256 (the value the 1-GPU measurements settled on) from 2^25.8 observations up
@@ -2387,7 +2583,9 @@ int vggp_obs_fwd_bwd_binned(vggp_plan* p, const vggp_binned_desc* desc, const vo
     VGGP_CUDA(cudaMemsetAsync(gbuf, 0, (size_t)total, st));
     if (desc->n == 0) return 0;
     if (!binned) return fail(VGGP_E_ARG, "null binned buffer");
-    if (p->family >= VGGP_SVGP_GRID) return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families take plain observation arrays (vggp_obs_fwd_bwd)");
+    if (p->family == VGGP_SVGP_GRID || p->family == VGGP_VFF_GRID)
+        return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families take plain observation arrays (vggp_obs_fwd_bwd)");
+    if (p->family == VGGP_SVGP_MARKOV) return obs_svgpm_dispatch(p, desc, binned, gbuf, st);  // Markov form (svgpm.cuh)
     if (p->family == VGGP_B0_GRIDDED) return obs_b0s_dispatch(p, desc, binned, gbuf, st);     // scan form (b0scan.cuh)
     return obs_binned_dispatch(p, desc, binned, gbuf, st);
 }
@@ -2428,6 +2626,7 @@ int vggp_grid_backward(vggp_plan* p, const double* theta, const double* m, const
     cudaStream_t st = (cudaStream_t)stream;
     const int D = p->D;
     int rc;
+    if (p->family == VGGP_SVGP_MARKOV) return svgpm_backward(p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
     if (p->g.structured == 3) return b1f_backward(p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
     i64 n_elems, soff, nsc, total;
     vggp_gbuf_layout(p, &n_elems, &soff, &nsc, &total);
@@ -2562,6 +2761,7 @@ int vggp_elbo_host(vggp_plan* p, const void* const* x_host, const void* y_host, 
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !theta_host || !m_host || !L_host || !out_host || !dtheta_host || !dm_host || !dL_host || n < 0)
         return fail(VGGP_E_ARG, "bad argument");
+    if (p->family == VGGP_SVGP_MARKOV) return fail(VGGP_E_UNSUPPORTED, "the Markov SVGP family takes the binned layout (vggp_obs_bin_prepare / _pack, vggp_obs_fwd_bwd_binned)");
     if (n > 0 && (!x_host || !y_host)) return fail(VGGP_E_ARG, "null observation pointers");
     cudaStream_t st = (cudaStream_t)stream;
     const int D = p->D;
@@ -2698,7 +2898,7 @@ int vggp_features_dense(const vggp_plan* p, int dim, const void* x, int64_t n, c
         if (p->family == VGGP_VFF_GRID) {
             if (p->obs_dtype == VGGP_F32) k_vff_dense<float><<<grid, 256, 0, st>>>(p->mesh[dim], (const float*)x, n, th[dim], (float*)phi);
             else k_vff_dense<double><<<grid, 256, 0, st>>>(p->mesh[dim], (const double*)x, n, th[dim], (double*)phi);
-        } else if (p->family == VGGP_SVGP_GRID) {
+        } else if (p->family == VGGP_SVGP_GRID || p->family == VGGP_SVGP_MARKOV) {     // the dense k_d(Z, x)
             if (p->obs_dtype == VGGP_F32)
                 k_svgp_dense<float><<<grid, 256, 0, st>>>(p->mesh[dim], (const float*)x, n, th[dim], th[p->D + dim], (float*)phi);
             else
@@ -2719,6 +2919,8 @@ int vggp_predict(vggp_plan* p, const void* const* x, int64_t n, void* mean, void
     if (!x || !mean || !var) return fail(VGGP_E_ARG, "null argument");
     for (int d = 0; d < p->D; ++d)
         if (!x[d]) return fail(VGGP_E_ARG, "null test-point pointer");
+    if (p->family == VGGP_SVGP_MARKOV)      // Markov form, O(1) per point (svgpm.cuh)
+        return predict_svgpm_dispatch(p, x, nullptr, n, mean, var, nullptr, (cudaStream_t)stream);
     if (p->family >= VGGP_SVGP_GRID)
         return fail(VGGP_E_UNSUPPORTED, "SVGP / VFF families: predictions are assembled from vggp_features_dense by the host mirror");
     if (p->family != VGGP_B1_ASVGP)      // B0 family: scan form, O(1) per point (b0scan.cuh)
@@ -2743,13 +2945,15 @@ int vggp_metrics(int dtype, const void* truth, const void* pred, int64_t n, doub
 int vggp_predict_metrics(vggp_plan* p, const void* const* x, const void* y, int64_t n, double* out, void* stream) {
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !out || n < 0) return fail(VGGP_E_ARG, "bad argument");
-    if (p->family != VGGP_B1_ASVGP) return fail(VGGP_E_UNSUPPORTED, "point prediction is built for the B1 family");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "fused prediction metrics are built for the B1 and Markov SVGP families");
     cudaStream_t st = (cudaStream_t)stream;
     VGGP_CUDA(cudaMemsetAsync(out, 0, 4 * sizeof(double), st));
     if (n == 0) return 0;
     if (!x || !y) return fail(VGGP_E_ARG, "null argument");
     for (int d = 0; d < p->D; ++d)
         if (!x[d]) return fail(VGGP_E_ARG, "null test-point pointer");
+    if (p->family == VGGP_SVGP_MARKOV) return predict_svgpm_dispatch(p, x, y, n, nullptr, nullptr, out, st);
     return predict_metrics_dispatch(p, x, y, n, out, st);
 }
 
@@ -2812,6 +3016,8 @@ int vggp_generate_tracks(int dtype, int D, int64_t n_total, int64_t lo, int64_t 
 int vggp_workspace_ptr(const vggp_plan* p, int which, int dim, double** ptr, int64_t* n_elems) {
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !ptr) return fail(VGGP_E_ARG, "null argument");
+    if (p->family == VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the Markov SVGP family keeps bands and per-cell tables only: no dense workspace array");
     if (which != VGGP_WS_ALPHA && which != VGGP_WS_SCAL && (dim < 0 || dim >= p->D)) return fail(VGGP_E_ARG, "bad dim");
     const i64 nn = (which == VGGP_WS_ALPHA || which == VGGP_WS_SCAL) ? 0 : (i64)p->n[dim] * p->n[dim];
     switch (which) {

@@ -115,7 +115,9 @@ class GriddedVariationalGP(nn.Module):
             # VGGP_OBS_LAYOUT=packed selects the round-1 layouts (B1: cell-sorted packed runs, B0: plain arrays through the
             # dense-feature kernel), kept as cross-checks.
             layout = os.environ.get("VGGP_OBS_LAYOUT", "binned")
-            if self.family in (_lib.SVGP_GRID, _lib.VFF_GRID):
+            if self.family == _lib.SVGP_MARKOV:
+                self._packed = self._plan.bin(xs, y)        # the only observation layout of the Markov form
+            elif self.family in (_lib.SVGP_GRID, _lib.VFF_GRID):
                 self._packed = None                 # dense-feature kernel: plain arrays
             elif layout == "binned" and not (self.family != _lib.B1_ASVGP and self.D > 2):
                 self._packed = self._plan.bin(xs, y)
@@ -161,6 +163,9 @@ class GriddedVariationalGP(nn.Module):
             xs, y = self._obs
         scale = 1.0
         if batch is not None:
+            if self.family == _lib.SVGP_MARKOV:
+                raise NotImplementedError("minibatches of the Markov SVGP form need the plain-array per-observation path, which "
+                                          "this family does not have yet: call _elbo() on the full (sharded) data set")
             xs = [x[batch].contiguous() for x in self._obs[0]]
             y = self._obs[1][batch].contiguous()
             n_local = self._obs[1].numel()

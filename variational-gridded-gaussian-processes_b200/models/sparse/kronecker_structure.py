@@ -85,10 +85,20 @@ class Matern12SVGP(_DenseFeatureModel):
     here); the columns of Z are sorted (the library wants increasing knots; the product grid is the same set); and Z is a
     fixed buffer -- the reference registers it as a parameter, d ELBO / d Z is not computed here.  Per-observation work
     goes through the dense-feature kernel (k_obs_b0 with s2 exp(-|x - z| / l) features): O(M + sum M_d^2) per observation,
-    the reference's own dense algorithm, meant for the grid sizes the reference uses (tens of points per dimension)."""
+    the reference's own dense algorithm, meant for the grid sizes the reference uses (tens of points per dimension).
+
+    `markov=True` evaluates the same model (same ELBO, gradients and predictions) in its O(1)-per-observation Markov form
+    (family SVGP_MARKOV, csrc/svgpm.cuh): K_d^-1 is tridiagonal for a Matern-1/2 kernel on sorted points, so every
+    observation touches two inducing points per dimension, the grid side is O(M + sum M_d^2), and 512 x 512 grids with
+    2^26 observations are in reach.  Full-batch `_elbo()` only (a minibatch raises NotImplementedError).  The default stays
+    the dense path for now; the intended follow-up makes `markov=True` the default and keeps SVGP_GRID as the test
+    reference."""
     family = _lib.SVGP_GRID
 
-    def __init__(self, X, y, Z: torch.Tensor):
+    def __init__(self, X, y, Z: torch.Tensor, markov: bool = False):
+        self.markov = bool(markov)
+        if self.markov:
+            self.family = _lib.SVGP_MARKOV
         Z = torch.as_tensor(Z).detach()
         if Z.dim() != 2 or Z.shape[1] != 2:
             raise ValueError("Z must be (m, 2): one column of inducing locations per dimension")
@@ -98,6 +108,13 @@ class Matern12SVGP(_DenseFeatureModel):
                 raise ValueError("the inducing locations of a dimension must be distinct")
         super().__init__(X, y, cols)
         self.register_buffer("Z", torch.stack(cols, dim=1))
+
+    def posterior(self, x: torch.Tensor) -> GriddedMarginals:
+        """Marginals of q(f(x*)): the dense-feature assembly, or with `markov=True` the library's O(1)-per-point prediction
+        (vggp_predict)."""
+        if self.markov:
+            return GriddedVariationalGP.posterior(self, x)
+        return super().posterior(x)
 
 
 class Matern12VFFGP(_DenseFeatureModel):
