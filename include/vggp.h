@@ -24,8 +24,8 @@
  *   - every function returns int: 0 = ok, < 0 = invalid argument (VGGP_E_*), > 0 = a cudaError_t value;
  *     vggp_last_error() returns a static/thread-local message for the last non-zero status.
  *   - all work is asynchronous and ordered on the `stream` argument (a cudaStream_t passed as void*;
- *     NULL = the legacy default stream).  No entry point except vggp_plan_create/destroy, vggp_read_info and
- *     vggp_elbo_host synchronises the host.
+ *     NULL = the legacy default stream).  No entry point except vggp_plan_create/destroy, vggp_read_info,
+ *     vggp_elbo_host and vggp_meanopt_solve synchronises the host.
  *   - the caller owns every buffer passed in; the library allocates only inside vggp_plan_create (its
  *     grid-side workspace) and frees it in vggp_plan_destroy.
  *   - pointers are DEVICE pointers unless the parameter name ends in `_host`.
@@ -103,7 +103,7 @@ int vggp_plan_destroy(vggp_plan* plan);
 /* Device memory behind a plan (SURVEY.md section 8b): `plan_bytes` = everything vggp_plan_create allocated (factors, work
  * tensors, tables: the callee never allocates in a step), `gbuf_bytes` = the caller-owned gradient buffer a step needs
  * (= vggp_gbuf_layout total), `scratch_bytes` = what the opt-in paths have grown so far (plain-array staging of
- * vggp_obs_fwd_bwd / vggp_elbo_host, deterministic mode, B0 scan tables).  Any output pointer may be null. */
+ * vggp_obs_fwd_bwd / vggp_elbo_host, deterministic mode, B0 scan tables, the optimal-mean system).  Any output pointer may be null. */
 int vggp_workspace_bytes(const vggp_plan* plan, int64_t* plan_bytes, int64_t* gbuf_bytes, int64_t* scratch_bytes);
 
 /* M_d (inducing variables per dimension) and M = prod M_d. */
@@ -287,6 +287,33 @@ int vggp_info_async(vggp_plan* plan, int* info_pinned_host, void* stream);
 int vggp_elbo_host(vggp_plan* plan, const void* const* x_host, const void* y_host, int64_t n,
                    const double* theta_host, const double* m_host, const double* L_host, double ell_scale,
                    double* out_host, double* dtheta_host, double* dm_host, double* dL_host, void* stream);
+
+/*
+ * Optimal variational mean (B1 family and VGGP_SVGP_MARKOV; VGGP_E_UNSUPPORTED otherwise): the m that maximises the ELBO for
+ * fixed theta, which is the mean of the reference's closed-form q_u(): m* = Kuu Sigma^-1 Kuf y / noise,
+ * Sigma = Kuu + Kuf Kuf^T / noise.  The m-dependent part of the ELBO, -(1/2 noise) ||y - mu(m)||^2 - (1/2) m^T Kuu^-1 m, does
+ * not depend on S, and every observation has 2^D non-zero weights w (the corners of its cell), so m* solves a symmetric
+ * positive definite 3^D-point stencil system on the node grid (csrc/meanopt.cuh):
+ *     B1:                (Kuu + G / noise) alpha = b / noise,   m* = Kuu alpha*      mu = Phi^T alpha,  Kuu = kron_d K_d
+ *     VGGP_SVGP_MARKOV:  (Kuu^-1 + G / noise) m* = b / noise                         mu = Psi^T m,  Psi = Kuu^-1 Kuf
+ * with G = sum_n w_n w_n^T and b = sum_n w_n y_n (B1: hat weights, observations outside the mesh contribute nothing; Markov:
+ * the two weights per dimension of the extended cells, virtual corners dropped).
+ *   vggp_meanopt_assemble  zeroes and fills G and b (plan-owned float64) in one pass over a binned buffer of this plan
+ *                          (vggp_obs_bin_pack).  Asynchronous; the first call allocates the system and the solver's
+ *                          vectors (about (3^D + 13) / 2 M float64, counted in scratch_bytes of vggp_workspace_bytes) and
+ *                          must not be captured.  VGGP_SVGP_MARKOV uses the theta of the last vggp_grid_forward; the B1
+ *                          system does not depend on theta.
+ *   vggp_meanopt_solve     Jacobi-preconditioned conjugate gradients in float64 at the theta of the last vggp_grid_forward,
+ *                          from the state of that forward (B1: its alpha; Markov: its m, in the observation dtype): a forward
+ *                          at m = 0 is a cold start, a forward at a previous m* a warm start.  Stops once
+ *                          ||r|| <= rtol ||b / noise|| or after max_iter iterations; writes m_out [M] (DEVICE, float64),
+ *                          the iterations and the final relative residual.  Returns 0 also when it did not converge
+ *                          (*iters_host == max_iter and *relres_host > rtol).  No data (b = 0): m* = 0, 0 iterations,
+ *                          relres 0.  VGGP_E_ARG without a previous vggp_meanopt_assemble.  Synchronises `stream`.
+ */
+int vggp_meanopt_assemble(vggp_plan* plan, const vggp_binned_desc* desc, const void* binned, void* stream);
+int vggp_meanopt_solve(vggp_plan* plan, double rtol, int max_iter, double* m_out,
+                       int* iters_host, double* relres_host, void* stream);
 
 /* ---- feature evaluation (bit-exact restatement of the reference's basis calls) ------------------------- */
 

@@ -66,6 +66,8 @@ SIGNATURES = {
     "vggp_minmax_scale": (C.c_int, [C.c_int, _dp, _i64, _dp, C.c_int, _dp, _vp]),
     "vggp_generate_tracks": (C.c_int, [C.c_int, C.c_int, _i64, _i64, _i64, _i64, C.c_int, C.c_double, C.POINTER(_vp), _vp, _vp]),
     "vggp_elbo_host": (C.c_int, [_vp, C.POINTER(_vp), _vp, _i64, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp]),
+    "vggp_meanopt_assemble": (C.c_int, [_vp, C.POINTER(BinnedDesc), _dp, _vp]),
+    "vggp_meanopt_solve": (C.c_int, [_vp, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), C.POINTER(C.c_double), _vp]),
     "vggp_b1_stencil": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _dp, _vp]),
     "vggp_features_dense": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _vp]),
     "vggp_workspace_ptr": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(_vp), C.POINTER(_i64)]),

@@ -17,6 +17,7 @@
 #include "metrics.cuh"
 #include "b0scan.cuh"
 #include "svgpm.cuh"
+#include "meanopt.cuh"
 #include "collective.cuh"
 
 // Every plan-taking entry point runs with the plan's device current and restores the caller's device on return
@@ -141,6 +142,9 @@ struct vggp_plan {
     int det = 0;
     void* det_buf = nullptr; size_t det_bytes = 0;
     double* det_fp = nullptr; size_t det_fp_elems = 0;
+    // optimal variational mean (meanopt.cuh): G, b, the CG vectors, the B1 prior bands and the CG status in one buffer,
+    // allocated at the first vggp_meanopt_assemble (scratch_bytes of vggp_workspace_bytes)
+    void* mo_buf = nullptr; size_t mo_bytes = 0; bool mo_assembled = false;
     void* band_rep = nullptr;              // B1 family, binned kernel: BAND_REPLICAS copies of the band block (obs dtype), kept zero
                                            // between launches (k_band_reduce clears what it sums)
     // schedules
@@ -2083,6 +2087,152 @@ int predict_svgpm_dispatch(vggp_plan* p, const void* const* x, const void* y, i6
     VGGP_DISPATCH_TD(p, launch_predict_svgpm, p, x, y, n, mean, var, out, st);
 }
 
+
+// ---- optimal variational mean (meanopt.cuh) ---------------------------------------------------------------------
+struct MoLayout {
+    double *G, *b, *x, *r, *p, *q, *dinv, *band;
+    MoStatus* st;
+    int band_stride;
+    size_t bytes;
+};
+
+MoLayout mo_layout(const vggp_plan* p) {
+    const int slots = p->D == 1 ? MoSlots<1>::v : (p->D == 2 ? MoSlots<2>::v : MoSlots<3>::v);
+    MoLayout L;
+    double* base = reinterpret_cast<double*>(p->mo_buf);
+    const i64 M = p->M;
+    L.G = base;
+    L.b = L.G + (i64)slots * M;
+    L.x = L.b + M; L.r = L.x + M; L.p = L.r + M; L.q = L.p + M; L.dinv = L.q + M;
+    L.band = L.dinv + M;
+    L.band_stride = 2 * p->nmax;
+    L.st = reinterpret_cast<MoStatus*>(L.band + (i64)p->D * L.band_stride);
+    L.bytes = (size_t)((i64)(slots + 6) * M + (i64)p->D * L.band_stride) * sizeof(double) + sizeof(MoStatus);
+    return L;
+}
+
+template <typename T, int D>
+int mo_assemble_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, cudaStream_t st) {
+    const MoLayout L = mo_layout(p);
+    unsigned int* counter = p->obs_counter + 2;          // slot 2: this kernel's work-stealing counter, cleared here
+    VGGP_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned int), st));
+    VGGP_CUDA(cudaMemsetAsync(L.G, 0, sizeof(double) * (size_t)(L.x - L.G), st));
+    if (desc->n_tasks == 0) return 0;
+    BinnedArgs<T, D> a;
+    memset(&a, 0, sizeof(a));
+    a.buf = reinterpret_cast<const unsigned char*>(binned);
+    a.off_task_off = desc->off_task_off; a.off_task_R = desc->off_task_R; a.off_run_cell = desc->off_run_cell;
+    a.off_run_n = desc->off_run_n; a.off_data = desc->off_data;
+    a.n_tasks = (int)desc->n_tasks;
+    a.counter = counter;
+    i64 blocks = (desc->n_tasks + BIN_WARPS - 1) / BIN_WARPS;
+    if (p->family == VGGP_B1_ASVGP) {
+        for (int d = 0; d < D; ++d) {
+            a.geo.K[d] = p->K[d];
+            a.geo.stride[d] = (int)p->stride[d];
+            a.geo.tab_off[d] = p->tab_off[d];
+            a.geo.knot_off[d] = p->knot_off[d];
+        }
+        a.tables = p->tables;
+        a.knots_byte_off = p->knots_byte_off;
+        int nb = 0;
+        VGGP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_mo_b1_assemble<T, D>, BIN_THREADS, 0));
+        blocks = std::max<i64>(1, std::min<i64>(blocks, (i64)p->sm_count * std::max(nb, 1)));
+        k_mo_b1_assemble<T, D><<<(unsigned)blocks, BIN_THREADS, 0, st>>>(a, L.G, L.b, p->M);
+    } else {
+        SvgpmArgs<T, D> sa;
+        memset(&sa, 0, sizeof(sa));
+        sa.bin = a;
+        sa.geo = svgpm_geom<D>(p);
+        sa.tab = reinterpret_cast<const T*>(p->svm_tab);
+        sa.theta = p->theta_dev;
+        int nb = 0;
+        VGGP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_mo_svm_assemble<T, D>, BIN_THREADS, 0));
+        blocks = std::max<i64>(1, std::min<i64>(blocks, (i64)p->sm_count * std::max(nb, 1)));
+        k_mo_svm_assemble<T, D><<<(unsigned)blocks, BIN_THREADS, 0, st>>>(sa, L.G, L.b, p->M);
+    }
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+int mo_assemble_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, mo_assemble_impl, p, desc, binned, st);
+}
+
+constexpr int MO_BATCH = 64;        // CG iterations launched between two reads of the status record
+
+template <int D>
+int mo_solve_impl(vggp_plan* p, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
+                  cudaStream_t st) {
+    const MoLayout L = mo_layout(p);
+    const bool b1 = p->family == VGGP_B1_ASVGP;
+    MoSys<D> s;
+    memset(&s, 0, sizeof(s));
+    s.M = p->M;
+    for (int d = 0; d < D; ++d) {
+        s.n[d] = p->n[d];
+        s.stride[d] = (int)p->stride[d];
+        if (b1) {
+            s.bd[d] = L.band + (i64)d * L.band_stride;
+            s.bo[d] = s.bd[d] + p->n[d];
+        } else {
+            s.bd[d] = p->svm_W[d] + (i64)SVW_PD * p->n[d];
+            s.bo[d] = p->svm_W[d] + (i64)SVW_PO * p->n[d];
+        }
+    }
+    s.G = L.G;
+    s.theta = p->theta_dev;
+    const unsigned blocks = (unsigned)std::min<i64>((p->M + 255) / 256, (i64)p->sm_count * 8);
+    if (b1) {
+        k_mo_b1_bands<<<dim3(ceil_div(p->nmax, 256), D), 256, 0, st>>>(p->g, p->theta_dev, L.band, L.band_stride);
+        VGGP_LAUNCH_CHECK();
+    }
+    VGGP_CUDA(cudaMemsetAsync(L.st, 0, sizeof(MoStatus), st));
+    // initial guess: the state of the last grid forward (B1: alpha = Kuu^-1 m in float64; Markov: m as the kernels read it)
+    if (b1) k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, p->alpha, L.x, L.r, L.p, L.dinv, L.st);
+    else if (p->obs_dtype == VGGP_F32)
+        k_mo_init<float, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const float*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
+    else k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const double*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
+    VGGP_LAUNCH_CHECK();
+    MoStatus h;
+    VGGP_CUDA(cudaMemcpyAsync(&h, L.st, sizeof(MoStatus), cudaMemcpyDeviceToHost, st));
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    if (h.bb == 0.0) {          // no data: m* = 0
+        VGGP_CUDA(cudaMemsetAsync(m_out, 0, sizeof(double) * (size_t)p->M, st));
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        *iters_host = 0;
+        *relres_host = 0.0;
+        return 0;
+    }
+    double relres = sqrt(h.rr_acc / h.bb);
+    int iters = 0;
+    while (relres > rtol && iters < max_iter) {
+        const int nb = std::min(MO_BATCH, max_iter - iters);
+        for (int k = 0; k < nb; ++k) {
+            k_mo_matvec<D><<<blocks, 256, 0, st>>>(s, L.p, L.q, L.st);
+            VGGP_LAUNCH_CHECK();
+            k_mo_update<<<blocks, 256, 0, st>>>(p->M, L.p, L.q, L.dinv, L.x, L.r, L.st);
+            VGGP_LAUNCH_CHECK();
+            k_mo_direction<<<blocks, 256, 0, st>>>(p->M, L.r, L.dinv, L.p, rtol, L.st);
+            VGGP_LAUNCH_CHECK();
+        }
+        VGGP_CUDA(cudaMemcpyAsync(&h, L.st, sizeof(MoStatus), cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        iters = h.iters;
+        relres = h.relres;
+        if (h.done) break;
+    }
+    if (b1) {
+        k_mo_prior_apply<D><<<blocks, 256, 0, st>>>(s, L.x, m_out);
+        VGGP_LAUNCH_CHECK();
+    } else {
+        VGGP_CUDA(cudaMemcpyAsync(m_out, L.x, sizeof(double) * (size_t)p->M, cudaMemcpyDeviceToDevice, st));
+    }
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    *iters_host = iters;
+    *relres_host = relres;
+    return 0;
+}
+
 extern "C" {
 
 int vggp_abi_version(void) { return VGGP_ABI_VERSION; }
@@ -2107,7 +2257,7 @@ int vggp_workspace_bytes(const vggp_plan* p, int64_t* plan_bytes, int64_t* gbuf_
     if (gbuf_bytes) *gbuf_bytes = total;
     if (scratch_bytes) {
         const size_t tsz = p->obs_dtype == VGGP_F32 ? 4 : 8;
-        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes;
+        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes;
         if (p->st_x) sc += (size_t)p->st_n * tsz * (p->D + 1) + sizeof(double) * (2 * (size_t)p->M + 2 * (size_t)p->Lsize) + (size_t)total;
         *scratch_bytes = (int64_t)sc;
     }
@@ -2347,6 +2497,7 @@ int vggp_plan_destroy(vggp_plan* p) {
     if (p->det_buf) cudaFree(p->det_buf);
     if (p->one_ws) cudaFree(p->one_ws);
     if (p->det_fp) cudaFree(p->det_fp);
+    if (p->mo_buf) cudaFree(p->mo_buf);
     for (auto& e : p->k1_ev) cudaEventDestroy(e);
     for (auto& e : p->k1_gev) if (e) cudaEventDestroy(e);
     for (auto& e : p->st_ev) cudaEventDestroy(e);
@@ -2926,6 +3077,44 @@ int vggp_predict(vggp_plan* p, const void* const* x, int64_t n, void* mean, void
     if (p->family != VGGP_B1_ASVGP)      // B0 family: scan form, O(1) per point (b0scan.cuh)
         return predict_b0s_dispatch(p, x, n, mean, var, (cudaStream_t)stream);
     return predict_dispatch(p, x, n, mean, var, (cudaStream_t)stream);
+}
+
+int vggp_meanopt_assemble(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !desc) return fail(VGGP_E_ARG, "null argument");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the optimal mean is built for the B1 and VGGP_SVGP_MARKOV families (3^D-stencil system)");
+    if (desc->D != p->D || desc->n_tasks < 0 || (desc->n_tasks > 0 && !binned))
+        return fail(VGGP_E_ARG, "binned buffer does not match the plan");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!p->mo_buf) {
+        const size_t want = mo_layout(p).bytes;
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusActive)
+            return fail(VGGP_E_UNSUPPORTED, "the first vggp_meanopt_assemble allocates: call it outside a stream capture");
+        VGGP_CUDA(cudaMalloc(&p->mo_buf, want));
+        p->mo_bytes = want;
+    }
+    p->mo_assembled = false;
+    if (int rc = mo_assemble_dispatch(p, desc, binned, st)) return rc;
+    p->mo_assembled = true;
+    return 0;
+}
+
+int vggp_meanopt_solve(vggp_plan* p, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
+                       void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !m_out || !iters_host || !relres_host) return fail(VGGP_E_ARG, "null argument");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the optimal mean is built for the B1 and VGGP_SVGP_MARKOV families (3^D-stencil system)");
+    if (!(rtol >= 0.0) || max_iter < 0) return fail(VGGP_E_ARG, "rtol must be >= 0 and max_iter >= 0");
+    if (!p->mo_assembled) return fail(VGGP_E_ARG, "vggp_meanopt_solve needs a previous vggp_meanopt_assemble on this plan");
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (p->D) {
+        case 1: return mo_solve_impl<1>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
+        case 2: return mo_solve_impl<2>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
+        default: return mo_solve_impl<3>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
+    }
 }
 
 int vggp_metrics(int dtype, const void* truth, const void* pred, int64_t n, double* out, void* stream) {

@@ -17,7 +17,7 @@ from torch import nn
 
 from .. import _lib
 from ..params import DenseNormal, GaussianLikelihood, GriddedMarginals, GriddedNormal, MaternKernel, ScaleKernel
-from ..plan import GridPlan, gridded_elbo
+from ..plan import BinnedObs, GridPlan, gridded_elbo
 from ..dist import shard_bounds
 
 
@@ -198,6 +198,45 @@ class GriddedVariationalGP(nn.Module):
             Lt = torch.tril(L.detach())
             Ss.append(Lt @ Lt.T)
         return GriddedNormal(self.variational_mean.detach(), Ss)
+
+    MEANOPT_MAX_ITER = 20000
+
+    @torch.no_grad()
+    def set_optimal_mean(self, rtol: float = 1e-10, max_iter: Optional[int] = None) -> dict:
+        """Load the optimal variational mean at the current hyper-parameters into `variational_mean`: the m that maximises
+        the ELBO for fixed theta and S, which is the mean of the reference's q_u() (m* = Kuu Sigma^-1 Kuf y / noise), at any
+        grid size.  One pass over the binned observations assembles a 3^D-stencil system, Jacobi-preconditioned conjugate
+        gradients solve it from the current mean (include/vggp.h, vggp_meanopt_*).  B1 and Markov SVGP families.
+        `max_iter` defaults to MEANOPT_MAX_ITER = 20000.  Measured on one B200 to rtol 1e-8 from m = 0 (float32 track
+        observations, profiles/optimal_mean/): 512 x 512 points, 2^26 observations: B1 678, Markov 59 iterations; 2^22
+        observations: B1 3054, Markov 283; 64 x 64 x 16 points, 2^20 observations: Markov 16046, B1 not converged after
+        60000 (Jacobi preconditioning is too weak for the 3-D B1 prior, DESIGN.md section 7).
+        Returns {"iterations", "relres"}; raises RuntimeError, leaving `variational_mean` unchanged, if the solve stops
+        above `rtol`."""
+        if self.family not in (_lib.B1_ASVGP, _lib.SVGP_MARKOV):
+            raise NotImplementedError("set_optimal_mean() needs the 3^D-stencil system of the B1 and Markov SVGP families; "
+                                      "for this family use set_optimal_q() (dense, M <= 4096)")
+        if self._group is not None:
+            raise NotImplementedError("set_optimal_mean() on a sharded model would need the rank sum of the assembled "
+                                      "system, which is not implemented")
+        plan = self._ensure_plan()
+        plan.grid_forward(self._theta(), self.variational_mean.detach().to(torch.float64).contiguous(),
+                          torch.cat([c.detach().to(torch.float64).reshape(-1) for c in self._chols()]).contiguous())
+        binned = self._packed if isinstance(self._packed, BinnedObs) else None
+        if binned is None:                         # VGGP_OBS_LAYOUT=packed: bin once, for this purpose only
+            if getattr(plan, "_mo_binned", (None,))[0] is not self._obs:
+                plan._mo_binned = (self._obs, plan.bin(*self._obs))
+            binned = plan._mo_binned[1]
+        # the B1 system does not depend on theta: assembled once per plan and data set; the Markov one on every call
+        if self.family != _lib.B1_ASVGP or getattr(plan, "_mo_obs", None) is not self._obs:
+            plan.meanopt_assemble(binned)
+            plan._mo_obs = self._obs if self.family == _lib.B1_ASVGP else None
+        m, iters, relres = plan.meanopt_solve(rtol, self.MEANOPT_MAX_ITER if max_iter is None else max_iter)
+        if not relres <= rtol:
+            raise RuntimeError(f"set_optimal_mean(): conjugate gradients stopped after {iters} iterations at relative residual "
+                               f"{relres:.3e} > rtol = {rtol:.1e}; variational_mean is unchanged")
+        self.variational_mean.copy_(m.to(self.variational_mean.dtype))
+        return {"iterations": iters, "relres": relres}
 
     # ---- the reference's closed-form (collapsed) quantities: dense M x M algebra, small problems only -------------
     DENSE_LIMIT = 4096          # largest M for which dense M x M matrices are formed (128 MiB in float64)

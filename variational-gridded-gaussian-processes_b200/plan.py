@@ -118,6 +118,24 @@ class GridPlan:
                                               _stream_ptr(self.device)))
         return BinnedObs(buf, desc, 4 if self.obs_dtype == torch.float32 else 8)
 
+    def meanopt_assemble(self, binned: "BinnedObs"):
+        """Fill the stencil system of the optimal variational mean from a binned buffer of this plan
+        (vggp_meanopt_assemble; B1 and SVGP_MARKOV families, the latter at the theta of the last grid_forward)."""
+        if not isinstance(binned, BinnedObs):
+            raise TypeError("meanopt_assemble takes the BinnedObs of GridPlan.bin")
+        _lib.check(self.lib.vggp_meanopt_assemble(self.handle, C.byref(binned.desc), binned.buf.data_ptr(),
+                                                  _stream_ptr(self.device)))
+
+    def meanopt_solve(self, rtol: float, max_iter: int):
+        """Conjugate gradients on the assembled system from the state of the last grid_forward (vggp_meanopt_solve;
+        synchronises).  Returns (m_star float64 [M], iterations, final relative residual); not converged when
+        relres > rtol."""
+        m = torch.empty(self.M, dtype=torch.float64, device=self.device)
+        it, rr = C.c_int(0), C.c_double(0.0)
+        _lib.check(self.lib.vggp_meanopt_solve(self.handle, float(rtol), int(max_iter), m.data_ptr(), C.byref(it),
+                                               C.byref(rr), _stream_ptr(self.device)))
+        return m, int(it.value), float(rr.value)
+
     def predict(self, xs: Sequence[torch.Tensor]):
         """Marginal mean and variance of q(f(x*)) at test points, from the state of the last grid_forward."""
         n = int(xs[0].numel())
