@@ -25,7 +25,7 @@
  *     vggp_last_error() returns a static/thread-local message for the last non-zero status.
  *   - all work is asynchronous and ordered on the `stream` argument (a cudaStream_t passed as void*;
  *     NULL = the legacy default stream).  No entry point except vggp_plan_create/destroy, vggp_read_info,
- *     vggp_elbo_host and vggp_meanopt_solve synchronises the host.
+ *     vggp_elbo_host, vggp_meanopt_solve and vggp_meanopt_solve_pc synchronises the host.
  *   - the caller owns every buffer passed in; the library allocates only inside vggp_plan_create (its
  *     grid-side workspace) and frees it in vggp_plan_destroy.
  *   - pointers are DEVICE pointers unless the parameter name ends in `_host`.
@@ -310,10 +310,24 @@ int vggp_elbo_host(vggp_plan* plan, const void* const* x_host, const void* y_hos
  *                          the iterations and the final relative residual.  Returns 0 also when it did not converge
  *                          (*iters_host == max_iter and *relres_host > rtol).  No data (b = 0): m* = 0, 0 iterations,
  *                          relres 0.  VGGP_E_ARG without a previous vggp_meanopt_assemble.  Synchronises `stream`.
+ *   vggp_meanopt_solve_pc  the same solve with a choice of preconditioner `precond`; VGGP_E_ARG for any other value:
+ *                          VGGP_MEANOPT_JACOBI      = vggp_meanopt_solve, bit for bit.
+ *                          VGGP_MEANOPT_KRONECKER   kron_d (F_d + g I)^-1, applied exactly: F_d is the tridiagonal prior
+ *                                                   factor of dimension d (B1: K_d; Markov: K_d^-1) and
+ *                                                   g = (trace(G) / (noise M))^(1/D).  One application is D batched
+ *                                                   tridiagonal solves along the modes of the node grid.  It converges on
+ *                                                   3-D B1 grids where Jacobi does not (DESIGN.md section 4, K1m).  The
+ *                                                   first call allocates its vector and factors (M + 3 sum M_d float64,
+ *                                                   counted in scratch_bytes).
+ *                          Synchronises `stream`.
  */
+#define VGGP_MEANOPT_JACOBI    0
+#define VGGP_MEANOPT_KRONECKER 1
 int vggp_meanopt_assemble(vggp_plan* plan, const vggp_binned_desc* desc, const void* binned, void* stream);
 int vggp_meanopt_solve(vggp_plan* plan, double rtol, int max_iter, double* m_out,
                        int* iters_host, double* relres_host, void* stream);
+int vggp_meanopt_solve_pc(vggp_plan* plan, int precond, double rtol, int max_iter, double* m_out,
+                          int* iters_host, double* relres_host, void* stream);
 
 /* ---- feature evaluation (bit-exact restatement of the reference's basis calls) ------------------------- */
 

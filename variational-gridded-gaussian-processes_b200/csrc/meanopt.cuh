@@ -514,5 +514,217 @@ __global__ void __launch_bounds__(256) k_mo_prior_apply(const __grid_constant__ 
         out[u] = mo_row<D, false, double>(s, u, x, 0.0, nullptr);
 }
 
+// ---- grid side: CG preconditioned by kron_d (F_d + g I)^-1 ---------------------------------------------------------
+// F_d is the tridiagonal prior factor of dimension d (MoSys::bd / bo) and g = (sum_u G[u][u] / (noise M))^(1 / D), so
+// kron_d (F_d + g I) matches the prior and the mean data diagonal of the system.  One application is D tridiagonal solves,
+// one per mode of the row-major (M_1, ..., M_D) tensor.  Per dimension the Thomas factors [l | 1 / d' | off] (n each):
+//     forward   y_i = x_i - l_i y_{i-1}                     (l_0 = 0)
+//     backward  z_i = (y_i - off_i z_{i+1}) / d'_i          (off_{n-1} = 0)
+// Kernels of one Kronecker iteration: k_mo_matvec, k_mo_kron_update (x, r, rr_acc), D x k_mo_kron_sweep (z = P r, the last
+// one adds r.z to rz_acc), k_mo_kron_direction (p = z + beta p).  The Jacobi kernels above are not used by this solve.
+struct MoKron {
+    double gsum;                 // sum_u G[0][u], the trace of G
+};
+template <int D> struct MoFacOff { int off[D]; };      // offset of dimension d's factors: 3 sum_{e < d} M_e
+
+// trace of G (slot 0 is the diagonal) into k->gsum (zeroed before)
+__global__ void __launch_bounds__(256) k_mo_kron_trace(i64 M, const double* __restrict__ G, MoKron* k) {
+    __shared__ double red[32];
+    double acc = 0.0;
+    for (i64 u = (i64)blockIdx.x * blockDim.x + threadIdx.x; u < M; u += (i64)gridDim.x * blockDim.x) acc += G[u];
+    acc = block_sum(acc, red);
+    if (threadIdx.x == 0) atomicAdd(&k->gsum, acc);
+}
+
+// Thomas LU of F_d + g I, one thread per dimension (SPD tridiagonal: no pivoting).  fac + fac_off[d]: [l | 1 / d' | off]
+template <int D>
+__global__ void __launch_bounds__(32) k_mo_kron_factors(const __grid_constant__ MoSys<D> s, const MoKron* k,
+                                                        double* __restrict__ fac, const __grid_constant__ MoFacOff<D> fo) {
+    const int d = threadIdx.x;
+    if (d >= D) return;
+    const double g = pow(fmax(k->gsum, 0.0) / (s.theta[2 * D] * (double)s.M), 1.0 / D);
+    const int n = s.n[d];
+    const double* bd = s.bd[d];
+    const double* bo = s.bo[d];
+    double* l = fac + fo.off[d];
+    double* invd = l + n;
+    double* off = invd + n;
+    double dinv = 1.0 / (bd[0] + g);
+    l[0] = 0.0;
+    invd[0] = dinv;
+    for (int i = 1; i < n; ++i) {
+        const double o = bo[i - 1], li = o * dinv;
+        dinv = 1.0 / (bd[i] + g - li * o);
+        l[i] = li;
+        invd[i] = dinv;
+        off[i - 1] = o;
+    }
+    off[n - 1] = 0.0;
+}
+
+// Tridiagonal solve along one mode, in place or from `in` to `out`.  The mode has n nodes and stride `inner`; its F = M / n
+// fibres are f = outer * inner + j at elements outer * n * inner + j + i * inner.  Each fibre is cut into S segments of Ls
+// nodes, one thread per (fibre, segment), so short fibre counts still fill the GPU.  An affine map x -> a x + b composes in
+// either order, so each segment needs only its own elements to know its start values:
+//   1. (S > 1) compose the forward map of the segment from a zero start: one read;
+//   2. chain the forward maps of the fibre's earlier segments in shared memory into this segment's start value y_{lo-1};
+//      run the exact forward recurrence from it, writing y, and compose the backward map of the segment from the y it
+//      produces: one read, one write;
+//   3. chain the backward maps of the later segments into z_{hi}; run the exact backward recurrence: one read, one write.
+//   STAGED = false (modes d < D - 1): thread t is fibre t % FB of segment t / FB, FB = 32 consecutive fibres per segment, so
+//                  a warp reads 32 consecutive doubles at every step.  Global traffic per element: 3 reads and 2 writes
+//                  (2 and 2 with S = 1); the second and third passes re-read what the block has just touched.
+//   STAGED = true  (the contiguous mode, inner = 1): the block's FB rows are one contiguous range, copied into shared memory
+//                  with coalesced loads, swept there, and written back the same way (one global read and one write per
+//                  element); thread t is segment t % S of row t / S, and segment s of a row starts at s * P in shared
+//                  memory with P = Ls | 1, so a half warp reads 16 different banks.
+// RZ (STAGED only: the last sweep of an application is the contiguous mode): also add r.z over the block's elements into
+// st->rz_acc.
+struct MoSweep {
+    i64 F, inner;
+    int n, S, Ls, P;
+    const double* fac;           // [l | 1 / d' | off] of this dimension
+};
+
+template <bool STAGED, bool RZ>
+__global__ void __launch_bounds__(1024) k_mo_kron_sweep(const __grid_constant__ MoSweep w, const double* in, double* out,
+                                                        const double* __restrict__ r, MoStatus* st) {
+    static_assert(STAGED || !RZ, "r.z is accumulated by the staged sweep of the contiguous mode");
+    __shared__ double sa[1024], sb[1024], red[32];
+    extern __shared__ double sm[];
+    if (st->done) return;
+    const int tid = threadIdx.x, S = w.S, FB = (int)blockDim.x / S, n = w.n;
+    const int seg = STAGED ? tid % S : tid / FB, fl = STAGED ? tid / S : tid % FB;
+    const i64 f0 = (i64)blockIdx.x * FB, f = f0 + fl;
+    const bool act = f < w.F;
+    const int lo = min(n, seg * w.Ls), hi = min(n, lo + w.Ls);
+    const double* __restrict__ l = w.fac;
+    const double* __restrict__ invd = l + n;
+    const double* __restrict__ off = invd + n;
+    // element i of this thread's fibre: src[i * step], dst[i * step]
+    const double* src;
+    double* dst;
+    i64 step;
+    const i64 nrows = min((i64)FB, w.F - f0);
+    if (STAGED) {
+        for (i64 j = tid; j < nrows * n; j += blockDim.x) {
+            const int row = (int)(j / n), i = (int)(j - (i64)row * n);
+            sm[(i64)row * S * w.P + (i / w.Ls) * w.P + i % w.Ls] = in[f0 * n + j];
+        }
+        __syncthreads();
+        dst = sm + (i64)fl * S * w.P + (i64)(seg * w.P) - lo;
+        src = dst;
+        step = 1;
+    } else {
+        const i64 outer = f / w.inner, j = f - outer * w.inner, base = outer * n * w.inner + j;
+        src = in + base;
+        dst = out + base;
+        step = w.inner;
+    }
+    auto idx = [&](int s2) { return STAGED ? fl * S + s2 : s2 * FB + fl; };
+
+    // 1. forward map of the segment, y_{hi-1} = A y_{lo-1} + B
+    double A = 1.0, B = 0.0, c = 0.0;
+    if (S > 1) {
+        if (act)
+            for (int i = lo; i < hi; ++i) { B = fma(-l[i], B, src[i * step]); A *= -l[i]; }
+        sa[tid] = A; sb[tid] = B;
+        __syncthreads();
+        for (int s2 = 0; s2 < seg; ++s2) c = fma(sa[idx(s2)], c, sb[idx(s2)]);
+        __syncthreads();
+    }
+    // 2. forward recurrence from y_{lo-1} = c; backward map z_lo = A z_hi + B composed along the way
+    //    (z_i = a_i z_{i+1} + b_i with a_i = -off_i / d'_i, b_i = y_i / d'_i)
+    A = 1.0; B = 0.0;
+    if (act)
+        for (int i = lo; i < hi; ++i) {
+            c = fma(-l[i], c, src[i * step]);
+            dst[i * step] = c;
+            B = fma(A, c * invd[i], B);
+            A *= -off[i] * invd[i];
+        }
+    // 3. backward recurrence from z_hi
+    c = 0.0;
+    if (S > 1) {
+        sa[tid] = A; sb[tid] = B;
+        __syncthreads();
+        for (int s2 = S - 1; s2 > seg; --s2) c = fma(sa[idx(s2)], c, sb[idx(s2)]);
+    }
+    if (act)
+        for (int i = hi - 1; i >= lo; --i) {
+            c = fma(-off[i], c, dst[i * step]) * invd[i];
+            dst[i * step] = c;
+        }
+    if (STAGED) {
+        double rz = 0.0;
+        __syncthreads();
+        for (i64 j = tid; j < nrows * n; j += blockDim.x) {
+            const int row = (int)(j / n), i = (int)(j - (i64)row * n);
+            const double v = sm[(i64)row * S * w.P + (i / w.Ls) * w.P + i % w.Ls];
+            out[f0 * n + j] = v;
+            if (RZ) rz = fma(r[f0 * n + j], v, rz);
+        }
+        if (RZ) {
+            rz = block_sum(rz, red);
+            if (tid == 0) atomicAdd(&st->rz_acc, rz);
+        }
+    }
+}
+
+// x = x0, r = b / noise - A x0; ||b / noise||^2 and r.r into the (zeroed) status.  r.z comes from the first application.
+template <typename X, int D>
+__global__ void __launch_bounds__(256) k_mo_kron_init(const __grid_constant__ MoSys<D> s, const double* __restrict__ b,
+                                                      const X* __restrict__ x0, double* __restrict__ x,
+                                                      double* __restrict__ r, MoStatus* st) {
+    __shared__ double red[32];
+    const double inv_noise = 1.0 / s.theta[2 * D];
+    double bb = 0.0, rr = 0.0;
+    for (i64 u = (i64)blockIdx.x * blockDim.x + threadIdx.x; u < s.M; u += (i64)gridDim.x * blockDim.x) {
+        const double ax = mo_row<D, true, X>(s, u, x0, inv_noise, nullptr);
+        const double rhs = b[u] * inv_noise, ri = rhs - ax;
+        x[u] = (double)x0[u];
+        r[u] = ri;
+        bb = fma(rhs, rhs, bb);
+        rr = fma(ri, ri, rr);
+    }
+    bb = block_sum(bb, red);
+    rr = block_sum(rr, red);
+    if (threadIdx.x == 0) { atomicAdd(&st->bb, bb); atomicAdd(&st->rr_acc, rr); }
+}
+
+__global__ void __launch_bounds__(256) k_mo_kron_update(i64 M, const double* __restrict__ p, const double* __restrict__ q,
+                                                        double* __restrict__ x, double* __restrict__ r, MoStatus* st) {
+    __shared__ double red[32];
+    if (st->done) return;
+    const double alpha = st->rz / st->pq;
+    double rr = 0.0;
+    for (i64 u = (i64)blockIdx.x * blockDim.x + threadIdx.x; u < M; u += (i64)gridDim.x * blockDim.x) {
+        x[u] = fma(alpha, p[u], x[u]);
+        const double ri = fma(-alpha, q[u], r[u]);
+        r[u] = ri;
+        rr = fma(ri, ri, rr);
+    }
+    rr = block_sum(rr, red);
+    if (threadIdx.x == 0) atomicAdd(&st->rr_acc, rr);
+}
+
+// as k_mo_direction with p = z + beta p
+__global__ void __launch_bounds__(256) k_mo_kron_direction(i64 M, const double* __restrict__ z, double* __restrict__ p,
+                                                           double rtol, MoStatus* st) {
+    if (st->done) return;
+    const double relres = sqrt(st->rr_acc / st->bb);
+    const bool conv = !(relres > rtol);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        st->pq = 0.0;
+        st->iters += 1;
+        st->relres = relres;
+        if (conv) st->done = 1;
+    }
+    if (conv) return;
+    const double beta = st->rz_acc / st->rz;
+    for (i64 u = (i64)blockIdx.x * blockDim.x + threadIdx.x; u < M; u += (i64)gridDim.x * blockDim.x)
+        p[u] = fma(beta, p[u], z[u]);
+}
+
 }  // namespace vggp
 #endif

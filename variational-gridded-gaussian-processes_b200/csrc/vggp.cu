@@ -145,6 +145,8 @@ struct vggp_plan {
     // optimal variational mean (meanopt.cuh): G, b, the CG vectors, the B1 prior bands and the CG status in one buffer,
     // allocated at the first vggp_meanopt_assemble (scratch_bytes of vggp_workspace_bytes)
     void* mo_buf = nullptr; size_t mo_bytes = 0; bool mo_assembled = false;
+    // the Kronecker-preconditioned solve's z vector, Thomas factors and trace, allocated at its first call (scratch_bytes)
+    void* mo_kbuf = nullptr; size_t mo_kbytes = 0;
     void* band_rep = nullptr;              // B1 family, binned kernel: BAND_REPLICAS copies of the band block (obs dtype), kept zero
                                            // between launches (k_band_reduce clears what it sums)
     // schedules
@@ -2111,6 +2113,89 @@ MoLayout mo_layout(const vggp_plan* p) {
     return L;
 }
 
+// Kronecker buffer: z [M] | Thomas factors [3 sum M_d] | MoKron
+struct MoKronLayout {
+    double *z, *fac;
+    MoKron* k;
+    int fac_off[VGGP_MAX_D];
+    size_t bytes;
+};
+
+MoKronLayout mo_kron_layout(const vggp_plan* p) {
+    MoKronLayout K;
+    double* base = reinterpret_cast<double*>(p->mo_kbuf);
+    i64 nf = 0;
+    for (int d = 0; d < p->D; ++d) { K.fac_off[d] = (int)nf; nf += 3 * (i64)p->n[d]; }
+    K.z = base;
+    K.fac = K.z + p->M;
+    K.k = reinterpret_cast<MoKron*>(K.fac + nf);
+    K.bytes = (size_t)(p->M + nf) * sizeof(double) + sizeof(MoKron);
+    return K;
+}
+
+constexpr int MO_SWEEP_SMEM = 32000;    // dynamic shared memory of a staged sweep; with its 16.6 KB static arrays <= 48 KB
+// a row of the longest mesh, cut into 32 segments, fits: the contiguous mode is always staged
+static_assert(32 * ((((NB * MAX_LEAVES) + 31) / 32) | 1) * sizeof(double) <= (size_t)MO_SWEEP_SMEM,
+              "a row of the longest mesh must fit the staged sweep");
+
+// launch shape of the tridiagonal sweep along mode d: S segments per fibre (a power of two <= 32, chosen so that the
+// fibres x segments fill the GPU while segments keep >= 4 nodes).  The contiguous mode (d = D - 1) is staged through shared
+// memory in tiles of whole rows, at least 32 / S rows per CTA; where such a tile exceeds MO_SWEEP_SMEM, S doubles (shorter
+// padded segments, fewer rows) until it fits, which S = 32 always does (static_assert above).
+struct MoSweepCfg {
+    MoSweep w;
+    unsigned blocks, threads;
+    size_t smem;
+};
+
+MoSweepCfg mo_sweep_cfg(const vggp_plan* p, const MoKronLayout& K, int d) {
+    MoSweepCfg c;
+    MoSweep& w = c.w;
+    w.n = p->n[d];
+    w.inner = p->stride[d];
+    w.F = p->M / w.n;
+    w.fac = K.fac + K.fac_off[d];
+    const i64 target = (i64)p->sm_count * 1024;
+    int S = 1;
+    while (S < 32 && w.F * S < target && (w.n + 2 * S - 1) / (2 * S) >= 4) S *= 2;
+    const bool staged = d == p->D - 1;
+    if (staged) {
+        for (;; S *= 2) {
+            const int P = ((w.n + S - 1) / S) | 1;
+            if (S == 32 || (size_t)32 * P * sizeof(double) <= (size_t)MO_SWEEP_SMEM) break;
+        }
+    }
+    w.S = S;
+    w.Ls = (w.n + S - 1) / S;
+    w.P = w.Ls | 1;
+    if (staged) {
+        const size_t row = (size_t)S * w.P * sizeof(double);
+        int rows = 256 / S;
+        while (rows > 32 / S && rows * row > (size_t)MO_SWEEP_SMEM) rows /= 2;
+        c.threads = (unsigned)(rows * S);
+        c.smem = rows * row;
+        c.blocks = (unsigned)((w.F + rows - 1) / rows);
+    } else {
+        c.threads = (unsigned)(32 * S);
+        c.smem = 0;
+        c.blocks = (unsigned)((w.F + 31) / 32);
+    }
+    return c;
+}
+
+// z = kron_d (F_d + g I)^-1 r, one sweep per mode (the first reads r, the others work in place on z); adds r.z to rz_acc
+int mo_kron_apply(const vggp_plan* p, const MoKronLayout& K, const double* r, double* z, MoStatus* mst, cudaStream_t st) {
+    for (int d = 0; d < p->D; ++d) {
+        const MoSweepCfg c = mo_sweep_cfg(p, K, d);
+        const double* in = d == 0 ? r : z;
+        const bool last = d == p->D - 1;
+        if (last) k_mo_kron_sweep<true, true><<<c.blocks, c.threads, c.smem, st>>>(c.w, in, z, r, mst);
+        else k_mo_kron_sweep<false, false><<<c.blocks, c.threads, 0, st>>>(c.w, in, z, r, mst);
+        VGGP_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
 template <typename T, int D>
 int mo_assemble_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, cudaStream_t st) {
     const MoLayout L = mo_layout(p);
@@ -2160,9 +2245,16 @@ int mo_assemble_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void*
 
 constexpr int MO_BATCH = 64;        // CG iterations launched between two reads of the status record
 
+// precond: VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER (the Jacobi launches are those of the solve before the choice)
 template <int D>
-int mo_solve_impl(vggp_plan* p, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
+int mo_solve_impl(vggp_plan* p, int precond, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
                   cudaStream_t st) {
+    const bool kron = precond == VGGP_MEANOPT_KRONECKER;
+    if (kron && !p->mo_kbuf) {
+        const size_t want = mo_kron_layout(p).bytes;
+        VGGP_CUDA(cudaMalloc(&p->mo_kbuf, want));
+        p->mo_kbytes = want;
+    }
     const MoLayout L = mo_layout(p);
     const bool b1 = p->family == VGGP_B1_ASVGP;
     MoSys<D> s;
@@ -2187,12 +2279,32 @@ int mo_solve_impl(vggp_plan* p, double rtol, int max_iter, double* m_out, int* i
         VGGP_LAUNCH_CHECK();
     }
     VGGP_CUDA(cudaMemsetAsync(L.st, 0, sizeof(MoStatus), st));
-    // initial guess: the state of the last grid forward (B1: alpha = Kuu^-1 m in float64; Markov: m as the kernels read it)
-    if (b1) k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, p->alpha, L.x, L.r, L.p, L.dinv, L.st);
-    else if (p->obs_dtype == VGGP_F32)
-        k_mo_init<float, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const float*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
-    else k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const double*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
-    VGGP_LAUNCH_CHECK();
+    MoKronLayout K{};
+    if (kron) {
+        K = mo_kron_layout(p);
+        MoFacOff<D> fo;
+        for (int d = 0; d < D; ++d) fo.off[d] = K.fac_off[d];
+        VGGP_CUDA(cudaMemsetAsync(K.k, 0, sizeof(MoKron), st));
+        k_mo_kron_trace<<<blocks, 256, 0, st>>>(p->M, L.G, K.k);
+        VGGP_LAUNCH_CHECK();
+        k_mo_kron_factors<D><<<1, 32, 0, st>>>(s, K.k, K.fac, fo);
+        VGGP_LAUNCH_CHECK();
+        // initial guess as below; z0 = P r0 adds r0.z0 to rz_acc, p0 = z0
+        if (b1) k_mo_kron_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, p->alpha, L.x, L.r, L.st);
+        else if (p->obs_dtype == VGGP_F32)
+            k_mo_kron_init<float, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const float*>(p->alphaT), L.x, L.r, L.st);
+        else k_mo_kron_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const double*>(p->alphaT), L.x, L.r, L.st);
+        VGGP_LAUNCH_CHECK();
+        if (int rc = mo_kron_apply(p, K, L.r, K.z, L.st, st)) return rc;
+        VGGP_CUDA(cudaMemcpyAsync(L.p, K.z, sizeof(double) * (size_t)p->M, cudaMemcpyDeviceToDevice, st));
+    } else {
+        // initial guess: the state of the last grid forward (B1: alpha = Kuu^-1 m in float64; Markov: m as the kernels read it)
+        if (b1) k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, p->alpha, L.x, L.r, L.p, L.dinv, L.st);
+        else if (p->obs_dtype == VGGP_F32)
+            k_mo_init<float, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const float*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
+        else k_mo_init<double, D><<<blocks, 256, 0, st>>>(s, L.b, reinterpret_cast<const double*>(p->alphaT), L.x, L.r, L.p, L.dinv, L.st);
+        VGGP_LAUNCH_CHECK();
+    }
     MoStatus h;
     VGGP_CUDA(cudaMemcpyAsync(&h, L.st, sizeof(MoStatus), cudaMemcpyDeviceToHost, st));
     VGGP_CUDA(cudaStreamSynchronize(st));
@@ -2210,10 +2322,18 @@ int mo_solve_impl(vggp_plan* p, double rtol, int max_iter, double* m_out, int* i
         for (int k = 0; k < nb; ++k) {
             k_mo_matvec<D><<<blocks, 256, 0, st>>>(s, L.p, L.q, L.st);
             VGGP_LAUNCH_CHECK();
-            k_mo_update<<<blocks, 256, 0, st>>>(p->M, L.p, L.q, L.dinv, L.x, L.r, L.st);
-            VGGP_LAUNCH_CHECK();
-            k_mo_direction<<<blocks, 256, 0, st>>>(p->M, L.r, L.dinv, L.p, rtol, L.st);
-            VGGP_LAUNCH_CHECK();
+            if (kron) {
+                k_mo_kron_update<<<blocks, 256, 0, st>>>(p->M, L.p, L.q, L.x, L.r, L.st);
+                VGGP_LAUNCH_CHECK();
+                if (int rc = mo_kron_apply(p, K, L.r, K.z, L.st, st)) return rc;
+                k_mo_kron_direction<<<blocks, 256, 0, st>>>(p->M, K.z, L.p, rtol, L.st);
+                VGGP_LAUNCH_CHECK();
+            } else {
+                k_mo_update<<<blocks, 256, 0, st>>>(p->M, L.p, L.q, L.dinv, L.x, L.r, L.st);
+                VGGP_LAUNCH_CHECK();
+                k_mo_direction<<<blocks, 256, 0, st>>>(p->M, L.r, L.dinv, L.p, rtol, L.st);
+                VGGP_LAUNCH_CHECK();
+            }
         }
         VGGP_CUDA(cudaMemcpyAsync(&h, L.st, sizeof(MoStatus), cudaMemcpyDeviceToHost, st));
         VGGP_CUDA(cudaStreamSynchronize(st));
@@ -2257,7 +2377,7 @@ int vggp_workspace_bytes(const vggp_plan* p, int64_t* plan_bytes, int64_t* gbuf_
     if (gbuf_bytes) *gbuf_bytes = total;
     if (scratch_bytes) {
         const size_t tsz = p->obs_dtype == VGGP_F32 ? 4 : 8;
-        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes;
+        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes + p->mo_kbytes;
         if (p->st_x) sc += (size_t)p->st_n * tsz * (p->D + 1) + sizeof(double) * (2 * (size_t)p->M + 2 * (size_t)p->Lsize) + (size_t)total;
         *scratch_bytes = (int64_t)sc;
     }
@@ -2498,6 +2618,7 @@ int vggp_plan_destroy(vggp_plan* p) {
     if (p->one_ws) cudaFree(p->one_ws);
     if (p->det_fp) cudaFree(p->det_fp);
     if (p->mo_buf) cudaFree(p->mo_buf);
+    if (p->mo_kbuf) cudaFree(p->mo_kbuf);
     for (auto& e : p->k1_ev) cudaEventDestroy(e);
     for (auto& e : p->k1_gev) if (e) cudaEventDestroy(e);
     for (auto& e : p->st_ev) cudaEventDestroy(e);
@@ -3103,17 +3224,24 @@ int vggp_meanopt_assemble(vggp_plan* p, const vggp_binned_desc* desc, const void
 
 int vggp_meanopt_solve(vggp_plan* p, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
                        void* stream) {
+    return vggp_meanopt_solve_pc(p, VGGP_MEANOPT_JACOBI, rtol, max_iter, m_out, iters_host, relres_host, stream);
+}
+
+int vggp_meanopt_solve_pc(vggp_plan* p, int precond, double rtol, int max_iter, double* m_out, int* iters_host,
+                          double* relres_host, void* stream) {
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !m_out || !iters_host || !relres_host) return fail(VGGP_E_ARG, "null argument");
     if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
         return fail(VGGP_E_UNSUPPORTED, "the optimal mean is built for the B1 and VGGP_SVGP_MARKOV families (3^D-stencil system)");
     if (!(rtol >= 0.0) || max_iter < 0) return fail(VGGP_E_ARG, "rtol must be >= 0 and max_iter >= 0");
+    if (precond != VGGP_MEANOPT_JACOBI && precond != VGGP_MEANOPT_KRONECKER)
+        return fail(VGGP_E_ARG, "precond must be VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER");
     if (!p->mo_assembled) return fail(VGGP_E_ARG, "vggp_meanopt_solve needs a previous vggp_meanopt_assemble on this plan");
     cudaStream_t st = (cudaStream_t)stream;
     switch (p->D) {
-        case 1: return mo_solve_impl<1>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
-        case 2: return mo_solve_impl<2>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
-        default: return mo_solve_impl<3>(p, rtol, max_iter, m_out, iters_host, relres_host, st);
+        case 1: return mo_solve_impl<1>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
+        case 2: return mo_solve_impl<2>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
+        default: return mo_solve_impl<3>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
     }
 }
 

@@ -202,17 +202,25 @@ class GriddedVariationalGP(nn.Module):
     MEANOPT_MAX_ITER = 20000
 
     @torch.no_grad()
-    def set_optimal_mean(self, rtol: float = 1e-10, max_iter: Optional[int] = None) -> dict:
+    def set_optimal_mean(self, rtol: float = 1e-10, max_iter: Optional[int] = None, preconditioner: str = "jacobi") -> dict:
         """Load the optimal variational mean at the current hyper-parameters into `variational_mean`: the m that maximises
         the ELBO for fixed theta and S, which is the mean of the reference's q_u() (m* = Kuu Sigma^-1 Kuf y / noise), at any
-        grid size.  One pass over the binned observations assembles a 3^D-stencil system, Jacobi-preconditioned conjugate
+        grid size.  One pass over the binned observations assembles a 3^D-stencil system, preconditioned conjugate
         gradients solve it from the current mean (include/vggp.h, vggp_meanopt_*).  B1 and Markov SVGP families.
-        `max_iter` defaults to MEANOPT_MAX_ITER = 20000.  Measured on one B200 to rtol 1e-8 from m = 0 (float32 track
-        observations, profiles/optimal_mean/): 512 x 512 points, 2^26 observations: B1 678, Markov 59 iterations; 2^22
-        observations: B1 3054, Markov 283; 64 x 64 x 16 points, 2^20 observations: Markov 16046, B1 not converged after
-        60000 (Jacobi preconditioning is too weak for the 3-D B1 prior, DESIGN.md section 7).
-        Returns {"iterations", "relres"}; raises RuntimeError, leaving `variational_mean` unchanged, if the solve stops
-        above `rtol`."""
+        `max_iter` defaults to MEANOPT_MAX_ITER = 20000.  `preconditioner`:
+          "jacobi"     (default) measured on one B200 to rtol 1e-8 from m = 0 (float32 track observations,
+                       profiles/optimal_mean/): 512 x 512 points, 2^26 observations: B1 678, Markov 59 iterations; 2^22
+                       observations: B1 3054, Markov 283; 64 x 64 x 16 points, 2^20 observations: Markov 16046, B1 not
+                       converged after 60000.
+          "kronecker"  kron_d (F_d + g I)^-1 of the per-dimension prior factors, applied exactly by D tridiagonal sweeps;
+                       it converges on 3-D B1 grids.  Same data on one B200 (profiles/optimal_mean_kron/):
+                       512 x 512 points, 2^26 observations: B1 100 iterations (7.1 ms, Jacobi 15.8 ms), Markov 37 (3.1 ms,
+                       Jacobi 1.4 ms); 256 x 256 x 64 points: B1 7855 iterations (6.0 s), Markov relres 2.1e-7 after 20000.
+                       Float64 oracle counts with 2^22 / 2^20 observations: 512 x 512 B1 196, Markov 66; 64 x 64 x 16 B1 990.
+        Any other value raises ValueError.  Returns {"iterations", "relres"}; raises RuntimeError, leaving
+        `variational_mean` unchanged, if the solve stops above `rtol`."""
+        if preconditioner not in ("jacobi", "kronecker"):
+            raise ValueError(f"preconditioner must be 'jacobi' or 'kronecker', not {preconditioner!r}")
         if self.family not in (_lib.B1_ASVGP, _lib.SVGP_MARKOV):
             raise NotImplementedError("set_optimal_mean() needs the 3^D-stencil system of the B1 and Markov SVGP families; "
                                       "for this family use set_optimal_q() (dense, M <= 4096)")
@@ -231,7 +239,7 @@ class GriddedVariationalGP(nn.Module):
         if self.family != _lib.B1_ASVGP or getattr(plan, "_mo_obs", None) is not self._obs:
             plan.meanopt_assemble(binned)
             plan._mo_obs = self._obs if self.family == _lib.B1_ASVGP else None
-        m, iters, relres = plan.meanopt_solve(rtol, self.MEANOPT_MAX_ITER if max_iter is None else max_iter)
+        m, iters, relres = plan.meanopt_solve(rtol, self.MEANOPT_MAX_ITER if max_iter is None else max_iter, preconditioner)
         if not relres <= rtol:
             raise RuntimeError(f"set_optimal_mean(): conjugate gradients stopped after {iters} iterations at relative residual "
                                f"{relres:.3e} > rtol = {rtol:.1e}; variational_mean is unchanged")

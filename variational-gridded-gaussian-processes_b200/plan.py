@@ -126,14 +126,20 @@ class GridPlan:
         _lib.check(self.lib.vggp_meanopt_assemble(self.handle, C.byref(binned.desc), binned.buf.data_ptr(),
                                                   _stream_ptr(self.device)))
 
-    def meanopt_solve(self, rtol: float, max_iter: int):
-        """Conjugate gradients on the assembled system from the state of the last grid_forward (vggp_meanopt_solve;
-        synchronises).  Returns (m_star float64 [M], iterations, final relative residual); not converged when
-        relres > rtol."""
+    MEANOPT_PRECONDITIONERS = {"jacobi": _lib.MEANOPT_JACOBI, "kronecker": _lib.MEANOPT_KRONECKER}
+
+    def meanopt_solve(self, rtol: float, max_iter: int, preconditioner: str = "jacobi"):
+        """Conjugate gradients on the assembled system from the state of the last grid_forward (vggp_meanopt_solve_pc;
+        synchronises).  `preconditioner`: "jacobi" (vggp_meanopt_solve) or "kronecker" (kron_d (F_d + g I)^-1 of the
+        per-dimension prior factors, applied exactly by tridiagonal sweeps).  Returns (m_star float64 [M], iterations,
+        final relative residual); not converged when relres > rtol."""
+        if preconditioner not in self.MEANOPT_PRECONDITIONERS:
+            raise ValueError(f"preconditioner must be one of {sorted(self.MEANOPT_PRECONDITIONERS)}, not {preconditioner!r}")
         m = torch.empty(self.M, dtype=torch.float64, device=self.device)
         it, rr = C.c_int(0), C.c_double(0.0)
-        _lib.check(self.lib.vggp_meanopt_solve(self.handle, float(rtol), int(max_iter), m.data_ptr(), C.byref(it),
-                                               C.byref(rr), _stream_ptr(self.device)))
+        _lib.check(self.lib.vggp_meanopt_solve_pc(self.handle, self.MEANOPT_PRECONDITIONERS[preconditioner], float(rtol),
+                                                  int(max_iter), m.data_ptr(), C.byref(it), C.byref(rr),
+                                                  _stream_ptr(self.device)))
         return m, int(it.value), float(rr.value)
 
     def predict(self, xs: Sequence[torch.Tensor]):
