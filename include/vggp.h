@@ -79,7 +79,7 @@ extern "C" {
 typedef struct vggp_plan vggp_plan;
 
 /* ABI version of this header; vggp_abi_version() must return the same value. */
-#define VGGP_ABI_VERSION 1
+#define VGGP_ABI_VERSION 2
 int vggp_abi_version(void);
 const char* vggp_last_error(void);
 /* Number of CUDA kernels this library has launched so far in this process (host-side counter). */
@@ -328,6 +328,30 @@ int vggp_meanopt_solve(vggp_plan* plan, double rtol, int max_iter, double* m_out
                        int* iters_host, double* relres_host, void* stream);
 int vggp_meanopt_solve_pc(vggp_plan* plan, int precond, double rtol, int max_iter, double* m_out,
                           int* iters_host, double* relres_host, void* stream);
+
+/* ---- optimal variational covariance within the Kronecker family (B1 and VGGP_SVGP_MARKOV) ------------------
+ * One coordinate update of S_d = tril(L_d) tril(L_d)^T: with theta, m and every S_e, e != d, fixed, the ELBO is strictly
+ * concave in S_d and maximised by S_d = (M / M_d) A_d^-1 (csrc/covopt.cuh, DESIGN.md section 4, K1s):
+ *     T_d = (ell_scale / noise) H_d + c_d F_d,   H_d = sum_n (prod_{e != d} q_e(x_n)) w_d w_d^T,   c_d = prod_{e != d} tr(K_e^-1 S_e)
+ *     VGGP_SVGP_MARKOV:  F_d = K_d^-1,  S_d = (M / M_d) T_d^-1;     B1:  F_d = K_d,  S_d = (M / M_d) K_d T_d^-1 K_d
+ * Cycling d = 0..D-1 is coordinate ascent on the ELBO; with set_optimal_mean's m* it gives the ELBO-optimal q(u) of the
+ * Kronecker family.  For D = 1 one update is the reference's S* = Kuu Sigma^-1 Kuu.
+ *   vggp_covopt_update  reads `L` (DEVICE, float64, the concatenated [M_1^2 | M_2^2 | ...] blocks given to the last
+ *                       vggp_grid_forward) and writes block `dim` of `L_out` (same layout; the other blocks are untouched;
+ *                       `L_out` may alias `L`) with the lower-triangular Cholesky factor of the new S_d (positive diagonal,
+ *                       strict upper triangle 0).  `gbuf` must be the gradient buffer of a step taken at exactly that
+ *                       forward (vggp_obs_fwd_bwd_binned or another per-observation call after it), already all-reduced
+ *                       when the observations are sharded; only its band block of dimension `dim` is read.  Adds
+ *                       ||L_new / ||L_new||_F - L_old / ||L_old||_F||_F (lower triangles) to the DEVICE float64 scalar
+ *                       `change`; the measure does not see the flat direction S_1 -> a S_1, S_2 -> S_2 / a of the family.
+ *                       A pivot of T_d that is not positive and finite sets the flag of vggp_read_info to dim + 1, leaves
+ *                       `L_out` untouched and adds +inf to `change`.  Asynchronous, no host synchronisation; the first call
+ *                       allocates 6 max M_d + 8 float64 (counted in scratch_bytes) and must not be captured, later calls
+ *                       may be.  VGGP_E_UNSUPPORTED for the B0, SVGP_GRID and VFF families and for M_d > 2560; VGGP_E_ARG
+ *                       for a bad `dim`, a null pointer, or no previous vggp_grid_forward on the plan.
+ */
+int vggp_covopt_update(vggp_plan* plan, int dim, const void* gbuf, double ell_scale, const double* L, double* L_out,
+                       double* change, void* stream);
 
 /* ---- feature evaluation (bit-exact restatement of the reference's basis calls) ------------------------- */
 

@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(HERE, "libvggp.so")
 B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID, SVGP_MARKOV = 0, 1, 2, 3, 4
 F32, F64 = 0, 1
 MEANOPT_JACOBI, MEANOPT_KRONECKER = 0, 1
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 WS_K, WS_P, WS_R, WS_Q, WS_S, WS_ALPHA, WS_SCAL, WS_KRAW, WS_QBAND = range(9)
 
@@ -71,6 +71,7 @@ SIGNATURES = {
     "vggp_meanopt_solve": (C.c_int, [_vp, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), C.POINTER(C.c_double), _vp]),
     "vggp_meanopt_solve_pc": (C.c_int, [_vp, C.c_int, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), C.POINTER(C.c_double),
                                         _vp]),
+    "vggp_covopt_update": (C.c_int, [_vp, C.c_int, _dp, C.c_double, _dp, _dp, _dp, _vp]),
     "vggp_b1_stencil": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _dp, _vp]),
     "vggp_features_dense": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _vp]),
     "vggp_workspace_ptr": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(_vp), C.POINTER(_i64)]),

@@ -18,6 +18,7 @@
 #include "b0scan.cuh"
 #include "svgpm.cuh"
 #include "meanopt.cuh"
+#include "covopt.cuh"
 #include "collective.cuh"
 
 // Every plan-taking entry point runs with the plan's device current and restores the caller's device on return
@@ -147,6 +148,10 @@ struct vggp_plan {
     void* mo_buf = nullptr; size_t mo_bytes = 0; bool mo_assembled = false;
     // the Kronecker-preconditioned solve's z vector, Thomas factors and trace, allocated at its first call (scratch_bytes)
     void* mo_kbuf = nullptr; size_t mo_kbytes = 0;
+    // optimal covariance (covopt.cuh): F band, U^-T recurrence, B1 X diagonals, change sums; allocated at the first
+    // vggp_covopt_update (scratch_bytes)
+    void* co_buf = nullptr; size_t co_bytes = 0;
+    bool forwarded = false;                // a vggp_grid_forward has run on this plan
     void* band_rep = nullptr;              // B1 family, binned kernel: BAND_REPLICAS copies of the band block (obs dtype), kept zero
                                            // between launches (k_band_reduce clears what it sums)
     // schedules
@@ -2243,6 +2248,39 @@ int mo_assemble_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void*
     VGGP_DISPATCH_TD(p, mo_assemble_impl, p, desc, binned, st);
 }
 
+// ---- optimal covariance (covopt.cuh) -------------------------------------------------------------------------
+template <typename T>
+int covopt_impl(vggp_plan* p, int dim, const void* gbuf, double ell_scale, const double* L, double* L_out, double* change,
+                cudaStream_t st) {
+    const int n = p->n[dim];
+    double* base = reinterpret_cast<double*>(p->co_buf);
+    CoArgs a;
+    a.n = n; a.d = dim; a.D = p->D; a.family = p->family;
+    a.scale = sqrt((double)p->M / (double)n);
+    a.fd = base; a.fo = base + n; a.ib = base + 2 * n; a.rr = base + 3 * n; a.xd = base + 4 * n; a.xs = base + 5 * n;
+    a.acc = base + 6 * n;
+    a.Lold = L + p->g.Loff[dim];
+    a.Lout = L_out + p->g.Loff[dim];
+    const bool b1 = p->family == VGGP_B1_ASVGP;
+    const T* band = reinterpret_cast<const T*>(gbuf) + p->M + p->band_off[dim];
+    const double* trs = b1 ? p->g.sc + SC_TR : p->svm_sc + SVS_TR;
+    k_co_factor<T><<<1, CO_THREADS, 0, st>>>(a, p->g, b1 ? nullptr : p->svm_W[dim], band, p->theta_dev, trs, ell_scale,
+                                             p->g.info);
+    VGGP_LAUNCH_CHECK();
+    const unsigned cols = (unsigned)ceil_div(n, CO_THREADS);
+    if (b1) {
+        k_co_b1_x<<<cols, CO_THREADS, 0, st>>>(a);
+        VGGP_LAUNCH_CHECK();
+        k_co_b1_rq<<<1, CO_THREADS, 0, st>>>(a);
+    } else {
+        k_co_markov<<<cols, CO_THREADS, 0, st>>>(a);
+    }
+    VGGP_LAUNCH_CHECK();
+    k_co_change<<<1, 32, 0, st>>>(a.acc, change);
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+
 constexpr int MO_BATCH = 64;        // CG iterations launched between two reads of the status record
 
 // precond: VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER (the Jacobi launches are those of the solve before the choice)
@@ -2377,7 +2415,7 @@ int vggp_workspace_bytes(const vggp_plan* p, int64_t* plan_bytes, int64_t* gbuf_
     if (gbuf_bytes) *gbuf_bytes = total;
     if (scratch_bytes) {
         const size_t tsz = p->obs_dtype == VGGP_F32 ? 4 : 8;
-        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes + p->mo_kbytes;
+        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes + p->mo_kbytes + p->co_bytes;
         if (p->st_x) sc += (size_t)p->st_n * tsz * (p->D + 1) + sizeof(double) * (2 * (size_t)p->M + 2 * (size_t)p->Lsize) + (size_t)total;
         *scratch_bytes = (int64_t)sc;
     }
@@ -2619,6 +2657,7 @@ int vggp_plan_destroy(vggp_plan* p) {
     if (p->det_fp) cudaFree(p->det_fp);
     if (p->mo_buf) cudaFree(p->mo_buf);
     if (p->mo_kbuf) cudaFree(p->mo_kbuf);
+    if (p->co_buf) cudaFree(p->co_buf);
     for (auto& e : p->k1_ev) cudaEventDestroy(e);
     for (auto& e : p->k1_gev) if (e) cudaEventDestroy(e);
     for (auto& e : p->st_ev) cudaEventDestroy(e);
@@ -2659,6 +2698,7 @@ int vggp_grid_forward(vggp_plan* p, const double* theta, const double* m, const 
     const int D = p->D;
     int rc;
     p->last_stream = st;
+    p->forwarded = true;
     if (p->family == VGGP_SVGP_MARKOV) return svgpm_forward(p, theta, m, L, st);
     if (p->g.structured == 3) return b1f_forward(p, theta, m, L, st);
     VGGP_CUDA(cudaMemcpyAsync(p->mws, m, sizeof(double) * p->M, cudaMemcpyDeviceToDevice, st));
@@ -3243,6 +3283,29 @@ int vggp_meanopt_solve_pc(vggp_plan* p, int precond, double rtol, int max_iter, 
         case 2: return mo_solve_impl<2>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
         default: return mo_solve_impl<3>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
     }
+}
+
+int vggp_covopt_update(vggp_plan* p, int dim, const void* gbuf, double ell_scale, const double* L, double* L_out,
+                       double* change, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !gbuf || !L || !L_out || !change) return fail(VGGP_E_ARG, "null argument");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the optimal covariance is built for the B1 and VGGP_SVGP_MARKOV families (tridiagonal "
+                                        "T_d); the dense families have the reference's dense q_u()");
+    if (dim < 0 || dim >= p->D) return fail(VGGP_E_ARG, "bad dim");
+    if (!p->forwarded) return fail(VGGP_E_ARG, "vggp_covopt_update needs a previous vggp_grid_forward on this plan");
+    if (p->n[dim] > CO_MAX_N) return fail(VGGP_E_UNSUPPORTED, "vggp_covopt_update supports M_d <= 2560");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!p->co_buf) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusActive)
+            return fail(VGGP_E_UNSUPPORTED, "the first vggp_covopt_update allocates: call it outside a stream capture");
+        const size_t want = sizeof(double) * (6 * (size_t)p->nmax + 8);
+        VGGP_CUDA(cudaMalloc(&p->co_buf, want));
+        p->co_bytes = want;
+    }
+    if (p->obs_dtype == VGGP_F32) return covopt_impl<float>(p, dim, gbuf, ell_scale, L, L_out, change, st);
+    return covopt_impl<double>(p, dim, gbuf, ell_scale, L, L_out, change, st);
 }
 
 int vggp_metrics(int dtype, const void* truth, const void* pred, int64_t n, double* out, void* stream) {

@@ -230,11 +230,7 @@ class GriddedVariationalGP(nn.Module):
         plan = self._ensure_plan()
         plan.grid_forward(self._theta(), self.variational_mean.detach().to(torch.float64).contiguous(),
                           torch.cat([c.detach().to(torch.float64).reshape(-1) for c in self._chols()]).contiguous())
-        binned = self._packed if isinstance(self._packed, BinnedObs) else None
-        if binned is None:                         # VGGP_OBS_LAYOUT=packed: bin once, for this purpose only
-            if getattr(plan, "_mo_binned", (None,))[0] is not self._obs:
-                plan._mo_binned = (self._obs, plan.bin(*self._obs))
-            binned = plan._mo_binned[1]
+        binned = self._binned_for_optimal_q(plan)
         # the B1 system does not depend on theta: assembled once per plan and data set; the Markov one on every call
         if self.family != _lib.B1_ASVGP or getattr(plan, "_mo_obs", None) is not self._obs:
             plan.meanopt_assemble(binned)
@@ -245,6 +241,75 @@ class GriddedVariationalGP(nn.Module):
                                f"{relres:.3e} > rtol = {rtol:.1e}; variational_mean is unchanged")
         self.variational_mean.copy_(m.to(self.variational_mean.dtype))
         return {"iterations": iters, "relres": relres}
+
+    def _binned_for_optimal_q(self, plan):
+        """The binned layout of the observations (VGGP_OBS_LAYOUT=packed: binned once, for the optimal-q methods only)."""
+        if isinstance(self._packed, BinnedObs):
+            return self._packed
+        if getattr(plan, "_mo_binned", (None,))[0] is not self._obs:
+            plan._mo_binned = (self._obs, plan.bin(*self._obs))
+        return plan._mo_binned[1]
+
+    @torch.no_grad()
+    def set_optimal_covariance(self, rtol: float = 1e-8, max_sweeps: int = 100) -> dict:
+        """Load the ELBO-optimal Kronecker-factored covariance S = kron_d tril(L_d) tril(L_d)^T at the current
+        hyper-parameters and variational mean into the `variational_chol_*` factors, at any grid size.  With everything
+        else fixed the ELBO is strictly concave in one S_d and its maximiser has a closed form built from a tridiagonal matrix
+        (include/vggp.h, vggp_covopt_update; DESIGN.md section 4, K1s); this method cycles d = 0..D-1 (coordinate ascent,
+        the ELBO cannot decrease), each update after a grid forward and one pass over the binned observations, all-reduced
+        over the model's process group when sharded.  It stops after the first sweep whose summed normalised factor change
+        ||L_new / ||L_new|| - L_old / ||L_old||||_F is <= rtol.  B1 and Markov SVGP families.
+
+        The result is the optimum within the Kronecker family, exact for D = 1 (the reference's S* = Kuu Sigma^-1 Kuu).
+        `set_optimal_q()` instead loads the Kronecker product nearest in the Frobenius norm to the unconstrained S* (dense,
+        M <= 4096, D <= 2), which is not the ELBO's optimum in this family for D = 2.  m and S separate in the bound, so
+        `set_optimal_mean()` followed by this method gives the ELBO-optimal q(u) of the family.
+
+        Sweeps to rtol 1e-8 from L_d = I, float64 oracle (Markov features, 4000 - 20000 observations): D = 1 one update,
+        D = 2 11 - 18 sweeps, D = 3 15 - 25 sweeps.  One B200 (1000 W), 2^26 float32 track observations
+        (profiles/optimal_cov/): 512 x 512 points B1 15 sweeps (28 ms), 256 x 256 x 64 B1 19 sweeps (35 ms); the Markov
+        change stalls near 3e-8 (reached after 11 and 17 sweeps): with float32 observations the band sums change in their last
+        bits from one data pass to the next, so use rtol >= 1e-7 there (DESIGN.md section 4, K1s).
+        Returns {"sweeps", "change" (of the last sweep), "elbo" (after the update)}.  Raises RuntimeError after `max_sweeps`
+        sweeps above `rtol`, and torch.linalg.LinAlgError if an update meets a matrix that is not positive definite; both
+        leave the factors as they were."""
+        if self.family not in (_lib.B1_ASVGP, _lib.SVGP_MARKOV):
+            raise NotImplementedError("set_optimal_covariance() needs the tridiagonal update of the B1 and Markov SVGP "
+                                      "families; for this family use set_optimal_q() (dense, M <= 4096)")
+        plan = self._ensure_plan()
+        binned = self._binned_for_optimal_q(plan)
+        group = None if self._group is None or isinstance(self._group, str) else self._group
+        theta = self._theta()
+        m = self.variational_mean.detach().to(torch.float64).contiguous()
+        L = torch.cat([c.detach().to(torch.float64).reshape(-1) for c in self._chols()]).contiguous()
+        change = torch.zeros(1, dtype=torch.float64, device=plan.device)
+        sweeps, last = 0, float("inf")
+        while sweeps < max_sweeps:
+            change.zero_()
+            for d in range(self.D):
+                plan.grid_forward(theta, m, L)
+                plan.obs_fwd_bwd(binned)
+                if self._group is not None:
+                    plan.allreduce_gbuf(group)
+                plan.covopt_update(d, plan.gbuf, 1.0, L, change)
+            sweeps += 1
+            last = float(change.item())
+            if not last < float("inf"):
+                raise torch.linalg.LinAlgError(
+                    "set_optimal_covariance(): an update met a tridiagonal matrix that is not positive definite (is a "
+                    "factor L_d singular?); the variational factors are unchanged")
+            if last <= rtol:
+                break
+        else:
+            raise RuntimeError(f"set_optimal_covariance(): the factor change is {last:.3e} > rtol = {rtol:.1e} after "
+                               f"{sweeps} sweeps; the variational factors are unchanged")
+        out = plan.step(theta, m, L, binned, None, 1.0, self._group)[0]
+        off = 0
+        for c in self._chols():
+            n = c.numel()
+            c.copy_(L[off:off + n].reshape(c.shape).to(c.dtype))
+            off += n
+        return {"sweeps": sweeps, "change": last, "elbo": float(out[0].item())}
 
     # ---- the reference's closed-form (collapsed) quantities: dense M x M algebra, small problems only -------------
     DENSE_LIMIT = 4096          # largest M for which dense M x M matrices are formed (128 MiB in float64)

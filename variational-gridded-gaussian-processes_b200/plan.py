@@ -142,6 +142,19 @@ class GridPlan:
                                                   _stream_ptr(self.device)))
         return m, int(it.value), float(rr.value)
 
+    def covopt_update(self, dim: int, gbuf: torch.Tensor, ell_scale: float, L: torch.Tensor, change: torch.Tensor):
+        """One coordinate update of the optimal Kronecker-factored covariance (vggp_covopt_update; B1 and SVGP_MARKOV):
+        block `dim` of the float64 factors `L` (the L of the last grid_forward) is overwritten in place with the Cholesky
+        factor of the S_dim that maximises the ELBO given the other factors, and the normalised factor change is added to
+        the float64 device scalar `change`.  `gbuf` is the gradient buffer of a step at that forward, all-reduced when
+        sharded.  Asynchronous."""
+        self._check_f64(L, self.L_total, "L")
+        self._check_f64(change, 1, "change")
+        if gbuf.device != self.device or gbuf.numel() < self.gbuf_bytes:
+            raise ValueError("gbuf must be a gradient buffer of this plan")
+        _lib.check(self.lib.vggp_covopt_update(self.handle, int(dim), gbuf.data_ptr(), float(ell_scale), L.data_ptr(),
+                                               L.data_ptr(), change.data_ptr(), _stream_ptr(self.device)))
+
     def predict(self, xs: Sequence[torch.Tensor]):
         """Marginal mean and variance of q(f(x*)) at test points, from the state of the last grid_forward."""
         n = int(xs[0].numel())
