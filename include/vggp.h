@@ -79,7 +79,7 @@ extern "C" {
 typedef struct vggp_plan vggp_plan;
 
 /* ABI version of this header; vggp_abi_version() must return the same value. */
-#define VGGP_ABI_VERSION 2
+#define VGGP_ABI_VERSION 3
 int vggp_abi_version(void);
 const char* vggp_last_error(void);
 /* Number of CUDA kernels this library has launched so far in this process (host-side counter). */
@@ -213,7 +213,7 @@ int vggp_set_binned_stream(int mode);
  * stealing order or the load of the machine.  No floating-point atomic is left on the path: every run of the binned
  * layout writes its flush values as a record and the records are summed in the order of the cell-sorted stream
  * (csrc/obs_binned.cuh); the fibre passes leave per-CTA partials that are summed in tile order (csrc/grid_b1_fast.cuh).
- * Covered: the B1 (ASVGP) family on its default fused grid path with M_d <= 512 and the binned observation layout
+ * Covered: the B1 (ASVGP) family with M_d <= 512 and the binned observation layout
  * (VGGP_E_UNSUPPORTED otherwise, also from vggp_obs_fwd_bwd / _packed while the mode is on).  The scratch is sized at the
  * first deterministic step (cudaMalloc): run one step eagerly before capturing a graph.  Costs a sort of the run list
  * and five small reductions per step; the default (0) is the atomics path.
@@ -415,11 +415,11 @@ int vggp_generate_tracks(int dtype, int D, int64_t n_total, int64_t lo, int64_t 
 
 /* ---- workspace views and primitives (tests, predictions, debugging) ------------------------------------ */
 
-/* Device pointer to a float64 workspace array of the last forward.  which: */
-#define VGGP_WS_K      0   /* Cholesky factor C_d of K_d (lower; upper triangle undefined); dense factor path only */
+/* Device pointer to a float64 workspace array of the last forward (VGGP_E_UNSUPPORTED for the Markov SVGP family).  which: */
+#define VGGP_WS_K      0   /* Cholesky factor C_d of K_d (lower; upper triangle undefined); B0 / SVGP / VFF families only */
 #define VGGP_WS_P      1   /* P_d = K_d^-1 */
 #define VGGP_WS_R      2   /* R_d = P_d tril(L_d) */
-#define VGGP_WS_Q      3   /* Q_d = R_d R_d^T (dense factor path only; the structured path keeps just its band) */
+#define VGGP_WS_Q      3   /* Q_d = R_d R_d^T; B0 / SVGP / VFF families only (the B1 family keeps just its band, VGGP_WS_QBAND) */
 #define VGGP_WS_S      4   /* (retired: S_d is not materialised) */
 #define VGGP_WS_ALPHA  5   /* alpha (M), dim ignored */
 #define VGGP_WS_SCAL   6   /* scalars: logdet K_d [3], logdet S_d [3], tr(P_d S_d) [3], <m,alpha> */
@@ -439,10 +439,6 @@ int vggp_mode_product(vggp_plan* plan, int dim, const double* A, const double* s
 
 /* Select the GEMM inner loop used by the grid-side path: 1 = DMMA tensor cores (default), 0 = SIMT. */
 int vggp_set_gemm_mode(int use_mma);
-
-/* Plans created afterwards for the B1 family use (1, default) the O(M_d^2) twisted-factorisation inverse of the
- * tridiagonal factor, or (0) the same dense blocked Cholesky + triangular inverse the B0 family uses (cross-check). */
-int vggp_set_b1_structured(int on);
 
 #ifdef __cplusplus
 }

@@ -1,8 +1,8 @@
 """The whole C ABI on the CPU under the SIMT emulator (tests/emul_lib.py, tests/host_emul): csrc/vggp.cu with its 45
 kernel launches rewritten, every kernel of csrc/*.cuh compiled unchanged by g++.  The same oracle parity checks the GPU
 suite makes (tests/test_gpu_elbo.py) are made here at small sizes.  Two purposes:
-  * the emulator is validated on the paths that passed on B200 (raw / packed layouts, structured and dense factor paths,
-    DMMA and SIMT GEMMs, B0 family);
+  * the emulator is validated on the paths that passed on B200 (raw / packed layouts, the fused B1 grid side and the
+    dense grid side of the B0 / SVGP / VFF families, DMMA and SIMT GEMMs);
   * the paths that have NOT run on a GPU yet -- the binned layout end to end through vggp_obs_bin_prepare / _pack /
     vggp_obs_fwd_bwd_binned, both streaming variants -- get the same parity check before their first GPU run.
 Test infrastructure only; the product library has no CPU path."""
@@ -153,28 +153,6 @@ def test_two_wave_run_length_under_emulation(emu, layout):
     obs = plan.pack(xs, yy, True) if layout == "packed_sorted" else plan.bin(xs, yy, run_cap=256)
     out, dtheta, dm, dL = plan.step(theta, m.numpy().copy(), Ls[0].reshape(-1).numpy().copy(), obs, None, 1.0)
     check_against_oracle(plan, out, dtheta, dm, dL, elbo_ref, g_ref, N, 1e-3)
-    plan.close()
-
-
-@pytest.mark.parametrize("structured", [0, 1, 2])
-def test_dense_factor_paths_under_emulation(emu, structured):
-    """B1 family through the dense Cholesky + GEMM path (0), the twisted inverse + GEMM products (1) and the round-1
-    semiseparable launches (2): grouped DMMA GEMMs (mma.m8n8k4 and cp.async stand-ins) on the CPU.  Every other test of
-    this file runs the default, the fused fibre passes of csrc/grid_b1.cuh (3)."""
-    lib, L = emu
-    knots, N = (10, 8), 600
-    meshes, X, y, l, s2, noise, m, Ls = make_problem(knots, N, seed=5)
-    elbo_ref, g_ref = oracle_value_and_grads(O.B1_ASVGP, meshes, X, y, l, s2, noise, m, Ls, scale=1.0)
-    lib.vggp_set_b1_structured(structured)
-    try:
-        plan = emul_lib.EmuPlan(lib, L, L.B1_ASVGP, [t.numpy() for t in meshes], np.float64)
-    finally:
-        lib.vggp_set_b1_structured(3)
-    theta = torch.cat([l, s2, noise.reshape(1)]).numpy().copy()
-    xs = [np.ascontiguousarray(X[:, d].numpy()) for d in range(2)]
-    out, dtheta, dm, dL = plan.step(theta, m.numpy().copy(), torch.cat([Lx.reshape(-1) for Lx in Ls]).numpy().copy(),
-                                    xs, y.numpy().copy(), 1.0)
-    check_against_oracle(plan, out, dtheta, dm, dL, elbo_ref, g_ref, N, 1e-9)
     plan.close()
 
 
@@ -661,6 +639,35 @@ def test_workspace_bytes_under_emulation(emu):
         plan.check(lib.vggp_workspace_bytes(plan.h, emul_lib.C.byref(a2), None, emul_lib.C.byref(c2)))
         assert a2.value == a.value and c2.value >= 300 * 4 * 3
         assert lib.vggp_workspace_bytes(None, None, None, None) == -1
+    finally:
+        plan.close()
+
+
+def test_b1_plan_holds_only_the_fused_grid_side_under_emulation(emu):
+    """A B1 plan has no dense factor path: VGGP_WS_K and VGGP_WS_Q are refused (the step never forms the Cholesky factor or
+    the full Q_d), the views the fused grid side does provide stay available, and the plan-owned memory is what the fused
+    grid side, the per-observation kernel and those views use, plus a few scalars."""
+    import ctypes as C
+    lib, L = emu
+    knots = (40, 33)
+    meshes = [np.linspace(0, 1, k, dtype=np.float32) for k in knots]
+    plan = emul_lib.EmuPlan(lib, L, L.B1_ASVGP, meshes, np.float32)
+    try:
+        ptr, n = C.c_void_p(), C.c_int64()
+        for which in (L.WS_K, L.WS_Q):
+            assert lib.vggp_workspace_ptr(plan.h, which, 0, C.byref(ptr), C.byref(n)) == -6      # VGGP_E_UNSUPPORTED
+            assert b"VGGP_WS_QBAND" in lib.vggp_last_error()
+        for which in (L.WS_P, L.WS_R, L.WS_QBAND, L.WS_KRAW):
+            assert lib.vggp_workspace_ptr(plan.h, which, 1, C.byref(ptr), C.byref(n)) == 0
+        a = C.c_int64()
+        plan.check(lib.vggp_workspace_bytes(plan.h, C.byref(a), None, None))
+        M, sn, tsz = int(np.prod(knots)), sum(knots), 4
+        kept = (8 * sum(3 * k * k for k in knots)         # K_d and P_d (filled on demand), R_d
+                + 8 * (2 + 3 + 3) * sn                    # band of Q_d, generators [pd | ru | rl], band accumulators of dK_d
+                + 8 * 3 * M                               # alpha, the two mode-product tensors
+                + tsz * (M + 8 * sn + 128 * 4 * sn)       # alpha in the observation dtype, per-cell tables, band replicas
+                + 2 * 4 * sn)                             # the knots, twice
+        assert kept <= a.value <= kept + 256, (a.value, kept)
     finally:
         plan.close()
 

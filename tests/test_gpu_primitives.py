@@ -150,25 +150,21 @@ def test_b0_features_dense(vg, dev, dtype, tol):
 # grid-side forward pieces against float64 torch
 # ---------------------------------------------------------------------------------------------------------
 _GF_KNOTS = [(9,), (70, 12), (131, 5, 66), (300, 7), (700,)]
-_GF_PATHS = [(0, 3, "b1_fused"), (0, 2, "b1_round1_semiseparable"), (0, 0, "b1_dense"), (1, 0, "b0_dense")]
+_GF_PATHS = [(0, "b1_fused"), (1, "b0_dense")]
 
 
 # B0 family at (700,): the reference's float32 Toeplitz row is indefinite at this l / delta (the test below covers that
 # case), so the combination is not generated
-@pytest.mark.parametrize("family,structured,knots",
-                         [pytest.param(f, s, k, id=f"{name}-{'x'.join(map(str, k))}")
-                          for (f, s, name) in _GF_PATHS for k in _GF_KNOTS if not (f == 1 and max(k) > 400)])
-def test_grid_forward_pieces(vg, dev, family, structured, knots):
-    """family 0 (B1) runs three factor paths: the fused fibre passes over the twisted factorisation (default), the round-1
-    launches of the same algebra, and the dense blocked Cholesky + triangular inverse that the B0 family always uses."""
+@pytest.mark.parametrize("family,knots",
+                         [pytest.param(f, k, id=f"{name}-{'x'.join(map(str, k))}")
+                          for (f, name) in _GF_PATHS for k in _GF_KNOTS if not (f == 1 and max(k) > 400)])
+def test_grid_forward_pieces(vg, dev, family, knots):
+    """family 0 (B1): the fused fibre passes over the twisted factorisation; family 1 (B0): the dense blocked Cholesky +
+    triangular inverse, whose Cholesky factor and full Q_d are checked too."""
     D = len(knots)
-    dense = structured == 0
+    dense = family != 0
     meshes = [torch.linspace(0, 1 + 0.5 * d, k) for d, k in enumerate(knots)]
-    vg._lib.load().vggp_set_b1_structured(structured)
-    try:
-        plan = vg.GridPlan(family, meshes, torch.float64, dev)
-    finally:
-        vg._lib.load().vggp_set_b1_structured(3)
+    plan = vg.GridPlan(family, meshes, torch.float64, dev)
     g = torch.Generator().manual_seed(100 + D)
     # B0 family: the reference's float32 rounding of (k +- 1) * delta (gridded_kronecker_structure.py:1312-1316)
     # makes the Toeplitz factor numerically indefinite once l / delta is large (min eigenvalue -8e-7 at 130 cells,

@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(HERE, "libvggp.so")
 B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID, SVGP_MARKOV = 0, 1, 2, 3, 4
 F32, F64 = 0, 1
 MEANOPT_JACOBI, MEANOPT_KRONECKER = 0, 1
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 WS_K, WS_P, WS_R, WS_Q, WS_S, WS_ALPHA, WS_SCAL, WS_KRAW, WS_QBAND = range(9)
 
@@ -80,7 +80,6 @@ SIGNATURES = {
                                 _dp, _i64, _i64, _i64, C.c_int, _vp]),
     "vggp_mode_product": (C.c_int, [_vp, C.c_int, _dp, _dp, _dp, _vp]),
     "vggp_set_gemm_mode": (C.c_int, [C.c_int]),
-    "vggp_set_b1_structured": (C.c_int, [C.c_int]),
 }
 
 _lib = None

@@ -1,5 +1,7 @@
-// Grid-side kernels: per-dimension factor build, blocked Cholesky, triangular inverse leaves, band / trace /
-// log-det reductions, and the elementwise + reduction pieces of the reverse pass.  All float64.
+// Dense grid side of the B0, SVGP and VFF families: per-dimension factor build, blocked Cholesky, triangular inverse
+// leaves, band / trace / log-det reductions, and the elementwise + reduction pieces of the reverse pass.  All float64.
+// The entries of every family's factor K_d (factor_entry, factor_entry_grad) are shared with the fused B1 grid side
+// (grid_b1.cuh), the optimal mean (meanopt.cuh) and the optimal covariance (covopt.cuh).
 // Maths: SURVEY.md appendix A.  Reference formulas: gridded_kronecker_structure.py:731-780 (B1/ASVGP Kuu),
 // :1286-1323 (B0 Toeplitz Kuu).
 #pragma once
@@ -9,7 +11,6 @@ namespace vggp {
 
 constexpr int NB = 64;            // Cholesky / triangular-inverse block size
 constexpr int MAX_LEAVES = 40;    // supports M_d <= 2560
-constexpr int SS_SEG = 32;        // segment length of the semiseparable product kernel
 
 // scalar slots in the plan's float64 scalar block
 enum {
@@ -31,13 +32,17 @@ struct GridDims {
     int band_off[VGGP_MAX_D];     // offset (elements) of dim d's block inside the gbuf band part [bp_d|bp_o|bq_d|bq_o]
     int tab_off[VGGP_MAX_D];      // offset (elements) of dim d's block inside the per-cell tables (8 n_d each)
     i64 gfac_off[VGGP_MAX_D];     // B0 family: offset of dim d's [bP | bQ] block inside the gbuf factor part
+    // allocated by every plan but the Markov SVGP's: K_d as built and P_d = K_d^-1 (B1: filled on demand by
+    // vggp_workspace_ptr), R_d = P_d tril(L_d), the band of Q_d = R_d R_d^T
     double* Kraw[VGGP_MAX_D];
+    double* P[VGGP_MAX_D];
+    double* R[VGGP_MAX_D];
+    double* Qb[VGGP_MAX_D];       // float64 main / first off diagonal of Q_d: [diag (n) | off (n)]
+    // allocated by the dense families only (B0, SVGP, VFF): the blocked Cholesky, triangular inverse and GEMM products
     double* cdiag[VGGP_MAX_D];    // NB x NB: factored diagonal block of the previous Cholesky panel (see k_chol_panel)
     double* Kc[VGGP_MAX_D];       // factored in place -> Cholesky factor (lower)
     double* W[VGGP_MAX_D];        // C^-1
-    double* P[VGGP_MAX_D];
     double* Lt[VGGP_MAX_D];       // tril(L_d)
-    double* R[VGGP_MAX_D];
     double* Q[VGGP_MAX_D];
     double* dP[VGGP_MAX_D];
     double* dR[VGGP_MAX_D];
@@ -46,13 +51,7 @@ struct GridDims {
     double* dK[VGGP_MAX_D];
     double* dLraw[VGGP_MAX_D];
     double* tmp[VGGP_MAX_D];
-    double* Qb[VGGP_MAX_D];       // float64 main / first off diagonal of Q_d: [diag (n) | off (n)]
-    int structured;               // B1 family: 0 dense Cholesky path, 1 twisted-factorisation inverse + GEMM products,
-                                  // 2 (default) twisted factorisation + semiseparable O(n^2) products with P_d
-    double* Ad[VGGP_MAX_D];       // structured == 2: A_d = ghat x_d P_d (M-tensors)
-    const double* alpha;          // alpha (M-tensor)
-    i64 inner[VGGP_MAX_D];        // row-major stride of mode d in the M-tensor
-    double* gen[VGGP_MAX_D];      // semiseparable generators of P_d: [pd | ru | rl | gl | gu] each n, then [glend | guend] each nseg
+    double* gen[VGGP_MAX_D];      // B1 plans only: generators of P_d, [pd | ru | rl] each n (k_b1_gens)
     double* sc;                   // SC_COUNT scalars
     int* info;
     void* bandT;                  // per-cell tables in obs dtype: per dim [pe0 pe1 pe2 qe0 qe1 qe2 h rh], each n[d] long
@@ -172,10 +171,8 @@ __global__ void k_build_factors(const __grid_constant__ GridDims g, const double
     const int i = (int)(e / n), j = (int)(e % n);
     const double k = factor_entry(g, theta, d, i, j);
     g.Kraw[d][e] = k;
-    if (!g.structured) {
-        g.Kc[d][e] = k;
-        g.W[d][e] = 0.0;
-    }
+    g.Kc[d][e] = k;
+    g.W[d][e] = 0.0;
     g.Lt[d][e] = (j <= i) ? L[g.Loff[d] + e] : 0.0;
 }
 
@@ -324,243 +321,9 @@ __global__ void __launch_bounds__(NB) k_triinv_leaf(const __grid_constant__ Grid
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Structured inverse of the tridiagonal B1/ASVGP factor K_d (diag a_i, off-diagonal b_i): twisted factorisation
-//   d_0 = a_0, d_k = a_k - b_{k-1}^2 / d_{k-1}   (top-down pivots; log det K = sum log d_k)
-//   e_{n-1} = a_{n-1}, e_k = a_k - b_k^2 / e_{k+1} (bottom-up pivots)
-//   P[j][j] = pd_j = 1 / (d_j + e_j - a_j)
-//   P[i][j] = pd_j prod_{k=i}^{j-1} ru_k (i < j), ru_k = -b_k / d_k ;  P[i][j] = pd_j prod_{k=j}^{i-1} rl_k (i > j), rl_k = -b_k / e_{k+1}
-// k_b1_factor: the two O(n) recurrences (two warps of one CTA per dimension) and the generator tables used by the
-// semiseparable products.
-// grid (D), 256 threads, dynamic smem 7 n doubles.
-// ---------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_b1_factor(const __grid_constant__ GridDims g, const double* __restrict__ theta) {
-    extern __shared__ double sm[];
-    __shared__ double red[32];
-    const int d = blockIdx.x;
-    const int n = g.n[d];
-    double* a = sm;
-    double* b = a + n;
-    double* dd = b + n;
-    double* ee = dd + n;
-    double* ru = ee + n;
-    double* rl = ru + n;
-    double* pd = rl + n;
-    const int tid = threadIdx.x;
-    for (int i = tid; i < n; i += 256) {
-        a[i] = factor_entry(g, theta, d, i, i);
-        b[i] = (i + 1 < n) ? factor_entry(g, theta, d, i, i + 1) : 0.0;
-    }
-    __syncthreads();
-    // The pivots change very slowly along the Toeplitz interior (contraction factor close to 1), so the reciprocal
-    // of the previous pivot is an excellent Newton seed: 1/d_k costs one Newton step (two dependent FMAs) plus a
-    // residual check, instead of a ~100-cycle float64 division on the serial critical path; whenever the residual
-    // is not at rounding level (first rows, last row) the exact division is used.
-    if (tid == 0) {
-        double prev = a[0];
-        dd[0] = prev;
-        double r = 1.0 / prev;
-        bool bad = !(prev > 0.0);
-        for (int k = 1; k < n; ++k) {
-            const double bk = b[k - 1];
-            const double nxt = fma(-bk * bk, r, a[k]);
-            dd[k] = nxt;
-            bad = bad || !(nxt > 0.0);
-            double e = fma(-nxt, r, 1.0);
-            double rn = fma(r, e, r);
-            e = fma(-nxt, rn, 1.0);
-            if (!(fabs(e) < 3e-16)) rn = 1.0 / nxt;
-            r = rn;
-        }
-        if (bad) atomicMax(g.info, d + 1);
-    } else if (tid == 32) {
-        double nxt = a[n - 1];
-        ee[n - 1] = nxt;
-        double r = 1.0 / nxt;
-        for (int k = n - 2; k >= 0; --k) {
-            const double bk = b[k];
-            const double cur = fma(-bk * bk, r, a[k]);
-            ee[k] = cur;
-            double e = fma(-cur, r, 1.0);
-            double rn = fma(r, e, r);
-            e = fma(-cur, rn, 1.0);
-            if (!(fabs(e) < 3e-16)) rn = 1.0 / cur;
-            r = rn;
-        }
-    }
-    __syncthreads();
-    double ld = 0.0;
-    for (int i = tid; i < n; i += 256) {
-        pd[i] = 1.0 / (dd[i] + ee[i] - a[i]);
-        ru[i] = (i + 1 < n) ? -b[i] / dd[i] : 0.0;
-        rl[i] = (i + 1 < n) ? -b[i] / ee[i + 1] : 0.0;
-        ld += log(dd[i]);
-    }
-    ld = block_sum(ld, red);
-    if (tid == 0) g.sc[SC_LOGDETK + d] = ld;
-    __syncthreads();
-    // generators for the semiseparable products (k_ss_apply): segment-local decay products
-    //   gl[i] = prod_{k=a}^{i-1} rl[k],  gu[i] = prod_{k=i}^{b-2} ru[k]   for i in segment [a, b)
-    //   glend[s] = prod_{k=a}^{b-1} rl[k],  guend[s] = ru[a-1] * gu[a]
-    double* gen = g.gen[d];
-    const int nseg = (n + SS_SEG - 1) / SS_SEG;
-    for (int i = tid; i < n; i += 256) { gen[i] = pd[i]; gen[n + i] = ru[i]; gen[2 * n + i] = rl[i]; }
-    for (int sgi = tid; sgi < nseg; sgi += 256) {
-        const int a0 = sgi * SS_SEG, b0 = min(n, a0 + SS_SEG);
-        double pl = 1.0;
-        for (int i = a0; i < b0; ++i) { gen[3 * n + i] = pl; pl *= rl[i]; }
-        gen[5 * n + sgi] = pl;
-        double pu = 1.0;
-        for (int i = b0 - 1; i >= a0; --i) { gen[4 * n + i] = pu; if (i > a0) pu *= ru[i - 1]; }
-        gen[5 * n + nseg + sgi] = (a0 > 0) ? ru[a0 - 1] * pu : 0.0;
-    }
-}
-
-// Explicit P_d from the generators (O(n^2)): needed by the GEMM product path (structured == 1) and by
-// vggp_workspace_ptr; the semiseparable path (structured == 2) never materialises P_d in a step.
-// grid (ceil(nmax / 256), D), 256 threads
-__global__ void __launch_bounds__(256) k_b1_fill_P(const __grid_constant__ GridDims g) {
-    const int d = blockIdx.y;
-    const int n = g.n[d];
-    const int j = (int)blockIdx.x * 256 + threadIdx.x;
-    if (j >= n) return;
-    const double* __restrict__ gen = g.gen[d];
-    double* __restrict__ P = g.P[d];
-    const double pj = gen[j];
-    double p = pj;
-    P[(i64)j * n + j] = p;
-    for (int i = j - 1; i >= 0; --i) {
-        p *= gen[n + i];
-        P[(i64)i * n + j] = p;
-    }
-    p = pj;
-    for (int i = j + 1; i < n; ++i) {
-        p *= gen[2 * n + i - 1];
-        P[(i64)i * n + j] = p;
-    }
-}
-
-// P_d[i][j] for |i - j| <= 1 from the generators
-__device__ __forceinline__ double b1_P_band(const double* __restrict__ gen, int n, int i, int j) {
-    if (i == j) return gen[i];
-    if (j == i + 1) return gen[j] * gen[n + i];
-    return gen[j] * gen[2 * n + j];          // j == i - 1
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Semiseparable product: dst = src x_mode P_d for the B1 family, O(M) per mode instead of a GEMM.
-//   P[i][j] = pd[j] prod_{k=i}^{j-1} ru[k] (i < j),  pd[i] (i == j),  pd[j] prod_{k=j}^{i-1} rl[k] (i > j)
-//   y_i = s_i + l_i + u_i,  s_i = pd_i x_i,  l_{i+1} = rl_i (s_i + l_i),  u_{i-1} = ru_{i-1} (s_i + u_i)
-// Every fibre is cut into segments of SS_SEG elements handled by one thread each (local recurrences with zero
-// carry-in, in registers); the carries are chained through shared memory by one thread per fibre and applied with
-// the precomputed segment-local decay products gl / gu.
-// One launch = a group of tasks (blockIdx.y); grid.x covers the fibres of the largest task.
-// ---------------------------------------------------------------------------------------------------------
-struct SsTask {
-    const double* src;
-    double* dst;
-    const double* gen;        // generators of the dimension being applied
-    int n;                    // M_d
-    int nseg;                 // ceil(n / SS_SEG)
-    int nseg_pad;             // power of two >= nseg, <= 256
-    i64 inner;                // element stride along the mode
-    i64 nfibres;              // outer * inner
-};
-
-constexpr int SS_MAX_TASKS = 12;
-struct SsGroup {
-    SsTask t[SS_MAX_TASKS];
-    int ntasks;
-};
-
-__global__ void __launch_bounds__(256) k_ss_apply(const __grid_constant__ SsGroup grp) {
-    extern __shared__ double sgen[];          // generators of this task's dimension: [pd | ru | rl | gl | gu], 5 n
-    __shared__ double sL[256], sU[256], sLin[256], sUin[256], sGl[256], sGu[256];
-    const SsTask& tk = grp.t[blockIdx.y];
-    const int fpb = 256 / tk.nseg_pad;                      // fibres per block
-    const int tid = threadIdx.x;
-    const int fl = tid % fpb, sg = tid / fpb;
-    const i64 f = (i64)blockIdx.x * fpb + fl;
-    if ((i64)blockIdx.x * fpb >= tk.nfibres) return;
-    const bool live = (f < tk.nfibres) && (sg < tk.nseg);
-    const int n = tk.n;
-    const int a0 = sg * SS_SEG;
-    const double* __restrict__ gen = tk.gen;
-    for (int i = tid; i < 5 * n; i += 256) sgen[i] = gen[i];
-    if (tid < tk.nseg) {                 // segment carry factors, read by the serial chain below
-        sGl[tid] = gen[5 * n + tid];
-        sGu[tid] = gen[5 * n + tk.nseg + tid];
-    }
-    double sv[SS_SEG], yv[SS_SEG];
-    i64 base = 0;
-    if (live) {
-        const i64 o = f / tk.inner, r = f - o * tk.inner;
-        base = o * (i64)n * tk.inner + r;
-#pragma unroll
-        for (int j = 0; j < SS_SEG; ++j) {
-            const int i = a0 + j;
-            sv[j] = (i < n) ? tk.src[base + (i64)i * tk.inner] : 0.0;
-        }
-    }
-    __syncthreads();
-    if (live) {
-        const double* pd = sgen;
-        const double* ru = sgen + n;
-        const double* rl = sgen + 2 * n;
-        double l = 0.0;
-#pragma unroll
-        for (int j = 0; j < SS_SEG; ++j) {
-            const int i = a0 + j;
-            if (i < n) {
-                sv[j] *= pd[i];
-                yv[j] = sv[j] + l;
-                l = rl[i] * (sv[j] + l);
-            } else {
-                yv[j] = 0.0;
-            }
-        }
-        double u = 0.0;
-#pragma unroll
-        for (int j = SS_SEG - 1; j >= 0; --j) {
-            const int i = a0 + j;
-            if (i < n) {
-                yv[j] += u;
-                u = (i > 0) ? ru[i - 1] * (sv[j] + u) : 0.0;
-            }
-        }
-        sL[tid] = l;
-        sU[tid] = u;
-    }
-    __syncthreads();
-    if (sg == 0 && f < tk.nfibres) {
-        // chain the carries of this fibre: Lin[s] = Lout[s-1], Lout[s] = Lloc[s] + Lin[s] * glend[s]
-        double c = 0.0;
-        for (int s2 = 0; s2 < tk.nseg; ++s2) {
-            sLin[s2 * fpb + fl] = c;
-            c = sL[s2 * fpb + fl] + c * sGl[s2];
-        }
-        c = 0.0;
-        for (int s2 = tk.nseg - 1; s2 >= 0; --s2) {
-            sUin[s2 * fpb + fl] = c;
-            c = sU[s2 * fpb + fl] + c * sGu[s2];
-        }
-    }
-    __syncthreads();
-    if (live) {
-        const double lin = sLin[tid], uin = sUin[tid];
-        const double* gl = sgen + 3 * n;
-        const double* gu = sgen + 4 * n;
-#pragma unroll
-        for (int j = 0; j < SS_SEG; ++j) {
-            const int i = a0 + j;
-            if (i < n) tk.dst[base + (i64)i * tk.inner] = yv[j] + lin * gl[i] + uin * gu[i];
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
 // Forward reductions, one warp per row i of dimension d: per-cell tables of P_d and Q_d (observation dtype,
 // monomial basis), the float64 band of Q_d, tr(P_d S_d) = <R_d, tril L_d>, log det S_d = 2 sum log |L_ii|.
-// The band of Q_d = R_d R_d^T is formed from row dot products (structured path: the full Q_d is never built).
+// The band of Q_d = R_d R_d^T is formed from row dot products.
 // grid (ceil(nmax / 8), D), 256 threads.
 // ---------------------------------------------------------------------------------------------------------
 template <typename T>
@@ -594,17 +357,9 @@ __global__ void __launch_bounds__(256) k_fwd_reduce(const __grid_constant__ Grid
         // per-cell tables, monomial basis in the hat weight a (w_lo = 1 - a):
         //   p(a) = A (1-a)^2 + 2 B (1-a) a + C a^2 = pe0 + pe1 a + pe2 a^2, A = P[c][c], B = P[c][c+1], C = P[c+1][c+1]
         T* tab = reinterpret_cast<T*>(g.bandT) + g.tab_off[d];       // [pe0 | pe1 | pe2 | qe0 | qe1 | qe2 | h | rh]
-        double A, B2, C;
-        if (g.structured == 2) {
-            const double* gen = g.gen[d];
-            A = b1_P_band(gen, n, i, i);
-            B2 = last ? 0.0 : 2.0 * b1_P_band(gen, n, i, i + 1);
-            C = last ? 0.0 : b1_P_band(gen, n, i + 1, i + 1);
-        } else {
-            A = P[(i64)i * n + i];
-            B2 = last ? 0.0 : 2.0 * P[(i64)i * n + i + 1];
-            C = last ? 0.0 : P[(i64)(i + 1) * n + i + 1];
-        }
+        const double A = P[(i64)i * n + i];
+        const double B2 = last ? 0.0 : 2.0 * P[(i64)i * n + i + 1];
+        const double C = last ? 0.0 : P[(i64)(i + 1) * n + i + 1];
         tab[i] = (T)A; tab[n + i] = (T)(B2 - 2.0 * A); tab[2 * n + i] = (T)(A - B2 + C);
         atomicAdd(g.sc + SC_TR + d, tr);
         atomicAdd(g.sc + SC_LOGDETS + d, 2.0 * log(fabs(Li[i])));
@@ -668,34 +423,6 @@ __device__ __forceinline__ double tr_others(const GridDims& g, int d) {
     return c;
 }
 
-// dP_d (holding the mode-d Gram contraction) += band scatter ;  dR_d = 2 sym(dQ band) R_d.
-// (the -c_d/2 S_d term of dP_d is routed straight to dK_d as +c_d/2 Q_d in k_bwd_theta: P S P = Q)
-// grid (ceil(nmax^2/256), D)
-template <typename T>
-__global__ void __launch_bounds__(256) k_bwd_dP_dR(const __grid_constant__ GridDims g, const T* __restrict__ gband,
-                                                   const double* __restrict__ theta, double ell_scale) {
-    const int d = blockIdx.y;
-    const int n = g.n[d];
-    const i64 e = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= (i64)n * n) return;
-    const int i = (int)(e / n), j = (int)(e % n);
-    const double noise = theta[2 * g.D];
-    const double cP = ell_scale / (2.0 * noise), cQ = -ell_scale / (2.0 * noise);
-    const T* __restrict__ b = gband + g.band_off[d];   // [bp_diag | bp_off | bq_diag | bq_off]
-    // structured == 2: only the band scatter goes through P . P (X_d); the Gram and dR L^T parts of dP_d enter dK_d's
-    // band as row dot products in k_bwd_theta, so dP_d itself is never formed
-    double v = (g.structured == 2) ? 0.0 : g.dP[d][e];
-    if (i == j) v += cP * (double)b[i];
-    else if (i - j == 1) v += cP * (double)b[n + j];
-    else if (j - i == 1) v += cP * (double)b[n + i];
-    if (g.structured == 2) g.X[d][e] = v; else g.dP[d][e] = v;
-    const double* __restrict__ R = g.R[d];
-    double r = (double)b[2 * n + i] * R[e];
-    if (i > 0) r += (double)b[3 * n + i - 1] * R[e - n];
-    if (i + 1 < n) r += (double)b[3 * n + i] * R[e + n];
-    g.dR[d][e] = 2.0 * cQ * r;
-}
-
 // Dense-feature (B0) family: the per-observation kernel returns FULL factor-gradient sums bP_d, bQ_d.
 //   dP_d += cP bP_d ;  X_d = cQ (bQ_d + bQ_d^T) = 2 cQ sym(bQ_d)   (then dR_d = X_d R_d by a GEMM)
 // grid (ceil(nmax^2/256), D)
@@ -750,8 +477,7 @@ __global__ void __launch_bounds__(256) k_bwd_dm(const double* __restrict__ pg, c
 // d theta and the ELBO scalars.
 //   dK_d(total) = -Y_d P_d + (c_d / 2) Q_d - (M / (2 M_d)) P_d,  Y_d = P_d sym(dP_d),  c_d = prod_{e != d} tr(P_e S_e)
 //   dl_d = <dK, dK/dl>, ds2_d = <dK, dK/ds2> + dkff * kff / s2_d        (accumulated atomically into dtheta)
-// Structured (B1) path: dK/dtheta is tridiagonal, so only the band of Y P is formed, one warp per band entry;
-// dense path: dK_d = -Y_d P_d comes from a GEMM and the full Q_d is used.
+// dK_d = -Y_d P_d comes from a GEMM.
 // grid (chunks, D), 256 threads; dtheta must be zero on entry.  Block (0, 0) also writes dnoise and out[0..3].
 __global__ void __launch_bounds__(256) k_bwd_theta(const __grid_constant__ GridDims g, const double* __restrict__ theta,
                                                    const double* __restrict__ gscal, double ell_scale,
@@ -763,62 +489,16 @@ __global__ void __launch_bounds__(256) k_bwd_theta(const __grid_constant__ GridD
     const double* __restrict__ P = g.P[d];
     const double half_ratio = 0.5 * (double)g.M / (double)n;
     const double half_c = 0.5 * tr_others(g, d);
+    const double* __restrict__ dK = g.dK[d];
+    const double* __restrict__ Q = g.Q[d];
     double sl = 0.0, ss = 0.0;
-    if (g.structured) {
-        const double* __restrict__ Y = g.Y[d];
-        const int lane = threadIdx.x & 31;
-        const int wglobal = (int)blockIdx.x * 8 + (threadIdx.x >> 5);
-        const int wtotal = (int)gridDim.x * 8;
-        for (int e = wglobal; e < 3 * n; e += wtotal) {
-            const int i = e / 3, j = i + (e % 3) - 1;
-            if (j < 0 || j >= n) continue;
-            double acc = 0.0;
-            if (g.structured == 2) {
-                // W = P dP P restricted to the band, dP = Gram + band scatter + dR L^T:
-                //   P (band scatter) P           -> Z (two semiseparable products, k_ss_apply), read at (i, j)
-                //   P unfold(ghat) unfold(T)^T P -> <A_d fibre i, alpha fibre j>,  A_d = ghat x_d P_d, alpha = T_d x_d P_d
-                //   P dR L^T P                   -> <(P dR) row i, (P L) row j> = <dLraw row i, R row j>
-                const double* __restrict__ A = g.Ad[d];
-                const double* __restrict__ al = g.alpha;
-                const i64 inner = g.inner[d];
-                const i64 rest = g.M / n;
-                for (i64 q = lane; q < rest; q += 32) {
-                    const i64 o = q / inner, r = q - o * inner;
-                    const i64 base = o * (i64)n * inner + r;
-                    acc = fma(A[base + (i64)i * inner], al[base + (i64)j * inner], acc);
-                }
-                const double* __restrict__ Li = g.dLraw[d] + (i64)i * n;
-                const double* __restrict__ Rj = g.R[d] + (i64)j * n;
-                for (int k = lane; k < n; k += 32) acc = fma(Li[k], Rj[k], acc);
-                acc = warp_sum(acc);
-                acc += g.dK[d][(i64)i * n + j];
-            } else {
-                const double* Yi = Y + (i64)i * n;
-                const double* Pj = P + (i64)j * n;      // P symmetric: column j = row j
-                for (int k = lane; k < n; k += 32) acc = fma(Yi[k], Pj[k], acc);
-                acc = warp_sum(acc);
-            }
-            if (lane == 0) {
-                const double q = (i == j) ? g.Qb[d][i] : g.Qb[d][n + (i < j ? i : j)];
-                const double pij = (g.structured == 2) ? b1_P_band(g.gen[d], n, i, j) : P[(i64)i * n + j];
-                const double v = -acc + half_c * q - half_ratio * pij;
-                double a, b;
-                factor_entry_grad(g, theta, d, i, j, a, b);
-                sl += v * a;
-                ss += v * b;
-            }
-        }
-    } else {
-        const double* __restrict__ dK = g.dK[d];
-        const double* __restrict__ Q = g.Q[d];
-        for (i64 e = (i64)blockIdx.x * blockDim.x + threadIdx.x; e < (i64)n * n; e += (i64)gridDim.x * blockDim.x) {
-            const int i = (int)(e / n), j = (int)(e % n);
-            double a, b;
-            factor_entry_grad(g, theta, d, i, j, a, b);
-            const double v = dK[e] + half_c * Q[e] - half_ratio * P[e];
-            sl += v * a;
-            ss += v * b;
-        }
+    for (i64 e = (i64)blockIdx.x * blockDim.x + threadIdx.x; e < (i64)n * n; e += (i64)gridDim.x * blockDim.x) {
+        const int i = (int)(e / n), j = (int)(e % n);
+        double a, b;
+        factor_entry_grad(g, theta, d, i, j, a, b);
+        const double v = dK[e] + half_c * Q[e] - half_ratio * P[e];
+        sl += v * a;
+        ss += v * b;
     }
     sl = block_sum(sl, red);
     ss = block_sum(ss, red);
@@ -832,12 +512,10 @@ __global__ void __launch_bounds__(256) k_bwd_theta(const __grid_constant__ GridD
             const double E = gscal[0], nobs = gscal[1];
             const double dkff = -ell_scale * nobs / (2.0 * noise);
             atomicAdd(dtheta + D + d, dkff * kff / theta[D + d]);
-            if (g.family != VGGP_B1_ASVGP) {
-                // the features themselves depend on (l_d, s2_d): sums accumulated by the per-observation kernel
-                atomicAdd(dtheta + d, (ell_scale / noise) * gscal[3 + d]);
-                if (g.family != VGGP_VFF_GRID)      // Fourier features do not scale with s2_d (phi = s2 * ... in the other families)
-                    atomicAdd(dtheta + D + d, (ell_scale / noise) * gscal[5 + d] / theta[D + d]);
-            }
+            // the features themselves depend on (l_d, s2_d): sums accumulated by the per-observation kernel
+            atomicAdd(dtheta + d, (ell_scale / noise) * gscal[3 + d]);
+            if (g.family != VGGP_VFF_GRID)      // Fourier features do not scale with s2_d (phi = s2 * ... in the other families)
+                atomicAdd(dtheta + D + d, (ell_scale / noise) * gscal[5 + d] / theta[D + d]);
             if (d == 0) {
                 const double tot = E + nobs * kff;
                 const double ell = -0.5 * nobs * log(2.0 * 3.14159265358979323846 * noise) - tot / (2.0 * noise);

@@ -1,8 +1,8 @@
 // Fused grid side of the B1 (ASVGP) family: the whole replicated part of a step in a handful of launches.
 //
 // The per-dimension factor K_d of this family is tridiagonal (gridded_kronecker_structure.py:731-780), so P_d = K_d^-1 is
-// semiseparable and every product with it is a pair of first-order recurrences along a fibre (grid.cuh, k_ss_apply).  Round 1
-// ran those as 14 dependent small launches (0.2 ms per step: the Amdahl term of the multi-GPU run).  Here
+// semiseparable and every product with it is a pair of first-order recurrences along a fibre.  Round 1 ran those as 14
+// dependent small launches (0.2 ms per step: the Amdahl term of the multi-GPU run).  Here
 //   k_b1_gens     pivots of the twisted factorisation by a chunk-parallel scan (2 x 2 Moebius composition for the chunk
 //                 carries, the plain recurrence inside a chunk), generators, log det K_d, the P-band tables
 //   k_fibre_pass  ONE engine for every product with P_d: a CTA stages a tile of F fibres in shared memory (coalesced for
@@ -14,7 +14,8 @@
 // A step is: gens, pass F1 (R_d = P_d tril L_d, first mode of alpha), pass F2 (last mode of alpha + casts + row reductions
 // of R_d), the per-observation kernel, pass B1 (last mode of (kron P) g, A_e), pass B2 (first mode, dL), theta (which also
 // forms the band of P X P by O(n) recurrences): 6 launches for D = 2 (one more forward and backward pass for D = 3).
-// Maths: SURVEY.md appendix A; same formulas as the round-1 path (grid.cuh), which stays as the cross-check.
+// This is the only grid side of the family; the reference it is tested against is the float64 oracle (oracle/vggp_oracle.py).
+// Maths: SURVEY.md appendix A.
 #pragma once
 #include "grid.cuh"
 
@@ -65,7 +66,7 @@ struct FpPass {
     i64 M;
     double ell_scale;
     const double* theta;
-    double* gen[VGGP_MAX_D];      // generators of P_d: [pd | ru | rl] (n each; the other slots belong to the round-1 path)
+    double* gen[VGGP_MAX_D];      // generators of P_d: [pd | ru | rl], n each
     double* acc[VGGP_MAX_D];      // band accumulators of dK_d: [3][n], slot (dl + 1, i) = W[i][i + dl]
     double* sc;                   // SC_* scalars
     double* Qb[VGGP_MAX_D];
@@ -193,8 +194,8 @@ __global__ void __launch_bounds__(GEN_THREADS) k_b1_gens(const __grid_constant__
     }
     __syncthreads();
     // plain recurrences inside the chunks.  1 / pivot is carried along by one Newton step from the previous reciprocal
-    // (the pivots change slowly) with an exact division whenever the residual is not at rounding level (round-1 scheme);
-    // the reciprocals are kept: the generators need them.
+    // (the pivots change slowly) with an exact division whenever the residual is not at rounding level; the reciprocals
+    // are kept: the generators need them.
     if (ch < nch) {
         const int k0 = ch * GEN_CHUNK, k1 = min(n, k0 + GEN_CHUNK);
         bool bad = false;
@@ -776,7 +777,6 @@ __device__ __forceinline__ void warp_recurrence(int n, FA a, FB b, double* __res
 //   T_i = xd_i pd_i^2 + 2 xo_i pd_i P[i][i+1] + ru_i^2 T_{i+1},      S_i = xd_i pd_i^2 + 2 xo_{i-1} pd_i P[i][i-1] + rl_{i-1}^2 S_{i-1}
 //   (P X P)[i][i]   = T_i + rl_{i-1}^2 S_{i-1} + 2 xo_{i-1} P[i][i-1] pd_i
 //   (P X P)[i][i+1] = ru_i T_{i+1} + rl_i S_i + xo_i (pd_i pd_{i+1} + P[i][i+1]^2)
-// (round 1 formed X_d P_d and P_d (X_d P_d) as two n x n semiseparable products for these 3 n numbers).
 // grid (D), 512 threads, dynamic smem 7 (n + n / S + 2) doubles.
 // ---------------------------------------------------------------------------------------------------------
 template <typename T>
@@ -916,7 +916,31 @@ __global__ void __launch_bounds__(512) k_b1_theta(const __grid_constant__ GridDi
 #undef TH_STAMP
 }
 
-// K_d as a dense matrix, on demand (vggp_workspace_ptr): the fused path never materialises it in a step.
+// Explicit P_d from the generators (O(n^2)), on demand (vggp_workspace_ptr): the fused path never materialises it in a step.
+//   P[i][j] = pd[j] prod_{k=i}^{j-1} ru[k] (i < j),  pd[i] (i == j),  pd[j] prod_{k=j}^{i-1} rl[k] (i > j)
+// grid (ceil(nmax / 256), D), 256 threads
+__global__ void __launch_bounds__(256) k_b1_fill_P(const __grid_constant__ GridDims g) {
+    const int d = blockIdx.y;
+    const int n = g.n[d];
+    const int j = (int)blockIdx.x * 256 + threadIdx.x;
+    if (j >= n) return;
+    const double* __restrict__ gen = g.gen[d];
+    double* __restrict__ P = g.P[d];
+    const double pj = gen[j];
+    double p = pj;
+    P[(i64)j * n + j] = p;
+    for (int i = j - 1; i >= 0; --i) {
+        p *= gen[n + i];
+        P[(i64)i * n + j] = p;
+    }
+    p = pj;
+    for (int i = j + 1; i < n; ++i) {
+        p *= gen[2 * n + i - 1];
+        P[(i64)i * n + j] = p;
+    }
+}
+
+// K_d as a dense matrix, on demand (vggp_workspace_ptr), like P_d.
 // grid (ceil(nmax^2 / 256), D)
 __global__ void __launch_bounds__(256) k_b1_fill_Kraw(const __grid_constant__ GridDims g, const double* __restrict__ theta) {
     const int d = blockIdx.y;

@@ -65,8 +65,6 @@ thread_local char g_err[512] = {0};
 unsigned long long g_launches = 0;
 static int g_use_mma = 1;
 static int g_bin_stream = 0;       // binned K1: 0 = LDG.128 register ping-pong, 1 = TMA ring through shared memory
-static int g_b1_structured = 3;    // B1 family: 0 dense, 1 twisted inverse + GEMMs, 2 + semiseparable products (round 1),
-                                   // 3 (default) fused fibre passes (grid_b1.cuh)
 
 constexpr int BAND_REPLICAS = 128;
 
@@ -90,7 +88,7 @@ struct vggp_plan {
     MeshView mesh[VGGP_MAX_D];
     GridDims g;
     int nmax;
-    // M-sized float64 work tensors
+    // M-sized float64 work tensors (the B1 family allocates alpha, pgA and pgB only)
     double *mws, *alpha, *Tm[VGGP_MAX_D], *tmpM[VGGP_MAX_D], *gM, *ghat, *pgA, *pgB;
     void* alphaT;
     double* theta_dev;                     // copy of theta of the last forward (the B0 features depend on it)
@@ -133,7 +131,7 @@ struct vggp_plan {
     void* svm_tab = nullptr; int svm_tab_off[VGGP_MAX_D] = {0, 0, 0};
     double* svm_W[VGGP_MAX_D] = {}; double* svm_sc = nullptr;
     int svm_blocks_per_sm = 0;
-    double* b1_acc = nullptr; int b1_acc_total = 0;      // structured == 3: band accumulators of dK_d, [3][n_d] per dimension
+    double* b1_acc = nullptr; int b1_acc_total = 0;      // B1 family: band accumulators of dK_d, [3][n_d] per dimension
     cudaStream_t last_stream = nullptr;                  // stream of the last grid forward (on-demand workspace fills)
     // deterministic mode (vggp_set_deterministic): run records + sort scratch of the per-observation kernel, per-CTA partials
     // of the fibre passes; both grown on demand (the first deterministic step must not run inside a stream capture)
@@ -154,14 +152,11 @@ struct vggp_plan {
     bool forwarded = false;                // a vggp_grid_forward has run on this plan
     void* band_rep = nullptr;              // B1 family, binned kernel: BAND_REPLICAS copies of the band block (obs dtype), kept zero
                                            // between launches (k_band_reduce clears what it sums)
-    // schedules
+    // GEMM schedules of the dense families
     std::vector<Phase> chol_trailing;      // one per panel (may be empty phase)
     int n_panels;
     std::vector<Phase> triinv;             // two launches per recursion depth, deepest first
-    Phase pinv, rs, qq, alpha_phase, bwdA, bwdMid, bwdB, Yp, dKp, dRp, gramOnly, dPOnly;
-    std::vector<SsGroup> ss_fwd;           // structured == 2: R_d, the T_d chains, alpha
-    std::vector<SsGroup> ss_dm;            // (kron P) g, one group per mode
-    SsGroup ss_Z;                          // D = 1 only: Z_0 = Y_0 P_0 needs its own launch
+    Phase pinv, rs, qq, alpha_phase, bwdA, bwdMid, bwdB, Yp, dKp, dRp;
     std::vector<Phase> chains;             // D-1 launches building T_d = m x_{e != d} P_e
     double* dm_result;
     std::vector<void*> allocs;
@@ -389,41 +384,6 @@ GemmDesc gram_desc(const vggp_plan* p, int e, const double* ghat, const double* 
     return d;
 }
 
-// dst = src x_e P_e through the semiseparable generators of dimension `gdim` applied along mode e of a tensor with
-// the given mode sizes (the M-tensor, or an n x n matrix when dims2 is used)
-SsTask ss_task(const double* gen, int n, i64 outer, i64 inner, const double* src, double* dst) {
-    SsTask t;
-    t.src = src; t.dst = dst; t.gen = gen; t.n = n;
-    t.nseg = (n + SS_SEG - 1) / SS_SEG;
-    int pad = 1;
-    while (pad < t.nseg) pad <<= 1;
-    t.nseg_pad = pad;
-    t.inner = inner;
-    t.nfibres = outer * inner;
-    return t;
-}
-
-SsTask ss_mode_task(const vggp_plan* p, int e, const double* src, double* dst) {
-    i64 outer = 1, inner = 1;
-    for (int f = 0; f < e; ++f) outer *= p->n[f];
-    for (int f = e + 1; f < p->D; ++f) inner *= p->n[f];
-    return ss_task(p->g.gen[e], p->n[e], outer, inner, src, dst);
-}
-
-int launch_ss(const SsGroup& grp, cudaStream_t st) {
-    if (grp.ntasks == 0) return 0;
-    i64 gx = 1;
-    int nmax = 1;
-    for (int i = 0; i < grp.ntasks; ++i) {
-        const int fpb = 256 / grp.t[i].nseg_pad;
-        gx = std::max<i64>(gx, (grp.t[i].nfibres + fpb - 1) / fpb);
-        nmax = std::max(nmax, grp.t[i].n);
-    }
-    k_ss_apply<<<dim3((unsigned)gx, grp.ntasks), 256, 5 * (size_t)nmax * sizeof(double), st>>>(grp);
-    VGGP_LAUNCH_CHECK();
-    return 0;
-}
-
 void build_leaves(int lo, int hi, std::vector<int>& bounds) {
     if (hi - lo <= NB) { bounds.push_back(lo); return; }
     const int half = (hi - lo + 1) / 2;
@@ -453,6 +413,7 @@ GemmDesc sub_desc(int n, const double* A, int ar, int ac, const double* B, int b
     return d;
 }
 
+// GEMM schedules of the dense grid side (B0, SVGP and VFF families)
 int build_schedules(vggp_plan* p) {
     const int D = p->D;
     GridDims& g = p->g;
@@ -504,7 +465,7 @@ int build_schedules(vggp_plan* p) {
         p->triinv.push_back(a);
         p->triinv.push_back(b);
     }
-    // ---- P = W^T W ; R = P Lt ; Q = R R^T (dense path only) ----
+    // ---- P = W^T W ; R = P Lt ; Q = R R^T ----
     {
         std::vector<GemmDesc> a, b, c;
         for (int d = 0; d < D; ++d) {
@@ -548,7 +509,7 @@ int build_schedules(vggp_plan* p) {
     // ---- reverse pass, three grouped launches:
     //   bwdA = { first mode of (kron P) g,  Gram contractions dP_d }
     //   bwdB = { remaining modes of (kron P) g (D = 2: the last one),  dP_d += dR_d Lt_d^T,  dLraw_d = P_d dR_d }
-    //   Yp   = { Y_d = P_d sym(dP_d) }     (+ dKp = { dK_d = -Y_d P_d } on the dense factor path)
+    //   Yp   = { Y_d = P_d sym(dP_d) },  dKp = { dK_d = -Y_d P_d }
     // For D = 3 the middle mode of (kron P) g gets its own launch between bwdA and bwdB.
     {
         std::vector<GemmDesc> A, B, mid, y, k, dr;
@@ -576,77 +537,11 @@ int build_schedules(vggp_plan* p) {
             dr.push_back(square_desc(n, g.X[d], false, g.R[d], false, g.dR[d], 1.0, 0.0));   // dense family: dR = 2 cQ sym(bQ) R
         }
         if ((rc = make_phase(p, dr, p->dRp))) return rc;
-        // structured == 2: the only GEMMs left are the Gram contractions and dP += dR Lt^T
-        std::vector<GemmDesc> go, po;
-        for (int d = 0; d < D; ++d) {
-            const int n = p->n[d];
-            go.push_back(gram_desc(p, d, p->ghat, p->Tm[d], g.dP[d], D));
-            GemmDesc x1 = square_desc(n, g.dR[d], false, g.Lt[d], true, g.dP[d], 1.0, 1.0);
-            x1.tri_b = 2;
-            po.push_back(x1);
-        }
-        if ((rc = make_phase(p, go, p->gramOnly))) return rc;
-        if ((rc = make_phase(p, po, p->dPOnly))) return rc;
         if ((rc = make_phase(p, A, p->bwdA))) return rc;
         if ((rc = make_phase(p, mid, p->bwdMid))) return rc;
         if ((rc = make_phase(p, B, p->bwdB))) return rc;
         if ((rc = make_phase(p, y, p->Yp))) return rc;
         if ((rc = make_phase(p, k, p->dKp))) return rc;
-    }
-    // ---- semiseparable product groups (B1 family, structured == 2) ----
-    if (g.structured == 2) {
-        if (3 * D + 1 > SS_MAX_TASKS) return fail(VGGP_E_DIM, "too many tasks for one semiseparable group");
-        SsGroup g0;
-        g0.ntasks = 0;
-        for (int d = 0; d < D; ++d)          // R_d = P_d Lt_d : mode 0 of an n x n matrix
-            g0.t[g0.ntasks++] = ss_task(g.gen[d], p->n[d], 1, p->n[d], g.Lt[d], g.R[d]);
-        for (int s = 0; s + 1 < D; ++s) {
-            SsGroup gs;
-            gs.ntasks = 0;
-            for (int d = 0; d < D; ++d) {
-                int e = s;
-                if (e >= d) e += 1;
-                const bool first = (s == 0), last = (s == D - 2);
-                const double* src = first ? p->mws : p->tmpM[d];
-                double* dst = last ? p->Tm[d] : p->tmpM[d];
-                gs.t[gs.ntasks++] = ss_mode_task(p, e, src, dst);
-            }
-            if (s == 0) {                    // first chain step shares the launch with the R_d products
-                for (int i = 0; i < gs.ntasks; ++i) g0.t[g0.ntasks++] = gs.t[i];
-            } else {
-                if (p->ss_fwd.empty()) p->ss_fwd.push_back(g0);
-                p->ss_fwd.push_back(gs);
-            }
-        }
-        if (p->ss_fwd.empty()) p->ss_fwd.push_back(g0);
-        SsGroup ga;
-        ga.ntasks = 1;
-        ga.t[0] = ss_mode_task(p, D - 1, p->Tm[D - 1], p->alpha);
-        p->ss_fwd.push_back(ga);
-        // reverse pass without GEMMs: launch e applies mode e of (kron P) g; launch 0 also carries A_d = ghat x_d P_d,
-        // dLraw_d = P_d dR_d and Y_d = P_d X_d (X_d = band scatter), launch 1 (or a launch of its own for D = 1)
-        // Z_d = Y_d P_d
-        const double* src = p->gM;
-        for (int e = 0; e < D; ++e) {
-            double* dst = (e % 2 == 0) ? p->pgA : p->pgB;
-            SsGroup gd;
-            gd.ntasks = 1;
-            gd.t[0] = ss_mode_task(p, e, src, dst);
-            if (e == 0) {
-                for (int d = 0; d < D; ++d) {
-                    gd.t[gd.ntasks++] = ss_mode_task(p, d, p->ghat, g.Ad[d]);
-                    gd.t[gd.ntasks++] = ss_task(g.gen[d], p->n[d], 1, p->n[d], g.dR[d], g.dLraw[d]);
-                    gd.t[gd.ntasks++] = ss_task(g.gen[d], p->n[d], 1, p->n[d], g.X[d], g.Y[d]);
-                }
-            }
-            if (e == 1)
-                for (int d = 0; d < D; ++d) gd.t[gd.ntasks++] = ss_task(g.gen[d], p->n[d], p->n[d], 1, g.Y[d], g.dK[d]);
-            p->ss_dm.push_back(gd);
-            src = dst;
-            p->dm_result = dst;
-        }
-        p->ss_Z.ntasks = 0;
-        if (D == 1) p->ss_Z.t[p->ss_Z.ntasks++] = ss_task(g.gen[0], p->n[0], p->n[0], 1, g.Y[0], g.dK[0]);
     }
     return 0;
 }
@@ -2424,17 +2319,12 @@ int vggp_workspace_bytes(const vggp_plan* p, int64_t* plan_bytes, int64_t* gbuf_
 
 int vggp_set_deterministic(vggp_plan* p, int on) {
     if (!p) return fail(VGGP_E_ARG, "null plan");
-    if (on && !(p->family == VGGP_B1_ASVGP && p->g.structured == 3))
-        return fail(VGGP_E_UNSUPPORTED, "deterministic mode covers the B1 (ASVGP) family on its default fused grid path");
+    if (on && p->family != VGGP_B1_ASVGP)
+        return fail(VGGP_E_UNSUPPORTED, "deterministic mode covers the B1 (ASVGP) family");
     if (on)
         for (int d = 0; d < p->D; ++d)
             if (p->n[d] > 512) return fail(VGGP_E_UNSUPPORTED, "deterministic mode needs M_d <= 512");
     p->det = on ? 1 : 0;
-    return 0;
-}
-
-int vggp_set_b1_structured(int on) {
-    g_b1_structured = on < 0 ? 0 : (on > 3 ? 3 : on);
     return 0;
 }
 
@@ -2468,12 +2358,12 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
     if (!p) return fail(VGGP_E_NOMEM, "out of host memory");
     p->family = family; p->D = D; p->obs_dtype = obs_dtype; p->device = device;
     const bool markov = family == VGGP_SVGP_MARKOV;     // O(M + sum M_d^2) grid side: no factor arrays, no GEMM schedules
+    const bool b1 = family == VGGP_B1_ASVGP;            // fused grid side (grid_b1.cuh): generators and R_d, no GEMM schedules
     p->M = 1; p->Lsize = 0; p->nmax = 0;
     int rc = 0;
     GridDims& g = p->g;
     memset(&g, 0, sizeof(g));
     g.D = D; g.family = family; g.obs_dtype = obs_dtype;
-    g.structured = (family == VGGP_B1_ASVGP) ? g_b1_structured : 0;
     int boff = 0, koff = 0, toff = 0;
     i64 foff = 0;
     for (int d = 0; d < D; ++d) {
@@ -2523,14 +2413,17 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
         }
         if (markov) continue;
         const i64 nn = (i64)p->n[d] * p->n[d];
-        TRY(dev_alloc(p, &g.Kraw[d], nn)); TRY(dev_alloc(p, &g.Kc[d], nn)); TRY(dev_alloc(p, &g.W[d], nn));
+        TRY(dev_alloc(p, &g.Kraw[d], nn)); TRY(dev_alloc(p, &g.P[d], nn)); TRY(dev_alloc(p, &g.R[d], nn));
+        TRY(dev_alloc(p, &g.Qb[d], 2 * (i64)p->n[d]));
+        if (b1) {
+            TRY(dev_alloc(p, &g.gen[d], 3 * (i64)p->n[d]));
+            continue;
+        }
+        TRY(dev_alloc(p, &g.Kc[d], nn)); TRY(dev_alloc(p, &g.W[d], nn));
         TRY(dev_alloc(p, &g.cdiag[d], (i64)NB * NB));
-        TRY(dev_alloc(p, &g.P[d], nn)); TRY(dev_alloc(p, &g.Lt[d], nn)); TRY(dev_alloc(p, &g.R[d], nn));
-        TRY(dev_alloc(p, &g.Q[d], nn)); TRY(dev_alloc(p, &g.dP[d], nn));
+        TRY(dev_alloc(p, &g.Lt[d], nn)); TRY(dev_alloc(p, &g.Q[d], nn)); TRY(dev_alloc(p, &g.dP[d], nn));
         TRY(dev_alloc(p, &g.dR[d], nn)); TRY(dev_alloc(p, &g.X[d], nn)); TRY(dev_alloc(p, &g.Y[d], nn));
         TRY(dev_alloc(p, &g.dK[d], nn)); TRY(dev_alloc(p, &g.dLraw[d], nn)); TRY(dev_alloc(p, &g.tmp[d], nn));
-        TRY(dev_alloc(p, &g.Qb[d], 2 * (i64)p->n[d]));
-        TRY(dev_alloc(p, &g.gen[d], 5 * (i64)p->n[d] + 2 * (((i64)p->n[d] + SS_SEG - 1) / SS_SEG) + 8));
         std::vector<int> bounds;
         build_leaves(0, p->n[d], bounds);
         bounds.push_back(p->n[d]);
@@ -2598,7 +2491,7 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
         TRY(dev_alloc(p, &a, p->M * (i64)tsz));
         p->alphaT = a;
     }
-    if (family == VGGP_B1_ASVGP) {
+    if (b1) {
         int acc_total = 0;
         for (int d = 0; d < D; ++d) acc_total += 3 * p->n[d];
         p->b1_acc_total = acc_total;
@@ -2611,31 +2504,28 @@ int vggp_plan_create(vggp_plan** out, int family, int D, const int* n_knots, con
     }
     TRY(dev_alloc(p, &p->theta_dev, 2 * VGGP_MAX_D + 1));
     TRY(dev_alloc(p, &p->obs_counter, 4));
-    TRY(dev_alloc(p, &p->mws, p->M)); TRY(dev_alloc(p, &p->alpha, p->M));
-    TRY(dev_alloc(p, &p->gM, p->M)); TRY(dev_alloc(p, &p->ghat, p->M));
+    TRY(dev_alloc(p, &p->alpha, p->M));
     TRY(dev_alloc(p, &p->pgA, p->M)); TRY(dev_alloc(p, &p->pgB, p->M));
-    for (int d = 0; d < D; ++d) TRY(dev_alloc(p, &g.Ad[d], p->M));
-    g.alpha = p->alpha;
-    for (int d = 0; d < D; ++d) g.inner[d] = p->stride[d];
-    for (int d = 0; d < D; ++d) {
-        if (D > 1) TRY(dev_alloc(p, &p->Tm[d], p->M));
-        if (D > 2) TRY(dev_alloc(p, &p->tmpM[d], p->M)); else p->tmpM[d] = nullptr;
+    if (!b1) {
+        TRY(dev_alloc(p, &p->mws, p->M));
+        TRY(dev_alloc(p, &p->gM, p->M)); TRY(dev_alloc(p, &p->ghat, p->M));
+        for (int d = 0; d < D; ++d) {
+            if (D > 1) TRY(dev_alloc(p, &p->Tm[d], p->M));
+            if (D > 2) TRY(dev_alloc(p, &p->tmpM[d], p->M)); else p->tmpM[d] = nullptr;
+        }
+        TRY(build_schedules(p));
     }
-    TRY(build_schedules(p));
     {
         cudaDeviceProp prop;
         rc = (int)cudaGetDeviceProperties(&prop, device);
         if (rc) { vggp_plan_destroy(p); return fail(rc, "cudaGetDeviceProperties failed"); }
         p->sm_count = prop.multiProcessorCount;
         p->obs_blocks_per_sm = 1;
-        if (family == VGGP_B1_ASVGP) TRY(obs_prepare_dispatch(p));
+        if (b1) TRY(obs_prepare_dispatch(p));
         // the scan form of the cell-integrated family (default for binned observations and for point prediction): its tables
         // (~75 MB at 512 x 512) belong to the plan's one allocation phase, not to the first stream-ordered call that needs them
         if (family == VGGP_B0_GRIDDED && D <= 2) TRY(b0scan_alloc(p));
     }
-    if (!rc) rc = raise_dyn_smem(k_b1_factor, 7 * (size_t)p->nmax * sizeof(double));
-    if (!rc) rc = raise_dyn_smem(k_ss_apply, 5 * (size_t)p->nmax * sizeof(double));
-    if (rc) { vggp_plan_destroy(p); return fail(rc, "cudaFuncSetAttribute(k_b1_factor / k_ss_apply) failed"); }
     rc = raise_dyn_smem(k_chol_panel, (2 * NB * CHOL_PITCH + 2 * NB) * sizeof(double));
     if (!rc) rc = raise_dyn_smem(k_triinv_leaf, 2 * NB * (NB + 1) * sizeof(double));
     if (rc) { vggp_plan_destroy(p); return fail(rc, "cudaFuncSetAttribute failed (is this an sm_100a device?)"); }
@@ -2700,45 +2590,29 @@ int vggp_grid_forward(vggp_plan* p, const double* theta, const double* m, const 
     p->last_stream = st;
     p->forwarded = true;
     if (p->family == VGGP_SVGP_MARKOV) return svgpm_forward(p, theta, m, L, st);
-    if (p->g.structured == 3) return b1f_forward(p, theta, m, L, st);
+    if (p->family == VGGP_B1_ASVGP) return b1f_forward(p, theta, m, L, st);
     VGGP_CUDA(cudaMemcpyAsync(p->mws, m, sizeof(double) * p->M, cudaMemcpyDeviceToDevice, st));
     VGGP_CUDA(cudaMemcpyAsync(p->theta_dev, theta, sizeof(double) * (2 * D + 1), cudaMemcpyDeviceToDevice, st));
     const i64 nn = (i64)p->nmax * p->nmax;
     dim3 egrid(ceil_div(nn, 256), D);
     k_build_factors<<<egrid, 256, 0, st>>>(p->g, theta, L);
     VGGP_LAUNCH_CHECK();
-    if (p->g.structured) {
-        // B1 family: tridiagonal factor -> twisted-factorisation inverse, O(n^2)
-        k_b1_factor<<<D, 256, 7 * (size_t)p->nmax * sizeof(double), st>>>(p->g, theta);
+    const size_t csm = 2 * NB * (NB + 1) * sizeof(double), cpsm = (2 * NB * CHOL_PITCH + 2 * NB) * sizeof(double);
+    for (int j = 0; j < p->n_panels; ++j) {
+        const int j0 = j * NB;
+        dim3 grid(ceil_div(p->nmax - j0, NB), D);
+        k_chol_panel<<<grid, 256, cpsm, st>>>(p->g, j0);
         VGGP_LAUNCH_CHECK();
-        if (p->g.structured == 1) {       // GEMM product path needs the explicit inverse
-            k_b1_fill_P<<<dim3(ceil_div(p->nmax, 256), D), 256, 0, st>>>(p->g);
-            VGGP_LAUNCH_CHECK();
-        }
-    } else {
-        const size_t csm = 2 * NB * (NB + 1) * sizeof(double), cpsm = (2 * NB * CHOL_PITCH + 2 * NB) * sizeof(double);
-        for (int j = 0; j < p->n_panels; ++j) {
-            const int j0 = j * NB;
-            dim3 grid(ceil_div(p->nmax - j0, NB), D);
-            k_chol_panel<<<grid, 256, cpsm, st>>>(p->g, j0);
-            VGGP_LAUNCH_CHECK();
-            if ((rc = launch_phase(p->chol_trailing[j], st))) return rc;
-        }
-        int max_leaves = 0;
-        for (int d = 0; d < D; ++d) max_leaves = std::max(max_leaves, p->g.leaf_cnt[d]);
-        k_triinv_leaf<<<dim3(max_leaves, D), NB, csm, st>>>(p->g);
-        VGGP_LAUNCH_CHECK();
-        for (auto& ph : p->triinv) if ((rc = launch_phase(ph, st))) return rc;
-        if ((rc = launch_phase(p->pinv, st))) return rc;
+        if ((rc = launch_phase(p->chol_trailing[j], st))) return rc;
     }
-    if (p->g.structured == 2) {
-        if ((rc = launch_ss(p->ss_fwd[0], st))) return rc;      // R_d (and the first step of the T_d chains)
-    } else {
-        if ((rc = launch_phase(p->rs, st))) return rc;
-    }
-    if (!p->g.structured) {
-        if ((rc = launch_phase(p->qq, st))) return rc;
-    }
+    int max_leaves = 0;
+    for (int d = 0; d < D; ++d) max_leaves = std::max(max_leaves, p->g.leaf_cnt[d]);
+    k_triinv_leaf<<<dim3(max_leaves, D), NB, csm, st>>>(p->g);
+    VGGP_LAUNCH_CHECK();
+    for (auto& ph : p->triinv) if ((rc = launch_phase(ph, st))) return rc;
+    if ((rc = launch_phase(p->pinv, st))) return rc;
+    if ((rc = launch_phase(p->rs, st))) return rc;
+    if ((rc = launch_phase(p->qq, st))) return rc;
     {
         dim3 rgrid(ceil_div(p->nmax, 8), D), tgrid(ceil_div(p->nmax, 256), D);
         if (p->obs_dtype == VGGP_F32) {
@@ -2752,12 +2626,8 @@ int vggp_grid_forward(vggp_plan* p, const double* theta, const double* m, const 
         }
         VGGP_LAUNCH_CHECK();
     }
-    if (p->g.structured == 2) {
-        for (size_t i = 1; i < p->ss_fwd.size(); ++i) if ((rc = launch_ss(p->ss_fwd[i], st))) return rc;
-    } else {
-        for (auto& ph : p->chains) if ((rc = launch_phase(ph, st))) return rc;
-        if ((rc = launch_phase(p->alpha_phase, st))) return rc;
-    }
+    for (auto& ph : p->chains) if ((rc = launch_phase(ph, st))) return rc;
+    if ((rc = launch_phase(p->alpha_phase, st))) return rc;
     const int cblocks = (int)std::min<i64>((p->M + 255) / 256, 148 * 4);
     if (p->obs_dtype == VGGP_F32)
         k_cast_alpha<float><<<cblocks, 256, 0, st>>>(p->alpha, p->mws, reinterpret_cast<float*>(p->alphaT), p->M, p->g.sc);
@@ -2939,7 +2809,7 @@ int vggp_grid_backward(vggp_plan* p, const double* theta, const double* m, const
     const int D = p->D;
     int rc;
     if (p->family == VGGP_SVGP_MARKOV) return svgpm_backward(p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
-    if (p->g.structured == 3) return b1f_backward(p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
+    if (p->family == VGGP_B1_ASVGP) return b1f_backward(p, theta, m, L, gbuf, ell_scale, out, dtheta, dm, dL, st);
     i64 n_elems, soff, nsc, total;
     vggp_gbuf_layout(p, &n_elems, &soff, &nsc, &total);
     const double* gscal = reinterpret_cast<const double*>(reinterpret_cast<const unsigned char*>(gbuf) + soff);
@@ -2949,51 +2819,29 @@ int vggp_grid_backward(vggp_plan* p, const double* theta, const double* m, const
     else
         k_bwd_prep<double><<<mblocks, 256, 0, st>>>(reinterpret_cast<const double*>(gbuf), p->mws, theta, D, ell_scale, p->gM, p->ghat, p->M);
     VGGP_LAUNCH_CHECK();
-    const bool ss = (p->g.structured == 2);
     const i64 nn = (i64)p->nmax * p->nmax;
     dim3 egrid(ceil_div(nn, 256), D);
-    if (!ss) {
-        for (int d = 0; d < D; ++d)
-            VGGP_CUDA(cudaMemsetAsync(p->g.dP[d], 0, sizeof(double) * (size_t)p->n[d] * p->n[d], st));
-        if ((rc = launch_phase(p->bwdA, st))) return rc;
-        if ((rc = launch_phase(p->bwdMid, st))) return rc;
-    }
-    if (p->family == VGGP_B1_ASVGP) {
-        if (p->obs_dtype == VGGP_F32)
-            k_bwd_dP_dR<float><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const float*>(gbuf) + p->M, theta, ell_scale);
-        else
-            k_bwd_dP_dR<double><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const double*>(gbuf) + p->M, theta, ell_scale);
-        VGGP_LAUNCH_CHECK();
-    } else {
-        if (p->obs_dtype == VGGP_F32)
-            k_bwd_dense_prep<float><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const float*>(gbuf) + p->M, theta, ell_scale);
-        else
-            k_bwd_dense_prep<double><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const double*>(gbuf) + p->M, theta, ell_scale);
-        VGGP_LAUNCH_CHECK();
-        if ((rc = launch_phase(p->dRp, st))) return rc;
-    }
-    if (ss) {
-        // B1 family, no GEMM in the reverse pass: everything that multiplies P_d is a semiseparable product and dK_d is
-        // needed on its band only (k_bwd_theta)
-        for (auto& grp : p->ss_dm) if ((rc = launch_ss(grp, st))) return rc;
-        if ((rc = launch_ss(p->ss_Z, st))) return rc;
-        k_bwd_dm<<<mblocks, 256, 0, st>>>(p->dm_result, p->alpha, dm, p->M);
-        VGGP_LAUNCH_CHECK();
-    } else {
-        if ((rc = launch_phase(p->bwdB, st))) return rc;
-        k_bwd_dm<<<mblocks, 256, 0, st>>>(p->dm_result, p->alpha, dm, p->M);
-        VGGP_LAUNCH_CHECK();
-        k_sym<<<egrid, 256, 0, st>>>(p->g);
-        VGGP_LAUNCH_CHECK();
-        if ((rc = launch_phase(p->Yp, st))) return rc;
-        if (!p->g.structured) {
-            if ((rc = launch_phase(p->dKp, st))) return rc;
-        }
-    }
+    for (int d = 0; d < D; ++d)
+        VGGP_CUDA(cudaMemsetAsync(p->g.dP[d], 0, sizeof(double) * (size_t)p->n[d] * p->n[d], st));
+    if ((rc = launch_phase(p->bwdA, st))) return rc;
+    if ((rc = launch_phase(p->bwdMid, st))) return rc;
+    if (p->obs_dtype == VGGP_F32)
+        k_bwd_dense_prep<float><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const float*>(gbuf) + p->M, theta, ell_scale);
+    else
+        k_bwd_dense_prep<double><<<egrid, 256, 0, st>>>(p->g, reinterpret_cast<const double*>(gbuf) + p->M, theta, ell_scale);
+    VGGP_LAUNCH_CHECK();
+    if ((rc = launch_phase(p->dRp, st))) return rc;
+    if ((rc = launch_phase(p->bwdB, st))) return rc;
+    k_bwd_dm<<<mblocks, 256, 0, st>>>(p->dm_result, p->alpha, dm, p->M);
+    VGGP_LAUNCH_CHECK();
+    k_sym<<<egrid, 256, 0, st>>>(p->g);
+    VGGP_LAUNCH_CHECK();
+    if ((rc = launch_phase(p->Yp, st))) return rc;
+    if ((rc = launch_phase(p->dKp, st))) return rc;
     k_bwd_dL<<<egrid, 256, 0, st>>>(p->g, dL);
     VGGP_LAUNCH_CHECK();
     VGGP_CUDA(cudaMemsetAsync(dtheta, 0, sizeof(double) * (2 * D + 1), st));
-    k_bwd_theta<<<dim3(p->g.structured == 2 ? 96 : (p->g.structured ? 24 : 64), D), 256, 0, st>>>(p->g, theta, gscal, ell_scale, out, dtheta);
+    k_bwd_theta<<<dim3(64, D), 256, 0, st>>>(p->g, theta, gscal, ell_scale, out, dtheta);
     VGGP_LAUNCH_CHECK();
     return 0;
 }
@@ -3399,11 +3247,14 @@ int vggp_workspace_ptr(const vggp_plan* p, int which, int dim, double** ptr, int
     if (p->family == VGGP_SVGP_MARKOV)
         return fail(VGGP_E_UNSUPPORTED, "the Markov SVGP family keeps bands and per-cell tables only: no dense workspace array");
     if (which != VGGP_WS_ALPHA && which != VGGP_WS_SCAL && (dim < 0 || dim >= p->D)) return fail(VGGP_E_ARG, "bad dim");
+    const bool b1 = p->family == VGGP_B1_ASVGP;
+    if (b1 && (which == VGGP_WS_K || which == VGGP_WS_Q))
+        return fail(VGGP_E_UNSUPPORTED, "the B1 family has no Cholesky factor and keeps only the band of Q_d (VGGP_WS_QBAND)");
     const i64 nn = (which == VGGP_WS_ALPHA || which == VGGP_WS_SCAL) ? 0 : (i64)p->n[dim] * p->n[dim];
     switch (which) {
         case VGGP_WS_K: *ptr = p->g.Kc[dim]; if (n_elems) *n_elems = nn; return 0;
         case VGGP_WS_P:
-            if (p->g.structured >= 2) {      // not materialised in a step: filled now, ordered on the stream of the last forward
+            if (b1) {      // not materialised in a step: filled now, ordered on the stream of the last forward
                 k_b1_fill_P<<<dim3(ceil_div(p->nmax, 256), p->D), 256, 0, p->last_stream>>>(p->g);
                 VGGP_LAUNCH_CHECK();
             }
@@ -3412,7 +3263,7 @@ int vggp_workspace_ptr(const vggp_plan* p, int which, int dim, double** ptr, int
         case VGGP_WS_Q: *ptr = p->g.Q[dim]; if (n_elems) *n_elems = nn; return 0;
         case VGGP_WS_S: return fail(VGGP_E_UNSUPPORTED, "S_d is no longer materialised");
         case VGGP_WS_KRAW:
-            if (p->g.structured == 3) {      // as VGGP_WS_P
+            if (b1) {      // as VGGP_WS_P
                 k_b1_fill_Kraw<<<dim3(ceil_div((i64)p->nmax * p->nmax, 256), p->D), 256, 0, p->last_stream>>>(p->g, p->theta_dev);
                 VGGP_LAUNCH_CHECK();
             }
