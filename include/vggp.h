@@ -79,7 +79,7 @@ extern "C" {
 typedef struct vggp_plan vggp_plan;
 
 /* ABI version of this header; vggp_abi_version() must return the same value. */
-#define VGGP_ABI_VERSION 3
+#define VGGP_ABI_VERSION 4
 int vggp_abi_version(void);
 const char* vggp_last_error(void);
 /* Number of CUDA kernels this library has launched so far in this process (host-side counter). */
@@ -203,6 +203,45 @@ int vggp_obs_bin_pack(vggp_plan* plan, const vggp_binned_desc* desc, const void*
                       void* binned, void* stream);
 int vggp_obs_fwd_bwd_binned(vggp_plan* plan, const vggp_binned_desc* desc, const void* binned, void* gbuf,
                             void* stream);
+/*
+ * Epoch-shuffled minibatches in the binned layout (csrc/minibatch.cuh; B1, VGGP_SVGP_MARKOV and B0 with D <= 2).
+ * Sampling law: epoch `epoch` of rank `rank` draws a pseudo-random permutation pi of the rank's n observations, a keyed
+ * bijection computed inline (a balanced 4-round Feistel network on the smallest even number of bits k with 2^k >= n, round
+ * function a 32-bit mixing hash of seed, epoch, rank, round and half, cycle-walking below n).  Batch b < P is
+ * { i : pi(i) in [b B, (b + 1) B) }, the other n - P B observations are dropped, so every observation is in a given batch
+ * with probability B / n: the expected log-likelihood of a batch scaled by n / B (ell_scale) is unbiased.
+ * One device pass bins all P batches into one buffer: P 256-byte headers, then each batch's sections.  Batch b is the view
+ * (binned + byte_offset, vggp_binned_desc) of vggp_epoch_batch, which every entry point taking a binned buffer accepts
+ * (vggp_obs_fwd_bwd_binned in both modes, vggp_meanopt_assemble); its n is B.  Its bytes equal vggp_obs_bin_pack of that
+ * batch's observations in ascending index order with the same run_cap.
+ *   vggp_epoch_bin_prepare  x[D] (n values each), B = batch_size, n_batches = P (0 = n / B; a sharded run passes the
+ *                           smallest shard's count so that every rank steps equally often), run_cap (0 = the automatic rule
+ *                           of vggp_obs_bin_prepare applied to B) -> desc, and totals_host [VGGP_EPOCH_TOTALS * P]: per batch
+ *                           { tasks, runs, observations inside the mesh, data elements, byte offset of its first section }.
+ *                           Sorts by (batch, cell), plans the runs of every batch on the device and reads back only the
+ *                           per-batch totals: synchronises `stream`, allocates temporaries that live until the matching
+ *                           vggp_epoch_bin_pack (one pending epoch per plan).  VGGP_E_UNSUPPORTED for VGGP_SVGP_GRID,
+ *                           VGGP_VFF_GRID and B0 with D = 3; VGGP_E_ARG for B < 1, B > n, n >= 2^31.
+ *   vggp_epoch_bin_pack     fills `binned` (desc->bytes, 256-byte aligned) from x[D], y; synchronises, frees the temporaries.
+ *   vggp_epoch_batch        host only: the descriptor of batch b and the byte offset of its view in `binned`.
+ */
+#define VGGP_EPOCH_TOTALS 5
+typedef struct vggp_epoch_desc {
+    int64_t bytes;          /* size of the epoch buffer */
+    int64_t n;              /* observations given */
+    int64_t batch_size;     /* B */
+    int64_t n_batches;      /* P */
+    int64_t n_tasks, n_runs, data_elems;   /* sums over the batches */
+    uint64_t seed, epoch;
+    int32_t rank, run_cap, D, elem_size;
+} vggp_epoch_desc;
+int vggp_epoch_bin_prepare(vggp_plan* plan, const void* const* x, int64_t n, int64_t batch_size, int64_t n_batches,
+                           int run_cap, uint64_t seed, uint64_t epoch, int rank, vggp_epoch_desc* desc,
+                           int64_t* totals_host, void* stream);
+int vggp_epoch_bin_pack(vggp_plan* plan, const vggp_epoch_desc* desc, const int64_t* totals_host, const void* const* x,
+                        const void* y, void* binned, void* stream);
+int vggp_epoch_batch(const vggp_epoch_desc* desc, const int64_t* totals_host, int64_t b, vggp_binned_desc* batch,
+                     int64_t* byte_offset);
 /* How vggp_obs_fwd_bwd_binned streams the observations: 0 (default) coalesced 16-byte global loads into two register
  * buffers; 1 = a per-warp shared-memory ring filled by TMA bulk copies (cp.async.bulk + mbarrier), two stages ahead. */
 int vggp_set_binned_stream(int mode);

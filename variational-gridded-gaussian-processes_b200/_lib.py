@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(HERE, "libvggp.so")
 B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID, SVGP_MARKOV = 0, 1, 2, 3, 4
 F32, F64 = 0, 1
 MEANOPT_JACOBI, MEANOPT_KRONECKER = 0, 1
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 WS_K, WS_P, WS_R, WS_Q, WS_S, WS_ALPHA, WS_SCAL, WS_KRAW, WS_QBAND = range(9)
 
@@ -24,6 +24,16 @@ class BinnedDesc(C.Structure):
                 ("data_elems", _i64), ("off_task_off", _i64), ("off_task_R", _i64), ("off_run_cell", _i64),
                 ("off_run_n", _i64), ("off_run_start", _i64), ("off_data", _i64),
                 ("run_cap", C.c_int32), ("D", C.c_int32)]
+
+
+class EpochDesc(C.Structure):
+    """vggp_epoch_desc (include/vggp.h): layout of one epoch of binned minibatches."""
+    _fields_ = [("bytes", _i64), ("n", _i64), ("batch_size", _i64), ("n_batches", _i64), ("n_tasks", _i64),
+                ("n_runs", _i64), ("data_elems", _i64), ("seed", C.c_uint64), ("epoch", C.c_uint64),
+                ("rank", C.c_int32), ("run_cap", C.c_int32), ("D", C.c_int32), ("elem_size", C.c_int32)]
+
+
+EPOCH_TOTALS = 5
 
 
 class ArDesc(C.Structure):
@@ -50,6 +60,10 @@ SIGNATURES = {
     "vggp_obs_bin_prepare": (C.c_int, [_vp, C.POINTER(_vp), _i64, C.c_int, C.POINTER(BinnedDesc), _vp]),
     "vggp_obs_bin_pack": (C.c_int, [_vp, C.POINTER(BinnedDesc), C.POINTER(_vp), _dp, _dp, _vp]),
     "vggp_obs_fwd_bwd_binned": (C.c_int, [_vp, C.POINTER(BinnedDesc), _dp, _dp, _vp]),
+    "vggp_epoch_bin_prepare": (C.c_int, [_vp, C.POINTER(_vp), _i64, _i64, _i64, C.c_int, C.c_uint64, C.c_uint64, C.c_int,
+                                         C.POINTER(EpochDesc), C.POINTER(_i64), _vp]),
+    "vggp_epoch_bin_pack": (C.c_int, [_vp, C.POINTER(EpochDesc), C.POINTER(_i64), C.POINTER(_vp), _dp, _dp, _vp]),
+    "vggp_epoch_batch": (C.c_int, [C.POINTER(EpochDesc), C.POINTER(_i64), _i64, C.POINTER(BinnedDesc), C.POINTER(_i64)]),
     "vggp_set_binned_stream": (C.c_int, [C.c_int]),
     "vggp_set_deterministic": (C.c_int, [_vp, C.c_int]),
     "vggp_workspace_bytes": (C.c_int, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),

@@ -6,6 +6,7 @@
 #include <mutex>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include "common.cuh"
 #include "gemm.cuh"
@@ -20,6 +21,7 @@
 #include "meanopt.cuh"
 #include "covopt.cuh"
 #include "collective.cuh"
+#include "minibatch.cuh"
 
 // Every plan-taking entry point runs with the plan's device current and restores the caller's device on return
 // (launches on a stream of another device fail with "invalid resource handle"; plan creation must not silently switch
@@ -69,6 +71,21 @@ static int g_bin_stream = 0;       // binned K1: 0 = LDG.128 register ping-pong,
 constexpr int BAND_REPLICAS = 128;
 
 struct ZeroJob { void* ptr; size_t pitch, width, height; };      // cudaMemset2DAsync of a split-K destination (beta = 0)
+// epoch binning planned by vggp_epoch_bin_prepare (minibatch.cuh): the device arrays the pack reads, until vggp_epoch_bin_pack
+struct MbPending {
+    bool active = false;
+    vggp_epoch_desc desc = {};
+    std::vector<void*> keep;
+    uint32_t* perm = nullptr;                          // sorted position -> input index (batch b from position b B)
+    unsigned long long *task_base = nullptr, *run_off = nullptr, *batch_runs = nullptr;
+    long long* task_goff = nullptr;
+    int32_t *task_R = nullptr, *run_len = nullptr;
+    uint32_t *run_sorted = nullptr, *run_cell = nullptr, *run_start = nullptr;
+    void clear() {
+        for (void* a : keep) cudaFree(a);
+        *this = MbPending();
+    }
+};
 struct Phase {
     GemmDesc* d_descs = nullptr;
     int ndesc = 0;
@@ -104,6 +121,7 @@ struct vggp_plan {
     void* pk_x[VGGP_MAX_D] = {nullptr, nullptr, nullptr}; void* pk_y = nullptr; i64 pk_cap = 0;
     // binned layout: the layout planned by vggp_obs_bin_prepare and the cell-sorted order, until vggp_obs_bin_pack
     BinLayout bin_pending; uint32_t* bin_perm = nullptr; bool bin_has_pending = false;
+    MbPending mb;                          // epoch minibatches: vggp_epoch_bin_prepare until vggp_epoch_bin_pack
     // B0 family, scan form (b0scan.cuh): per-dimension transform rows and products, per-cell tables; allocated at first use
     bool b0s_ready = false;
     double* b0s_G[VGGP_MAX_D][4] = {};     // GL, GR, dGL/dl, dGR/dl: (K+1) x (K-1)
@@ -1105,6 +1123,44 @@ int bin_prepare_impl(vggp_plan* p, const void* const* x, i64 n, int run_cap, vgg
     return 0;
 }
 
+// data blocks of one binned set whose tables are already in `buf`: perm maps its stream positions to input indices
+template <typename T, int D>
+int launch_bin_gather(vggp_plan* p, const void* const* x, const void* y, const uint32_t* perm, unsigned char* buf,
+                      const vggp_binned_desc* desc, i64 n_tasks, cudaStream_t st) {
+    const int blocks = (int)std::min<i64>(n_tasks, (i64)p->sm_count * 8);
+    if (p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV) {
+        B0sGatherArgs<T, D> gb0;
+        for (int d = 0; d < D; ++d) {
+            gb0.x[d] = reinterpret_cast<const T*>(x[d]);
+            gb0.knots[d] = p->d_knots[d];
+            gb0.K[d] = p->K[d];
+        }
+        gb0.y = reinterpret_cast<const T*>(y);
+        gb0.perm = perm;
+        gb0.buf = buf;
+        gb0.off_task_off = desc->off_task_off; gb0.off_task_R = desc->off_task_R; gb0.off_run_cell = desc->off_run_cell;
+        gb0.off_run_n = desc->off_run_n; gb0.off_run_start = desc->off_run_start; gb0.off_data = desc->off_data;
+        gb0.n_tasks = (int)n_tasks;
+        k_b0s_gather<T, D><<<blocks, 256, 0, st>>>(gb0);
+    } else {
+        BinGatherArgs<T, D> ga;
+        for (int d = 0; d < D; ++d) {
+            ga.x[d] = reinterpret_cast<const T*>(x[d]);
+            ga.knots[d] = p->d_knots[d];
+            ga.K[d] = p->K[d];
+        }
+        ga.y = reinterpret_cast<const T*>(y);
+        ga.perm = perm;
+        ga.buf = buf;
+        ga.off_task_off = desc->off_task_off; ga.off_task_R = desc->off_task_R; ga.off_run_cell = desc->off_run_cell;
+        ga.off_run_n = desc->off_run_n; ga.off_run_start = desc->off_run_start; ga.off_data = desc->off_data;
+        ga.n_tasks = (int)n_tasks;
+        k_bin_gather<T, D><<<blocks, 256, 0, st>>>(ga);
+    }
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+
 template <typename T, int D>
 int bin_pack_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* const* x, const void* y, void* binned,
                   cudaStream_t st) {
@@ -1117,37 +1173,7 @@ int bin_pack_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* const*
         VGGP_CUDA(cudaMemcpyAsync(buf + desc->off_run_cell, L.run_cell.data(), sizeof(uint32_t) * 32 * L.n_tasks, cudaMemcpyHostToDevice, st));
         VGGP_CUDA(cudaMemcpyAsync(buf + desc->off_run_n, L.run_n.data(), sizeof(int32_t) * 32 * L.n_tasks, cudaMemcpyHostToDevice, st));
         VGGP_CUDA(cudaMemcpyAsync(buf + desc->off_run_start, L.run_start.data(), sizeof(uint32_t) * 32 * L.n_tasks, cudaMemcpyHostToDevice, st));
-        const int blocks = (int)std::min<i64>(L.n_tasks, (i64)p->sm_count * 8);
-        if (p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV) {
-            B0sGatherArgs<T, D> gb0;
-            for (int d = 0; d < D; ++d) {
-                gb0.x[d] = reinterpret_cast<const T*>(x[d]);
-                gb0.knots[d] = p->d_knots[d];
-                gb0.K[d] = p->K[d];
-            }
-            gb0.y = reinterpret_cast<const T*>(y);
-            gb0.perm = p->bin_perm;
-            gb0.buf = buf;
-            gb0.off_task_off = desc->off_task_off; gb0.off_task_R = desc->off_task_R; gb0.off_run_cell = desc->off_run_cell;
-            gb0.off_run_n = desc->off_run_n; gb0.off_run_start = desc->off_run_start; gb0.off_data = desc->off_data;
-            gb0.n_tasks = (int)L.n_tasks;
-            k_b0s_gather<T, D><<<blocks, 256, 0, st>>>(gb0);
-        } else {
-            BinGatherArgs<T, D> ga;
-            for (int d = 0; d < D; ++d) {
-                ga.x[d] = reinterpret_cast<const T*>(x[d]);
-                ga.knots[d] = p->d_knots[d];
-                ga.K[d] = p->K[d];
-            }
-            ga.y = reinterpret_cast<const T*>(y);
-            ga.perm = p->bin_perm;
-            ga.buf = buf;
-            ga.off_task_off = desc->off_task_off; ga.off_task_R = desc->off_task_R; ga.off_run_cell = desc->off_run_cell;
-            ga.off_run_n = desc->off_run_n; ga.off_run_start = desc->off_run_start; ga.off_data = desc->off_data;
-            ga.n_tasks = (int)L.n_tasks;
-            k_bin_gather<T, D><<<blocks, 256, 0, st>>>(ga);
-        }
-        VGGP_LAUNCH_CHECK();
+        if (int rc = launch_bin_gather<T, D>(p, x, y, p->bin_perm, buf, desc, L.n_tasks, st)) return rc;
     }
     if (L.n > L.n_inside) {
         const i64 nout = L.n - L.n_inside;
@@ -1220,6 +1246,218 @@ int bin_prepare_dispatch(vggp_plan* p, const void* const* x, i64 n, int cap, vgg
 }
 int bin_pack_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void* const* x, const void* y, void* binned, cudaStream_t st) {
     VGGP_DISPATCH_TD(p, bin_pack_impl, p, desc, x, y, binned, st);
+}
+// ---- epoch minibatches in the binned layout (minibatch.cuh) ----------------------------------------------
+inline int mb_bits(uint64_t max_value) {        // tight end_bit of a radix sort whose largest key is max_value
+    int b = 1;
+    while (b < 64 && (max_value >> b) != 0) ++b;
+    return b;
+}
+
+template <typename KT>
+int mb_sort_pairs(const KT* kin, KT* kout, const uint32_t* vin, uint32_t* vout, i64 n, int end_bit, DevTemps& tmp,
+                  cudaStream_t st) {
+    size_t bytes = 0;
+    VGGP_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, kin, kout, vin, vout, (int)n, 0, end_bit, st));
+    void* temp = nullptr;
+    VGGP_CUDA(tmp.alloc(&temp, bytes));
+    VGGP_CUDA(cub::DeviceRadixSort::SortPairs(temp, bytes, kin, kout, vin, vout, (int)n, 0, end_bit, st));
+    return 0;
+}
+
+template <typename V, typename W>
+int mb_exclusive_sum(const V* in, W* out, i64 n, DevTemps& tmp, cudaStream_t st) {
+    size_t bytes = 0;
+    VGGP_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, n, st));
+    void* temp = nullptr;
+    VGGP_CUDA(tmp.alloc(&temp, bytes));
+    VGGP_CUDA(cub::DeviceScan::ExclusiveSum(temp, bytes, in, out, n, st));
+    return 0;
+}
+
+// The per-batch binned descriptor and view offset (bytes from the epoch buffer) of batch b.  totals[MB_TOTALS b + 4] is the
+// byte offset of the batch's first section; its sections follow in the order and alignment of bin_offsets.
+void mb_batch_desc(const vggp_epoch_desc* e, const int64_t* totals, i64 b, vggp_binned_desc* out, int64_t* view_off) {
+    const int64_t* t = totals + MB_TOTALS * b;
+    const BinOffsets o = bin_offsets(t[0], t[3], e->elem_size);
+    const i64 view = (i64)BIN_HEADER_BYTES * b, rel = t[4] - o.task_off - view;   // section offsets relative to the view
+    memset(out, 0, sizeof(*out));
+    out->bytes = o.bytes + rel;
+    out->n = e->batch_size; out->n_inside = t[2]; out->n_tasks = t[0]; out->n_runs = t[1]; out->data_elems = t[3];
+    out->off_task_off = o.task_off + rel; out->off_task_R = o.task_R + rel; out->off_run_cell = o.run_cell + rel;
+    out->off_run_n = o.run_n + rel; out->off_run_start = o.run_start + rel; out->off_data = o.data + rel;
+    out->run_cap = e->run_cap; out->D = e->D;
+    *view_off = view;
+}
+
+template <typename T, int D, typename KT>
+int epoch_prepare_kt(vggp_plan* p, const void* const* x, vggp_epoch_desc* e, int64_t* totals, cudaStream_t st) {
+    const bool ext = p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV;
+    const i64 n = e->n, B = e->batch_size, P = e->n_batches, m = P * B;
+    const uint32_t cap = (uint32_t)e->run_cap;
+    i64 ncells = 1;
+    for (int d = 0; d < D; ++d) ncells *= (ext ? p->K[d] + 1 : p->K[d] - 1);
+    const i64 nck = ext ? ncells : ncells + 1;                  // cell keys per batch (B1: the outside key last)
+    const int blocks_n = (int)std::min<i64>((n + 256) / 256, (i64)p->sm_count * 16);
+    const int blocks_m = (int)std::min<i64>((m + 256) / 256, (i64)p->sm_count * 16);
+    DevTemps tmp;
+    // 1. keys (batch, cell) with the permutation fused in, one radix sort
+    KT *keys_in = nullptr, *keys = nullptr;
+    uint32_t *idx_in = nullptr, *perm = nullptr;
+    VGGP_CUDA(tmp.alloc(&keys_in, sizeof(KT) * n));
+    VGGP_CUDA(tmp.alloc(&keys, sizeof(KT) * n));
+    VGGP_CUDA(tmp.alloc(&idx_in, sizeof(uint32_t) * n));
+    VGGP_CUDA(tmp.alloc(&perm, sizeof(uint32_t) * n));
+    MbKeyArgs<T, D> ka;
+    for (int d = 0; d < D; ++d) { ka.x[d] = reinterpret_cast<const T*>(x[d]); ka.mesh[d] = p->mesh[d]; }
+    ka.perm = mb_perm_make(n, e->seed, e->epoch, e->rank);
+    ka.B = (uint32_t)B; ka.P = (uint32_t)P; ka.ncell_keys = (uint64_t)nck; ka.ext = ext ? 1 : 0;
+    k_mb_keys<T, D, KT><<<blocks_n, 256, 0, st>>>(ka, keys_in, idx_in);
+    VGGP_LAUNCH_CHECK();
+    if (int rc = mb_sort_pairs<KT>(keys_in, keys, idx_in, perm, n, mb_bits((uint64_t)P * (uint64_t)nck), tmp, st)) return rc;
+    // 2. segments of equal key among the m kept positions, runs per segment, per-batch sums
+    uint32_t *flags = nullptr, *segid = nullptr, *seg_start = nullptr, *seg_nruns = nullptr, *run_base = nullptr;
+    for (uint32_t** a : {&flags, &segid, &seg_start, &seg_nruns, &run_base}) VGGP_CUDA(tmp.alloc(a, sizeof(uint32_t) * (m + 1)));
+    unsigned long long *batch_runs = nullptr, *batch_inside = nullptr, *run_off = nullptr, *batch_tasks = nullptr, *task_base = nullptr;
+    for (unsigned long long** a : {&batch_runs, &batch_inside, &run_off, &batch_tasks, &task_base})
+        VGGP_CUDA(tmp.alloc(a, sizeof(unsigned long long) * (P + 1)));
+    VGGP_CUDA(cudaMemsetAsync(batch_runs, 0, sizeof(unsigned long long) * (P + 1), st));
+    VGGP_CUDA(cudaMemsetAsync(batch_inside, 0, sizeof(unsigned long long) * (P + 1), st));
+    VGGP_CUDA(cudaMemsetAsync(seg_nruns, 0, sizeof(uint32_t) * (m + 1), st));
+    k_mb_heads<KT><<<blocks_m, 256, 0, st>>>(keys, m, flags);
+    VGGP_LAUNCH_CHECK();
+    if (int rc = mb_exclusive_sum(flags, segid, m + 1, tmp, st)) return rc;
+    k_mb_seg_starts<<<blocks_m, 256, 0, st>>>(flags, segid, m, seg_start);
+    VGGP_LAUNCH_CHECK();
+    k_mb_seg_runs<KT><<<blocks_m, 256, 0, st>>>(keys, seg_start, segid + m, (uint64_t)nck, ext ? ~0ull : (uint64_t)ncells, cap,
+                                              seg_nruns, batch_runs, batch_inside);
+    VGGP_LAUNCH_CHECK();
+    if (int rc = mb_exclusive_sum(seg_nruns, run_base, m + 1, tmp, st)) return rc;
+    uint32_t n_runs_h = 0;
+    VGGP_CUDA(cudaMemcpyAsync(&n_runs_h, run_base + m, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    const i64 R = n_runs_h;
+    // 3. the runs in cell order, then a stable sort by (batch, longest first)
+    KT *run_key = nullptr, *run_key_s = nullptr;
+    uint32_t *run_idx = nullptr, *run_sorted = nullptr, *run_cell = nullptr, *run_start = nullptr;
+    int32_t* run_len = nullptr;
+    VGGP_CUDA(tmp.alloc(&run_key, sizeof(KT) * R));
+    VGGP_CUDA(tmp.alloc(&run_key_s, sizeof(KT) * R));
+    for (uint32_t** a : {&run_idx, &run_sorted, &run_cell, &run_start}) VGGP_CUDA(tmp.alloc(a, sizeof(uint32_t) * R));
+    VGGP_CUDA(tmp.alloc(&run_len, sizeof(int32_t) * R));
+    if (R > 0) {
+        k_mb_emit_runs<KT><<<(int)std::min<i64>((R + 255) / 256, (i64)p->sm_count * 16), 256, 0, st>>>(
+            keys, seg_start, run_base, segid + m, R, (uint64_t)nck, cap, (uint32_t)B, run_key, run_idx, run_cell, run_len, run_start);
+        VGGP_LAUNCH_CHECK();
+        if (int rc = mb_sort_pairs<KT>(run_key, run_key_s, run_idx, run_sorted, R, mb_bits((uint64_t)P * (cap + 1ull) - 1), tmp, st))
+            return rc;
+    }
+    // 4. tasks: per-batch run and task offsets, padded run length and streamed elements of every task, their scan
+    if (int rc = mb_exclusive_sum(batch_runs, run_off, P + 1, tmp, st)) return rc;
+    const int blocks_p = (int)std::min<i64>((P + 256) / 256, (i64)p->sm_count * 16);
+    k_mb_batch_tasks<<<blocks_p, 256, 0, st>>>(batch_runs, P, batch_tasks);
+    VGGP_LAUNCH_CHECK();
+    if (int rc = mb_exclusive_sum(batch_tasks, task_base, P + 1, tmp, st)) return rc;
+    const i64 T_ub = (R + 31) / 32 + P;                         // >= sum over batches of ceil(runs / 32)
+    int32_t* task_R = nullptr;
+    long long *task_elems = nullptr, *task_goff = nullptr, *d_tot = nullptr;
+    VGGP_CUDA(tmp.alloc(&task_R, sizeof(int32_t) * T_ub));
+    VGGP_CUDA(tmp.alloc(&task_elems, sizeof(long long) * (T_ub + 1)));
+    VGGP_CUDA(tmp.alloc(&task_goff, sizeof(long long) * (T_ub + 1)));
+    VGGP_CUDA(tmp.alloc(&d_tot, sizeof(long long) * 4 * P));
+    k_mb_task_R<<<(int)std::min<i64>((T_ub + 256) / 256, (i64)p->sm_count * 16), 256, 0, st>>>(
+        task_base, run_off, run_sorted, run_len, P, T_ub, D, task_R, task_elems);
+    VGGP_LAUNCH_CHECK();
+    if (int rc = mb_exclusive_sum(task_elems, task_goff, T_ub + 1, tmp, st)) return rc;
+    k_mb_totals<<<blocks_p, 256, 0, st>>>(batch_runs, batch_inside, task_base, task_goff, P, d_tot);
+    VGGP_LAUNCH_CHECK();
+    // 5. the per-batch totals back to the host, which lays the buffer out: P headers, then each batch's sections
+    std::vector<long long> h((size_t)(4 * P));
+    VGGP_CUDA(cudaMemcpyAsync(h.data(), d_tot, sizeof(long long) * 4 * P, cudaMemcpyDeviceToHost, st));
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    i64 off = (i64)BIN_HEADER_BYTES * P;
+    e->n_tasks = e->n_runs = e->data_elems = 0;
+    for (i64 b = 0; b < P; ++b) {
+        int64_t* t = totals + MB_TOTALS * b;
+        for (int j = 0; j < 4; ++j) t[j] = h[(size_t)(4 * b + j)];
+        t[4] = off;
+        off += bin_offsets(t[0], t[3], (int)sizeof(T)).bytes - BIN_HEADER_BYTES;
+        e->n_tasks += t[0]; e->n_runs += t[1]; e->data_elems += t[3];
+    }
+    e->bytes = off;
+    // what the pack needs lives on in the plan until vggp_epoch_bin_pack
+    MbPending& q = p->mb;
+    q.perm = perm; q.task_base = task_base; q.task_goff = task_goff; q.task_R = task_R; q.run_off = run_off;
+    q.batch_runs = batch_runs; q.run_sorted = run_sorted; q.run_cell = run_cell; q.run_len = run_len; q.run_start = run_start;
+    for (void* a : {(void*)perm, (void*)task_base, (void*)task_goff, (void*)task_R, (void*)run_off, (void*)batch_runs,
+                    (void*)run_sorted, (void*)run_cell, (void*)run_len, (void*)run_start}) {
+        tmp.release(a);
+        q.keep.push_back(a);
+    }
+    q.desc = *e;
+    q.active = true;
+    return 0;
+}
+
+template <typename T, int D>
+int epoch_prepare_impl(vggp_plan* p, const void* const* x, vggp_epoch_desc* e, int64_t* totals, cudaStream_t st) {
+    const bool ext = p->family == VGGP_B0_GRIDDED || p->family == VGGP_SVGP_MARKOV;
+    uint64_t ncells = 1;
+    for (int d = 0; d < D; ++d) ncells *= (uint64_t)(ext ? p->K[d] + 1 : p->K[d] - 1);
+    const uint64_t P = (uint64_t)e->n_batches, kmax = std::max<uint64_t>(P * (ext ? ncells : ncells + 1), P * ((uint64_t)e->run_cap + 1));
+    if (kmax < 0xffffffffull) return epoch_prepare_kt<T, D, uint32_t>(p, x, e, totals, st);
+    return epoch_prepare_kt<T, D, unsigned long long>(p, x, e, totals, st);
+}
+
+template <typename T, int D>
+int epoch_pack_impl(vggp_plan* p, const int64_t* totals, const void* const* x, const void* y, void* binned, cudaStream_t st) {
+    MbPending& q = p->mb;
+    const vggp_epoch_desc& e = q.desc;
+    const i64 P = e.n_batches, B = e.batch_size;
+    unsigned char* buf = reinterpret_cast<unsigned char*>(binned);
+    DevTemps tmp;
+    VGGP_CUDA(cudaMemsetAsync(buf, 0, (size_t)BIN_HEADER_BYTES * P, st));
+    std::vector<long long> sec((size_t)(6 * P));
+    std::vector<vggp_binned_desc> bd((size_t)P);
+    for (i64 b = 0; b < P; ++b) {
+        int64_t view = 0;
+        mb_batch_desc(&e, totals, b, &bd[(size_t)b], &view);
+        const vggp_binned_desc& d = bd[(size_t)b];
+        const i64 o[6] = {d.off_task_off, d.off_task_R, d.off_run_cell, d.off_run_n, d.off_run_start, d.off_data};
+        for (int j = 0; j < 6; ++j) sec[(size_t)(6 * b + j)] = view + o[j];
+    }
+    long long* d_sec = nullptr;
+    VGGP_CUDA(tmp.alloc(&d_sec, sizeof(long long) * 6 * P));
+    VGGP_CUDA(cudaMemcpyAsync(d_sec, sec.data(), sizeof(long long) * 6 * P, cudaMemcpyHostToDevice, st));
+    if (e.n_tasks > 0) {
+        k_mb_tables<<<(int)std::min<i64>((32 * e.n_tasks + 255) / 256, (i64)p->sm_count * 16), 256, 0, st>>>(
+            q.task_base, q.task_goff, q.task_R, q.run_off, q.batch_runs, q.run_sorted, q.run_cell, q.run_len, q.run_start, d_sec, P,
+            buf);
+        VGGP_LAUNCH_CHECK();
+    }
+    for (i64 b = 0; b < P; ++b) {
+        const vggp_binned_desc& d = bd[(size_t)b];
+        unsigned char* view = buf + (i64)BIN_HEADER_BYTES * b;
+        const uint32_t* perm = q.perm + b * B;
+        if (d.n_tasks > 0)
+            if (int rc = launch_bin_gather<T, D>(p, x, y, perm, view, &d, d.n_tasks, st)) return rc;
+        if (d.n_inside < B) {                 // B1: sum of y^2 of the batch's observations outside the mesh, in its own header
+            const i64 nout = B - d.n_inside;
+            const int blocks = (int)std::min<i64>((nout + 255) / 256, 148 * 4);
+            k_bin_sum_y2<T><<<blocks, 256, 0, st>>>(reinterpret_cast<const T*>(y), perm, d.n_inside, B, reinterpret_cast<double*>(view));
+            VGGP_LAUNCH_CHECK();
+        }
+    }
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    p->mb.clear();
+    return 0;
+}
+
+int epoch_prepare_dispatch(vggp_plan* p, const void* const* x, vggp_epoch_desc* e, int64_t* totals, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, epoch_prepare_impl, p, x, e, totals, st);
+}
+int epoch_pack_dispatch(vggp_plan* p, const int64_t* totals, const void* const* x, const void* y, void* binned, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, epoch_pack_impl, p, totals, x, y, binned, st);
 }
 // grow-only scratch (never inside a stream capture: cudaMalloc is not capturable)
 int det_reserve(void** buf, size_t* have, size_t want, cudaStream_t st) {
@@ -2542,6 +2780,7 @@ int vggp_plan_destroy(vggp_plan* p) {
         if (p->pk_x[d]) cudaFree(p->pk_x[d]);
     if (p->pk_y) cudaFree(p->pk_y);
     if (p->bin_perm) cudaFree(p->bin_perm);
+    p->mb.clear();
     if (p->det_buf) cudaFree(p->det_buf);
     if (p->one_ws) cudaFree(p->one_ws);
     if (p->det_fp) cudaFree(p->det_fp);
@@ -2712,19 +2951,21 @@ int vggp_obs_fwd_bwd(vggp_plan* p, const void* const* x, const void* y, int64_t 
     return vggp_obs_fwd_bwd_packed(p, p->pk_x, p->pk_y, n, gbuf, stream);
 }
 
+// run_cap = 0 of the binned layouts: about two tasks (of 32 runs) per resident warp, so that thin shards and cell-range shards
+// (few, full cells) still spread over the whole GPU; 256 (the value the 1-GPU measurements settled on) from 2^25.8 observations up
+static int auto_run_cap(const vggp_plan* p, i64 n) {
+    const i64 warps = (i64)p->sm_count * 24;
+    const i64 want = (n + 64 * warps - 1) / (64 * warps);
+    return (int)std::min<i64>(256, std::max<i64>(32, (want + 3) / 4 * 4));
+}
+
 int vggp_obs_bin_prepare(vggp_plan* p, const void* const* x, int64_t n, int run_cap, vggp_binned_desc* desc, void* stream) {
     DeviceGuard dev_guard(p ? p->device : -1);
     if (!p || !desc || n < 0) return fail(VGGP_E_ARG, "bad argument");
     if (p->family == VGGP_B0_GRIDDED && p->D > 2) return fail(VGGP_E_UNSUPPORTED, "the B0 (cell-integrated) family is built for D <= 2, as in the reference");
     if (p->family == VGGP_SVGP_GRID || p->family == VGGP_VFF_GRID)
         return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families take plain observation arrays (vggp_obs_fwd_bwd)");
-    if (run_cap == 0) {
-        // automatic: about two tasks (of 32 runs) per resident warp, so that thin shards and cell-range shards (few, full cells)
-        // still spread over the whole GPU; 256 (the value the 1-GPU measurements settled on) from 2^25.8 observations up
-        const i64 warps = (i64)p->sm_count * 24;
-        const i64 want = (n + 64 * warps - 1) / (64 * warps);
-        run_cap = (int)std::min<i64>(256, std::max<i64>(32, (want + 3) / 4 * 4));
-    }
+    if (run_cap == 0) run_cap = auto_run_cap(p, n);
     if (run_cap < 4) return fail(VGGP_E_ARG, "run_cap must be >= 4 (0 = automatic)");
     if (n >= ((i64)1 << 31)) return fail(VGGP_E_UNSUPPORTED, "binning supports n < 2^31 observations per shard");
     if (n > 0) {
@@ -2770,6 +3011,54 @@ int vggp_obs_fwd_bwd_binned(vggp_plan* p, const vggp_binned_desc* desc, const vo
     if (p->family == VGGP_SVGP_MARKOV) return obs_svgpm_dispatch(p, desc, binned, gbuf, st);  // Markov form (svgpm.cuh)
     if (p->family == VGGP_B0_GRIDDED) return obs_b0s_dispatch(p, desc, binned, gbuf, st);     // scan form (b0scan.cuh)
     return obs_binned_dispatch(p, desc, binned, gbuf, st);
+}
+
+int vggp_epoch_bin_prepare(vggp_plan* p, const void* const* x, int64_t n, int64_t batch_size, int64_t n_batches, int run_cap,
+                           uint64_t seed, uint64_t epoch, int rank, vggp_epoch_desc* desc, int64_t* totals_host, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !desc || !totals_host) return fail(VGGP_E_ARG, "bad argument");
+    if (p->family == VGGP_SVGP_GRID || p->family == VGGP_VFF_GRID)
+        return fail(VGGP_E_UNSUPPORTED, "the SVGP and VFF families have no binned layout: index their plain arrays");
+    if (p->family == VGGP_B0_GRIDDED && p->D > 2) return fail(VGGP_E_UNSUPPORTED, "the B0 (cell-integrated) family is built for D <= 2, as in the reference");
+    if (n < 1 || n >= ((i64)1 << 31)) return fail(VGGP_E_ARG, "epoch binning needs 1 <= n < 2^31 observations per shard");
+    if (batch_size < 1 || batch_size > n) return fail(VGGP_E_ARG, "batch_size must be in 1..n");
+    if (n_batches < 0 || n_batches > n / batch_size) return fail(VGGP_E_ARG, "n_batches must be in 0..n / batch_size (0 = n / batch_size)");
+    if (rank < 0) return fail(VGGP_E_ARG, "rank must be >= 0");
+    if (run_cap == 0) run_cap = auto_run_cap(p, batch_size);
+    if (run_cap < 4) return fail(VGGP_E_ARG, "run_cap must be >= 4 (0 = automatic)");
+    if (!x) return fail(VGGP_E_ARG, "null observation pointers");
+    for (int d = 0; d < p->D; ++d)
+        if (!x[d]) return fail(VGGP_E_ARG, "null observation pointer");
+    p->mb.clear();
+    memset(desc, 0, sizeof(*desc));
+    desc->n = n; desc->batch_size = batch_size; desc->n_batches = n_batches ? n_batches : n / batch_size;
+    desc->seed = seed; desc->epoch = epoch; desc->rank = rank;
+    desc->run_cap = run_cap / 4 * 4; desc->D = p->D; desc->elem_size = p->obs_dtype == VGGP_F32 ? 4 : 8;
+    const int rc = epoch_prepare_dispatch(p, x, desc, totals_host, (cudaStream_t)stream);
+    if (rc) p->mb.clear();
+    return rc;
+}
+
+int vggp_epoch_bin_pack(vggp_plan* p, const vggp_epoch_desc* desc, const int64_t* totals_host, const void* const* x, const void* y,
+                        void* binned, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !desc || !totals_host || !binned) return fail(VGGP_E_ARG, "bad argument");
+    if (!p->mb.active) return fail(VGGP_E_ARG, "vggp_epoch_bin_pack without a pending vggp_epoch_bin_prepare on this plan");
+    if (memcmp(desc, &p->mb.desc, sizeof(*desc)) != 0) return fail(VGGP_E_ARG, "descriptor does not match the pending epoch");
+    if (!x || !y) return fail(VGGP_E_ARG, "null observation pointers");
+    for (int d = 0; d < p->D; ++d)
+        if (!x[d]) return fail(VGGP_E_ARG, "null observation pointer");
+    const int rc = epoch_pack_dispatch(p, totals_host, x, y, binned, (cudaStream_t)stream);
+    if (rc) p->mb.clear();
+    return rc;
+}
+
+int vggp_epoch_batch(const vggp_epoch_desc* desc, const int64_t* totals_host, int64_t b, vggp_binned_desc* batch,
+                     int64_t* byte_offset) {
+    if (!desc || !totals_host || !batch || !byte_offset) return fail(VGGP_E_ARG, "bad argument");
+    if (b < 0 || b >= desc->n_batches) return fail(VGGP_E_ARG, "batch index out of range");
+    mb_batch_desc(desc, totals_host, b, batch, byte_offset);
+    return 0;
 }
 
 int vggp_allreduce_gbuf(vggp_plan* p, const vggp_ar_desc* desc, int* err_flag, void* stream) {

@@ -17,7 +17,7 @@ from torch import nn
 
 from .. import _lib
 from ..params import DenseNormal, GaussianLikelihood, GriddedMarginals, GriddedNormal, MaternKernel, ScaleKernel
-from ..plan import BinnedObs, GridPlan, gridded_elbo
+from ..plan import BinnedBatch, BinnedObs, GridPlan, gridded_elbo
 from ..dist import shard_bounds
 
 
@@ -58,6 +58,7 @@ class GriddedVariationalGP(nn.Module):
         self._obs = None
         self._packed = None
         self._group = None
+        self._shard = (0, 1)                    # (rank, world) of shard_observations
         self._n_total = int(y.numel())
         self._terms = None                      # [ELBO, scaled ELL, KL, n_obs] of the last _elbo() (device tensor)
         self.strict_checks = bool(int(os.environ.get("VGGP_STRICT", "0")))   # synchronise and check after every _elbo()
@@ -87,6 +88,7 @@ class GriddedVariationalGP(nn.Module):
         self.train_inputs = (X[lo:hi],)
         self.train_targets = y[lo:hi]
         self._group = group if world > 1 else None
+        self._shard = (int(rank), int(world))
         self._obs = None
 
     def _device_dtype(self):
@@ -152,9 +154,13 @@ class GriddedVariationalGP(nn.Module):
         """Synchronise and raise torch.linalg.LinAlgError if the last `_elbo()` hit a non-positive-definite factor."""
         self._raise_if_failed(wait=True)
 
-    def _elbo(self, batch: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Evidence lower bound (0-dim tensor with grad_fn).  `batch`: optional index tensor / slice selecting a
-        minibatch of this rank's observations; the expected log-likelihood is rescaled by N / B."""
+    def _elbo(self, batch=None) -> torch.Tensor:
+        """Evidence lower bound (0-dim tensor with grad_fn).  `batch` selects a minibatch of this rank's observations, and the
+        expected log-likelihood is rescaled by N / B:
+          a BinnedBatch of `minibatches()`   the binned per-observation kernel of the family on that batch (B1, B0 with
+                                             D <= 2, Markov SVGP), ell_scale = batch.scale;
+          an index tensor or slice           gathers x[batch] and runs the plain-array kernel (B1: unsorted raw kernel, B0 and
+                                             the dense families: dense features); the Markov SVGP form has no such path."""
         self._raise_if_failed(wait=False)
         plan = self._ensure_plan()
         if self._packed is not None:
@@ -162,10 +168,12 @@ class GriddedVariationalGP(nn.Module):
         else:
             xs, y = self._obs
         scale = 1.0
-        if batch is not None:
+        if isinstance(batch, BinnedBatch):
+            xs, y, scale = batch, None, batch.scale
+        elif batch is not None:
             if self.family == _lib.SVGP_MARKOV:
-                raise NotImplementedError("minibatches of the Markov SVGP form need the plain-array per-observation path, which "
-                                          "this family does not have yet: call _elbo() on the full (sharded) data set")
+                raise NotImplementedError("the Markov SVGP form takes no index batches (it has no plain-array per-observation "
+                                          "path): draw binned batches with minibatches(), or call _elbo() on the full data set")
             xs = [x[batch].contiguous() for x in self._obs[0]]
             y = self._obs[1][batch].contiguous()
             n_local = self._obs[1].numel()
@@ -178,6 +186,18 @@ class GriddedVariationalGP(nn.Module):
         if self.strict_checks:
             self._raise_if_failed(wait=True)
         return elbo
+
+    def minibatches(self, batch_size: int, seed: int = 0, run_cap: int = 256) -> "Minibatches":
+        """Epoch-shuffled minibatches of this rank's observations in the binned layout (GridPlan.bin_epoch): `.epoch(e)` bins
+        the P = n // batch_size batches of epoch e in one device pass and yields them in order b = 0..P-1; pass each to
+        `_elbo(batch=...)`.  Every epoch is a fresh permutation keyed by (seed, e, rank) without replacement, the remainder
+        dropped.  On a sharded model every rank draws from its own shard and P comes from the smallest shard, so that all
+        ranks step equally often.  B1, B0 (D <= 2) and Markov SVGP families."""
+        if self.family in (_lib.SVGP_GRID, _lib.VFF_GRID) or (self.family == _lib.B0_GRIDDED and self.D > 2):
+            raise NotImplementedError("this family has no binned layout: pass index tensors to _elbo(batch=...)")
+        if batch_size < 1:
+            raise ValueError("batch_size must be >= 1")
+        return Minibatches(self, int(batch_size), int(seed), int(run_cap))
 
     def elbo_terms(self) -> torch.Tensor:
         """[ELBO, scaled expected log-likelihood, KL, n_obs over all ranks] of the last `_elbo()` call (float64 device
@@ -483,6 +503,29 @@ class GriddedVariationalGP(nn.Module):
             k.base_kernel.lengthscale = X[:, d].std() / lmbda
         mean_os = sum(k.outputscale for k in self._kernels) / len(self._kernels)
         self.likelihood.noise = y.var() - mean_os
+
+
+class Minibatches:
+    """The iterable of GriddedVariationalGP.minibatches(): `epoch(e)` re-bins once on the device and yields the batches."""
+
+    def __init__(self, model: GriddedVariationalGP, batch_size: int, seed: int, run_cap: int):
+        self.model, self.batch_size, self.seed, self.run_cap = model, batch_size, seed, run_cap
+
+    def epoch(self, e: int):
+        m = self.model
+        plan = m._ensure_plan()
+        xs, y = m._obs
+        rank, world = m._shard
+        n_batches = (m._n_total // world) // self.batch_size
+        if n_batches < 1:
+            raise ValueError(f"batch_size {self.batch_size} exceeds the smallest shard ({m._n_total // world} observations)")
+        bins = plan.bin_epoch(xs, y, self.batch_size, self.seed, int(e), self.run_cap, rank, n_batches)
+        if world > 1:
+            # the ranks' batches are summed by the all-reduce before the grid side applies one ell_scale: every rank
+            # must use the same one, N / (world B) (equal to n_rank / B when the shards are equal)
+            for bo in bins:
+                bo.scale = float(m._n_total) / float(world * self.batch_size)
+        yield from bins
 
 
 def b0_cell_cov(delta32: torch.Tensor, m: int, lengthscale: torch.Tensor, outputscale: torch.Tensor) -> torch.Tensor:

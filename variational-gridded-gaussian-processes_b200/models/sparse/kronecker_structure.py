@@ -90,7 +90,8 @@ class Matern12SVGP(_DenseFeatureModel):
     `markov=True` evaluates the same model (same ELBO, gradients and predictions) in its O(1)-per-observation Markov form
     (family SVGP_MARKOV, csrc/svgpm.cuh): K_d^-1 is tridiagonal for a Matern-1/2 kernel on sorted points, so every
     observation touches two inducing points per dimension, the grid side is O(M + sum M_d^2), and 512 x 512 grids with
-    2^26 observations are in reach.  Full-batch `_elbo()` only (a minibatch raises NotImplementedError).  The default stays
+    2^26 observations are in reach.  Minibatches are binned: `minibatches(B).epoch(e)` yields batches for `_elbo(batch=...)`
+    (an index-tensor batch raises NotImplementedError).  The default stays
     the dense path for now; the intended follow-up makes `markov=True` the default and keeps SVGP_GRID as the test
     reference."""
     family = _lib.SVGP_GRID

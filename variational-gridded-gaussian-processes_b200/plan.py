@@ -118,6 +118,33 @@ class GridPlan:
                                               _stream_ptr(self.device)))
         return BinnedObs(buf, desc, 4 if self.obs_dtype == torch.float32 else 8)
 
+    def bin_epoch(self, xs: Sequence[torch.Tensor], y: torch.Tensor, batch_size: int, seed: int, epoch: int,
+                  run_cap: int = 256, rank: int = 0, n_batches: int = 0) -> "EpochBins":
+        """All minibatches of one epoch in the binned layout, binned in one device pass (include/vggp.h, vggp_epoch_bin_*).
+        Epoch `epoch` of `rank` draws a pseudo-random permutation pi of the n observations (keyed by seed, epoch and rank);
+        batch b is {i : pi(i) in [b B, (b + 1) B)} for b < P = n // B (or `n_batches`, which a sharded run sets to the
+        smallest shard's count), the rest of the epoch is dropped.  Each batch is a BinnedBatch view of one buffer: a
+        BinnedObs with n = B and scale = n / B, bit-identical to `bin` of its observations in ascending index order."""
+        n = int(y.numel())
+        self._check_obs(xs, y, n)
+        B = int(batch_size)
+        P = int(n_batches) or (n // B if B >= 1 else 0)
+        desc = _lib.EpochDesc()
+        totals = (C.c_int64 * max(1, _lib.EPOCH_TOTALS * P))()
+        src = (C.c_void_p * self.D)(*[t.data_ptr() for t in xs])
+        _lib.check(self.lib.vggp_epoch_bin_prepare(self.handle, src, n, B, int(n_batches), int(run_cap), int(seed), int(epoch),
+                                                   int(rank), C.byref(desc), totals, _stream_ptr(self.device)))
+        buf = torch.empty(int(desc.bytes), dtype=torch.uint8, device=self.device)
+        _lib.check(self.lib.vggp_epoch_bin_pack(self.handle, C.byref(desc), totals, src, y.data_ptr(), buf.data_ptr(),
+                                                _stream_ptr(self.device)))
+        esz = 4 if self.obs_dtype == torch.float32 else 8
+        batches = []
+        for b in range(int(desc.n_batches)):
+            bd, off = _lib.BinnedDesc(), C.c_int64()
+            _lib.check(self.lib.vggp_epoch_batch(C.byref(desc), totals, b, C.byref(bd), C.byref(off)))
+            batches.append(BinnedBatch(buf[int(off.value):], bd, esz, float(n) / float(B)))
+        return EpochBins(buf, desc, batches)
+
     def meanopt_assemble(self, binned: "BinnedObs"):
         """Fill the stencil system of the optimal variational mean from a binned buffer of this plan
         (vggp_meanopt_assemble; B1 and SVGP_MARKOV families, the latter at the theta of the last grid_forward)."""
@@ -469,6 +496,31 @@ class BinnedObs:
     def streamed_bytes(self) -> int:
         """Bytes of observation data the fused kernel reads per launch (padding included)."""
         return int(self.desc.data_elems) * self.elem_size
+
+
+class BinnedBatch(BinnedObs):
+    """One minibatch of an epoch (GridPlan.bin_epoch): a view into the epoch's buffer that every binned entry point takes,
+    plus `scale` = n / B, the ell_scale that makes its expected log-likelihood an unbiased estimate of the full one."""
+
+    def __init__(self, buf: torch.Tensor, desc, elem_size: int, scale: float):
+        super().__init__(buf, desc, elem_size)
+        self.scale = scale
+
+
+class EpochBins:
+    """The binned minibatches of one epoch: one device buffer (`buf`), its descriptor and the P BinnedBatch views."""
+
+    def __init__(self, buf: torch.Tensor, desc, batches):
+        self.buf, self.desc, self.batches = buf, desc, batches
+
+    def __len__(self) -> int:
+        return len(self.batches)
+
+    def __iter__(self):
+        return iter(self.batches)
+
+    def __getitem__(self, b: int) -> BinnedBatch:
+        return self.batches[b]
 
 
 class _DevArray:
