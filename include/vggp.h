@@ -25,7 +25,7 @@
  *     vggp_last_error() returns a static/thread-local message for the last non-zero status.
  *   - all work is asynchronous and ordered on the `stream` argument (a cudaStream_t passed as void*;
  *     NULL = the legacy default stream).  No entry point except vggp_plan_create/destroy, vggp_read_info,
- *     vggp_elbo_host, vggp_meanopt_solve and vggp_meanopt_solve_pc synchronises the host.
+ *     vggp_elbo_host, vggp_meanopt_solve, vggp_meanopt_solve_pc and vggp_logdet_system synchronises the host.
  *   - the caller owns every buffer passed in; the library allocates only inside vggp_plan_create (its
  *     grid-side workspace) and frees it in vggp_plan_destroy.
  *   - pointers are DEVICE pointers unless the parameter name ends in `_host`.
@@ -79,7 +79,7 @@ extern "C" {
 typedef struct vggp_plan vggp_plan;
 
 /* ABI version of this header; vggp_abi_version() must return the same value. */
-#define VGGP_ABI_VERSION 4
+#define VGGP_ABI_VERSION 5
 int vggp_abi_version(void);
 const char* vggp_last_error(void);
 /* Number of CUDA kernels this library has launched so far in this process (host-side counter). */
@@ -391,6 +391,45 @@ int vggp_meanopt_solve_pc(vggp_plan* plan, int precond, double rtol, int max_ite
  */
 int vggp_covopt_update(vggp_plan* plan, int dim, const void* gbuf, double ell_scale, const double* L, double* L_out,
                        double* change, void* stream);
+
+/* ---- collapsed ELBO at any grid size (B1 and VGGP_SVGP_MARKOV; csrc/collapsed.cuh, DESIGN.md section 4, K1l) -------------
+ * The reference's objective (its collapsed _elbo()) from the stencil system A = F + G / noise of the optimal mean (F = Kuu for
+ * B1, F = Kuu^-1 for Markov) and the solver's iterate x* (B1: alpha*, Markov: m*), by the matrix determinant lemma:
+ *     ELBO = -1/2 [N log 2 pi + N log noise + log det A - log det F + (y^T y - b^T x*) / noise] - (N prod_d s2_d - tr(F^-1 G)) / (2 noise)
+ * with log det F = log det Kuu (B1) or -log det Kuu (Markov), tr(F^-1 G) = tr(Kuu^-1 G) (B1) or tr(Kuu G) (Markov).
+ *   vggp_logdet_system    log det A by preconditioned stochastic Lanczos quadrature: log det A = log det P + tr log(C^-1 A C^-T)
+ *                         with the preconditioner P = C C^T of vggp_meanopt_solve_pc (`precond`: VGGP_MEANOPT_JACOBI,
+ *                         C = diag(A)^1/2; VGGP_MEANOPT_KRONECKER, C = kron_d L_d D_d^1/2 of the Thomas factors of F_d + g I).
+ *                         log det P is exact; the trace is estimated from `n_probes` probes eps_j, each by Gauss quadrature on
+ *                         its Lanczos tridiagonal.  probe_kind VGGP_PROBE_RADEMACHER: signs from a counter hash of
+ *                         (seed_or_first, probe, node), estimate = log det P + mean_j eps_j^T log(B) eps_j, standard error =
+ *                         sample deviation / sqrt(n_probes); VGGP_PROBE_UNIT: e_first .. e_{first + n_probes - 1}
+ *                         (first = seed_or_first), estimate = log det P + sum_j, exact when the probes cover all M nodes,
+ *                         standard error 0.  A probe has converged once its quadrature value moves by <= rtol (relative)
+ *                         between two checks (8 steps apart, from 128 steps on steps / 8
+ *                         apart), or when its Krylov space is exhausted; max_steps bounds the
+ *                         iteration.  out_host[VGGP_LOGDET_FIELDS] = { estimate, standard error, log det P, Lanczos steps (max
+ *                         over probes), probes converged, probes }; per_probe_host [n_probes] (or NULL) the per-probe values.
+ *                         For one assembly and seed the output is bitwise reproducible (fixed-order reductions).  The first
+ *                         call allocates (4 k + 1) M float64 and small arrays (k = n_probes; grown when k or max_steps grows;
+ *                         counted in scratch_bytes, refused under stream capture).  Synchronises `stream`.
+ *   vggp_collapsed_terms  out [VGGP_CT_FIELDS] (DEVICE float64) = { N (all observations of the binned set), sum y^2 (including
+ *                         the observations outside the mesh), b^T x*, tr(F^-1 G), log det Kuu }: exact, fixed-order
+ *                         reductions over the binned data section and the grid.  Needs a vggp_meanopt_solve /
+ *                         vggp_meanopt_solve_pc on the current assembly after the last vggp_grid_forward (a forward
+ *                         invalidates the solve), whose iterate it reads; `desc` / `binned` must be the set given to
+ *                         vggp_meanopt_assemble (its n, n_tasks and data_elems are compared).  Asynchronous.
+ * Both: VGGP_E_UNSUPPORTED for the B0, SVGP_GRID and VFF families; VGGP_E_ARG without a previous vggp_meanopt_assemble (and,
+ * for the terms, without a solve on it or with another binned set), for n_probes outside 1 .. VGGP_MAX_PROBES, max_steps < 1, unit probes past M and an unknown precond.
+ */
+#define VGGP_PROBE_RADEMACHER 0
+#define VGGP_PROBE_UNIT       1
+#define VGGP_LOGDET_FIELDS    6
+#define VGGP_MAX_PROBES       65535   /* the probe index is a grid dimension of the Lanczos kernels */
+int vggp_logdet_system(vggp_plan* plan, int precond, int probe_kind, int n_probes, uint64_t seed_or_first,
+                       int max_steps, double rtol, double* out_host, double* per_probe_host, void* stream);
+#define VGGP_CT_FIELDS 5
+int vggp_collapsed_terms(vggp_plan* plan, const vggp_binned_desc* desc, const void* binned, double* out, void* stream);
 
 /* ---- feature evaluation (bit-exact restatement of the reference's basis calls) ------------------------- */
 

@@ -9,7 +9,9 @@ LIB_PATH = os.path.join(HERE, "libvggp.so")
 B1_ASVGP, B0_GRIDDED, SVGP_GRID, VFF_GRID, SVGP_MARKOV = 0, 1, 2, 3, 4
 F32, F64 = 0, 1
 MEANOPT_JACOBI, MEANOPT_KRONECKER = 0, 1
-ABI_VERSION = 4
+PROBE_RADEMACHER, PROBE_UNIT = 0, 1
+LOGDET_FIELDS, CT_FIELDS = 6, 5
+ABI_VERSION = 5
 
 WS_K, WS_P, WS_R, WS_Q, WS_S, WS_ALPHA, WS_SCAL, WS_KRAW, WS_QBAND = range(9)
 
@@ -85,6 +87,8 @@ SIGNATURES = {
     "vggp_meanopt_solve": (C.c_int, [_vp, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), C.POINTER(C.c_double), _vp]),
     "vggp_meanopt_solve_pc": (C.c_int, [_vp, C.c_int, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), C.POINTER(C.c_double),
                                         _vp]),
+    "vggp_logdet_system": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_double, _vp, _vp, _vp]),
+    "vggp_collapsed_terms": (C.c_int, [_vp, C.POINTER(BinnedDesc), _dp, _dp, _vp]),
     "vggp_covopt_update": (C.c_int, [_vp, C.c_int, _dp, C.c_double, _dp, _dp, _dp, _vp]),
     "vggp_b1_stencil": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _dp, _vp]),
     "vggp_features_dense": (C.c_int, [_vp, C.c_int, _dp, _i64, _dp, _dp, _vp]),

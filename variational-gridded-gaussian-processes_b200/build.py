@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvggp.so")
 SOURCES = ["vggp.cu"]
-HEADERS = ["common.cuh", "gemm.cuh", "grid.cuh", "obs.cuh", "obs_binned.cuh", "binplan.hpp", "metrics.cuh", "b0scan.cuh", "svgpm.cuh", "meanopt.cuh", "covopt.cuh", "minibatch.cuh", "grid_b1.cuh", "grid_b1_fast.cuh", "collective.cuh", os.path.join("..", "..", "include", "vggp.h")]
+HEADERS = ["common.cuh", "gemm.cuh", "grid.cuh", "obs.cuh", "obs_binned.cuh", "binplan.hpp", "metrics.cuh", "b0scan.cuh", "svgpm.cuh", "meanopt.cuh", "covopt.cuh", "collapsed.cuh", "minibatch.cuh", "grid_b1.cuh", "grid_b1_fast.cuh", "collective.cuh", os.path.join("..", "..", "include", "vggp.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -20,6 +20,7 @@
 #include "svgpm.cuh"
 #include "meanopt.cuh"
 #include "covopt.cuh"
+#include "collapsed.cuh"
 #include "collective.cuh"
 #include "minibatch.cuh"
 
@@ -164,6 +165,11 @@ struct vggp_plan {
     void* mo_buf = nullptr; size_t mo_bytes = 0; bool mo_assembled = false;
     // the Kronecker-preconditioned solve's z vector, Thomas factors and trace, allocated at its first call (scratch_bytes)
     void* mo_kbuf = nullptr; size_t mo_kbytes = 0;
+    bool mo_solved = false;                // a solve ran on the current assembly at the theta of the last forward
+    int64_t mo_set[3] = {0, 0, 0};         // n, n_tasks, data_elems of the binned set of the current assembly
+    // collapsed ELBO (collapsed.cuh): exact-term scratch, Lanczos vectors and coefficients; grown by vggp_logdet_system /
+    // vggp_collapsed_terms (scratch_bytes)
+    void* ct_buf = nullptr; size_t ct_bytes = 0;
     // optimal covariance (covopt.cuh): F band, U^-T recurrence, B1 X diagonals, change sums; allocated at the first
     // vggp_covopt_update (scratch_bytes)
     void* co_buf = nullptr; size_t co_bytes = 0;
@@ -2286,12 +2292,12 @@ struct MoSweepCfg {
     size_t smem;
 };
 
-MoSweepCfg mo_sweep_cfg(const vggp_plan* p, const MoKronLayout& K, int d) {
+MoSweepCfg mo_sweep_cfg(const vggp_plan* p, const MoKronLayout& K, int d, i64 nvec = 1) {
     MoSweepCfg c;
     MoSweep& w = c.w;
     w.n = p->n[d];
     w.inner = p->stride[d];
-    w.F = p->M / w.n;
+    w.F = nvec * (p->M / w.n);       // nvec vectors of M back to back: the outer index runs over them as well
     w.fac = K.fac + K.fac_off[d];
     const i64 target = (i64)p->sm_count * 1024;
     int S = 1;
@@ -2414,19 +2420,9 @@ int covopt_impl(vggp_plan* p, int dim, const void* gbuf, double ell_scale, const
     return 0;
 }
 
-constexpr int MO_BATCH = 64;        // CG iterations launched between two reads of the status record
-
-// precond: VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER (the Jacobi launches are those of the solve before the choice)
+// the assembled system at the theta of the last forward (the B1 bands are filled by k_mo_b1_bands)
 template <int D>
-int mo_solve_impl(vggp_plan* p, int precond, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
-                  cudaStream_t st) {
-    const bool kron = precond == VGGP_MEANOPT_KRONECKER;
-    if (kron && !p->mo_kbuf) {
-        const size_t want = mo_kron_layout(p).bytes;
-        VGGP_CUDA(cudaMalloc(&p->mo_kbuf, want));
-        p->mo_kbytes = want;
-    }
-    const MoLayout L = mo_layout(p);
+MoSys<D> mo_system(const vggp_plan* p, const MoLayout& L) {
     const bool b1 = p->family == VGGP_B1_ASVGP;
     MoSys<D> s;
     memset(&s, 0, sizeof(s));
@@ -2444,6 +2440,24 @@ int mo_solve_impl(vggp_plan* p, int precond, double rtol, int max_iter, double* 
     }
     s.G = L.G;
     s.theta = p->theta_dev;
+    return s;
+}
+
+constexpr int MO_BATCH = 64;        // CG iterations launched between two reads of the status record
+
+// precond: VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER (the Jacobi launches are those of the solve before the choice)
+template <int D>
+int mo_solve_impl(vggp_plan* p, int precond, double rtol, int max_iter, double* m_out, int* iters_host, double* relres_host,
+                  cudaStream_t st) {
+    const bool kron = precond == VGGP_MEANOPT_KRONECKER;
+    if (kron && !p->mo_kbuf) {
+        const size_t want = mo_kron_layout(p).bytes;
+        VGGP_CUDA(cudaMalloc(&p->mo_kbuf, want));
+        p->mo_kbytes = want;
+    }
+    const MoLayout L = mo_layout(p);
+    const bool b1 = p->family == VGGP_B1_ASVGP;
+    const MoSys<D> s = mo_system<D>(p, L);
     const unsigned blocks = (unsigned)std::min<i64>((p->M + 255) / 256, (i64)p->sm_count * 8);
     if (b1) {
         k_mo_b1_bands<<<dim3(ceil_div(p->nmax, 256), D), 256, 0, st>>>(p->g, p->theta_dev, L.band, L.band_stride);
@@ -2524,6 +2538,304 @@ int mo_solve_impl(vggp_plan* p, int precond, double rtol, int max_iter, double* 
     return 0;
 }
 
+// ---- collapsed ELBO (collapsed.cuh) ---------------------------------------------------------------------------------
+// One buffer, grown on demand: [inverse bands 4 sum M_d | d'^-1/2 sum M_d | log det F_d 4 | term partials 3 NB | diag(A)^-1/2 M |
+//                               Lanczos partials 2 k NB | alpha k S | beta k S | v0, v1, t, y: 4 k M | nsteps k | done k]
+// with NB = CT_NB_PER_SM * SMs CTAs at most per probe and S = max_steps.
+constexpr int CT_NB_PER_SM = 8;
+constexpr int CT_CHECK = 8;             // Lanczos steps launched between the first reads of the coefficients
+
+struct CtLayout {
+    double *ib, *rs, *ldf, *tpart, *sdiag, *part, *alpha, *beta, *v[4];
+    int *nsteps, *done;
+    int nb;
+    size_t bytes;
+};
+
+CtLayout ct_layout(const vggp_plan* p, void* buf, int k, int max_steps) {
+    CtLayout c;
+    c.nb = p->sm_count * CT_NB_PER_SM;
+    i64 nf = 0;
+    for (int d = 0; d < p->D; ++d) nf += 4 * (i64)p->n[d];
+    double* q = reinterpret_cast<double*>(buf);
+    c.ib = q; q += nf;
+    c.rs = q; q += nf / 4;
+    c.ldf = q; q += 4;
+    c.tpart = q; q += 3 * (i64)c.nb;
+    c.sdiag = q; q += p->M;
+    c.part = q; q += 2 * (i64)k * c.nb;
+    c.alpha = q; q += (i64)k * max_steps;
+    c.beta = q; q += (i64)k * max_steps;
+    for (int i = 0; i < 4; ++i) { c.v[i] = q; q += (i64)k * p->M; }
+    c.nsteps = reinterpret_cast<int*>(q);
+    c.done = c.nsteps + k;
+    c.bytes = (size_t)(reinterpret_cast<char*>(c.done + k) - reinterpret_cast<char*>(buf));
+    return c;
+}
+
+int ct_reserve(vggp_plan* p, int k, int max_steps, cudaStream_t st) {
+    const size_t want = ct_layout(p, nullptr, k, max_steps).bytes;
+    if (p->ct_buf && p->ct_bytes >= want) return 0;
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusActive)
+        return fail(VGGP_E_UNSUPPORTED, "the collapsed-ELBO scratch grows here: call it outside a stream capture");
+    if (p->ct_buf) {
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        VGGP_CUDA(cudaFree(p->ct_buf));
+        p->ct_buf = nullptr;
+        p->ct_bytes = 0;
+    }
+    VGGP_CUDA(cudaMalloc(&p->ct_buf, want));
+    p->ct_bytes = want;
+    return 0;
+}
+
+// Eigenvalues theta_i of the symmetric tridiagonal (a [n], b [n - 1]) and the squared first components tau_i^2 of its
+// eigenvectors, by the implicit QL method with Wilkinson shifts (Golub-Welsch: only the first row of the eigenvector matrix
+// is carried).  Returns sum_i tau_i^2 log theta_i, NaN if an eigenvalue is not positive or the iteration does not settle.
+double ct_gauss_log(int n, const double* a, const double* b, std::vector<double>& d, std::vector<double>& e,
+                    std::vector<double>& z) {
+    d.assign(a, a + n);
+    e.assign(n, 0.0);
+    for (int i = 0; i + 1 < n; ++i) e[i] = b[i];
+    z.assign(n, 0.0);
+    z[0] = 1.0;
+    for (int l = 0; l < n; ++l) {
+        int iter = 0, m;
+        do {
+            for (m = l; m < n - 1; ++m) {
+                const double dd = fabs(d[m]) + fabs(d[m + 1]);
+                if (fabs(e[m]) <= 1e-16 * dd) break;
+            }
+            if (m != l) {
+                if (iter++ == 100) return NAN;
+                double g = (d[l + 1] - d[l]) / (2.0 * e[l]);
+                double r = hypot(g, 1.0);
+                g = d[m] - d[l] + e[l] / (g + copysign(r, g));
+                double sn = 1.0, c = 1.0, pp = 0.0;
+                int i;
+                for (i = m - 1; i >= l; --i) {
+                    double f = sn * e[i];
+                    const double bb = c * e[i];
+                    r = hypot(f, g);
+                    e[i + 1] = r;
+                    if (r == 0.0) {
+                        d[i + 1] -= pp;
+                        e[m] = 0.0;
+                        break;
+                    }
+                    sn = f / r;
+                    c = g / r;
+                    g = d[i + 1] - pp;
+                    r = (d[i] - g) * sn + 2.0 * c * bb;
+                    pp = sn * r;
+                    d[i + 1] = g + pp;
+                    g = c * r - bb;
+                    f = z[i + 1];
+                    z[i + 1] = sn * z[i] + c * f;
+                    z[i] = c * z[i] - sn * f;
+                }
+                if (r == 0.0 && i >= l) continue;
+                d[l] -= pp;
+                e[l] = g;
+                e[m] = 0.0;
+            }
+        } while (m != l);
+    }
+    double acc = 0.0;
+    for (int i = 0; i < n; ++i) {
+        if (!(d[i] > 0.0)) return NAN;
+        acc += z[i] * z[i] * log(d[i]);
+    }
+    return acc;
+}
+
+template <int D>
+int ct_logdet_impl(vggp_plan* p, int precond, int kind, int k, uint64_t seed, int max_steps, double rtol, double* out,
+                   double* per_probe, cudaStream_t st) {
+    const bool kron = precond == VGGP_MEANOPT_KRONECKER;
+    if (kron && !p->mo_kbuf) {
+        const size_t want = mo_kron_layout(p).bytes;
+        VGGP_CUDA(cudaMalloc(&p->mo_kbuf, want));
+        p->mo_kbytes = want;
+    }
+    if (int rc = ct_reserve(p, k, max_steps, st)) return rc;
+    const CtLayout c = ct_layout(p, p->ct_buf, k, max_steps);
+    const MoLayout L = mo_layout(p);
+    const MoSys<D> s = mo_system<D>(p, L);
+    const i64 M = p->M;
+    const unsigned nb = (unsigned)std::min<i64>((M + CT_THREADS - 1) / CT_THREADS, (i64)c.nb);
+    if (p->family == VGGP_B1_ASVGP) {
+        k_mo_b1_bands<<<dim3(ceil_div(p->nmax, 256), D), 256, 0, st>>>(p->g, p->theta_dev, L.band, L.band_stride);
+        VGGP_LAUNCH_CHECK();
+    }
+    // preconditioner and log det P
+    double logdet_p = 0.0;
+    MoKronLayout K{};
+    if (kron) {
+        K = mo_kron_layout(p);
+        MoFacOff<D> fo;
+        for (int d = 0; d < D; ++d) fo.off[d] = K.fac_off[d];
+        k_ct_gtrace<<<nb, CT_THREADS, 0, st>>>(M, L.G, c.tpart);
+        VGGP_LAUNCH_CHECK();
+        k_ct_gtrace_final<<<1, CT_THREADS, 0, st>>>(c.tpart, (int)nb, K.k);
+        VGGP_LAUNCH_CHECK();
+        k_mo_kron_factors<D><<<1, 32, 0, st>>>(s, K.k, K.fac, fo);
+        VGGP_LAUNCH_CHECK();
+        k_ct_rsqrt_pivots<D><<<dim3(ceil_div(p->nmax, CT_THREADS), D), CT_THREADS, 0, st>>>(s, K.fac, fo, c.rs);
+        VGGP_LAUNCH_CHECK();
+        i64 nf = 0;
+        for (int d = 0; d < D; ++d) nf += 3 * (i64)p->n[d];
+        std::vector<double> fac((size_t)nf);
+        VGGP_CUDA(cudaMemcpyAsync(fac.data(), K.fac, sizeof(double) * (size_t)nf, cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        for (int d = 0; d < D; ++d) {
+            double ld = 0.0;
+            for (int i = 0; i < p->n[d]; ++i) ld -= log(fac[(size_t)K.fac_off[d] + p->n[d] + i]);
+            logdet_p += ((double)M / (double)p->n[d]) * ld;
+        }
+    } else {
+        k_ct_jacobi<D><<<nb, CT_THREADS, 0, st>>>(s, c.sdiag, c.tpart);
+        VGGP_LAUNCH_CHECK();
+        std::vector<double> part(nb);
+        VGGP_CUDA(cudaMemcpyAsync(part.data(), c.tpart, sizeof(double) * nb, cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        for (unsigned i = 0; i < nb; ++i) logdet_p += part[i];
+    }
+    // Lanczos on B = C^-1 A C^-T from the probes
+    CtLanczos z;
+    z.M = M; z.k = k; z.max_steps = max_steps;
+    z.alpha = c.alpha; z.beta = c.beta; z.nsteps = c.nsteps; z.done = c.done; z.part = c.part; z.nb = (int)nb;
+    VGGP_CUDA(cudaMemsetAsync(c.nsteps, 0, sizeof(int) * 2 * (size_t)k, st));
+    double *v0 = c.v[0], *v1 = c.v[1], *y = c.v[3], *t = c.v[2];
+    k_ct_probe_init<<<dim3(nb, k), CT_THREADS, 0, st>>>(M, kind, seed, v0, v1);
+    VGGP_LAUNCH_CHECK();
+    const unsigned sb = (unsigned)std::min<i64>((M + CT_THREADS - 1) / CT_THREADS, (i64)p->sm_count * 8);
+    auto apply = [&](const double* in, double* outv) -> int {
+        if (!kron) {
+            k_ct_stencil<D, true><<<sb, CT_THREADS, 0, st>>>(s, k, in, outv, c.sdiag, c.done);
+            VGGP_LAUNCH_CHECK();
+            return 0;
+        }
+        auto sweep = [&](int d, bool fwd, const double* src, double* dst) -> int {
+            const MoSweepCfg cf = mo_sweep_cfg(p, K, d, k);
+            const double* rs = c.rs + K.fac_off[d] / 3;
+            if (d == D - 1) {
+                if (fwd) k_ct_kron_half<true, true><<<cf.blocks, cf.threads, cf.smem, st>>>(cf.w, M, rs, src, dst, c.done);
+                else k_ct_kron_half<false, true><<<cf.blocks, cf.threads, cf.smem, st>>>(cf.w, M, rs, src, dst, c.done);
+            } else {
+                if (fwd) k_ct_kron_half<true, false><<<cf.blocks, cf.threads, 0, st>>>(cf.w, M, rs, src, dst, c.done);
+                else k_ct_kron_half<false, false><<<cf.blocks, cf.threads, 0, st>>>(cf.w, M, rs, src, dst, c.done);
+            }
+            VGGP_LAUNCH_CHECK();
+            return 0;
+        };
+        for (int d = D - 1; d >= 0; --d)            // t = C^-T in
+            if (int rc = sweep(d, false, d == D - 1 ? in : t, t)) return rc;
+        k_ct_stencil<D, false><<<sb, CT_THREADS, 0, st>>>(s, k, t, outv, nullptr, c.done);
+        VGGP_LAUNCH_CHECK();
+        for (int d = 0; d < D; ++d)                 // out = C^-1 A t
+            if (int rc = sweep(d, true, outv, outv)) return rc;
+        return 0;
+    };
+    std::vector<double> ha((size_t)k * max_steps), hb((size_t)k * max_steps), q(k, NAN), qprev(k, NAN);
+    std::vector<int> hn(2 * (size_t)k), conv(k, 0), fin(k, 0);
+    std::vector<double> wd, we, wz;
+    const double norm2 = kind == 0 ? (double)M : 1.0;
+    int step = 0;
+    while (step < max_steps) {
+        // checks every 8 steps up to 128, then every step / 8 rounded down to a multiple of 8: the host quadrature of a
+        // probe costs O(steps^2), so the checks stay a small share of long runs
+        const int nsb = std::min(CT_CHECK * std::max(1, step / (8 * CT_CHECK)), max_steps - step);
+        for (int i = 0; i < nsb; ++i, ++step) {
+            if (int rc = apply(v1, y)) return rc;
+            k_ct_dot<<<dim3(nb, k), CT_THREADS, 0, st>>>(z, y, v1);
+            VGGP_LAUNCH_CHECK();
+            k_ct_alpha<<<k, CT_THREADS, 0, st>>>(z, step);
+            VGGP_LAUNCH_CHECK();
+            k_ct_update<<<dim3(nb, k), CT_THREADS, 0, st>>>(z, step, y, v1, v0);
+            VGGP_LAUNCH_CHECK();
+            k_ct_beta<<<k, CT_THREADS, 0, st>>>(z, step);
+            VGGP_LAUNCH_CHECK();
+            k_ct_next<<<dim3(nb, k), CT_THREADS, 0, st>>>(z, step, y);
+            VGGP_LAUNCH_CHECK();
+            double* old = v0;
+            v0 = v1; v1 = y; y = old;
+        }
+        VGGP_CUDA(cudaMemcpyAsync(ha.data(), c.alpha, sizeof(double) * ha.size(), cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaMemcpyAsync(hb.data(), c.beta, sizeof(double) * hb.size(), cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaMemcpyAsync(hn.data(), c.nsteps, sizeof(int) * hn.size(), cudaMemcpyDeviceToHost, st));
+        VGGP_CUDA(cudaStreamSynchronize(st));
+        // a probe converges once its quadrature moves by <= rtol (relative) from one check to the next, or when its Krylov
+        // space is exhausted; the host then marks it done for the kernels.  done = 3 (step limit) ends it unconverged.
+        bool all = true, changed = false;
+        for (int j = 0; j < k; ++j) {
+            int& dn = hn[(size_t)k + j];
+            if (fin[j]) continue;
+            qprev[j] = q[j];
+            q[j] = norm2 * ct_gauss_log(hn[j], ha.data() + (size_t)j * max_steps, hb.data() + (size_t)j * max_steps, wd, we, wz);
+            conv[j] = dn == 2 || fabs(q[j] - qprev[j]) <= rtol * fabs(q[j]);
+            if (conv[j] && dn == 0) { dn = 1; changed = true; }
+            fin[j] = conv[j] || dn != 0;
+            all = all && fin[j];
+        }
+        if (all) break;
+        if (changed) VGGP_CUDA(cudaMemcpyAsync(c.done, hn.data() + k, sizeof(int) * (size_t)k, cudaMemcpyHostToDevice, st));
+    }
+    VGGP_CUDA(cudaStreamSynchronize(st));
+    double sum = 0.0, sq = 0.0;
+    int steps = 0, nconv = 0;
+    for (int j = 0; j < k; ++j) {
+        sum += q[j];
+        steps = std::max(steps, hn[j]);
+        nconv += conv[j];
+        if (per_probe) per_probe[j] = q[j];
+    }
+    const double mean = sum / k;
+    for (int j = 0; j < k; ++j) sq += (q[j] - mean) * (q[j] - mean);
+    out[0] = logdet_p + (kind == 0 ? mean : sum);
+    out[1] = kind == 0 && k > 1 ? sqrt(sq / (k - 1) / k) : 0.0;
+    out[2] = logdet_p;
+    out[3] = steps;
+    out[4] = nconv;
+    out[5] = k;
+    return 0;
+}
+
+template <typename T, int D>
+int ct_terms_impl(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, double* out, cudaStream_t st) {
+    if (int rc = ct_reserve(p, 0, 0, st)) return rc;
+    const CtLayout c = ct_layout(p, p->ct_buf, 0, 0);
+    const MoLayout L = mo_layout(p);
+    const MoSys<D> s = mo_system<D>(p, L);
+    if (p->family == VGGP_B1_ASVGP) {
+        k_mo_b1_bands<<<dim3(ceil_div(p->nmax, 256), D), 256, 0, st>>>(p->g, p->theta_dev, L.band, L.band_stride);
+        VGGP_LAUNCH_CHECK();
+    }
+    k_ct_inv_bands<D><<<1, 32, 0, st>>>(s, c.ib, c.ldf);
+    VGGP_LAUNCH_CHECK();
+    CtTermArgs a;
+    a.data = reinterpret_cast<const unsigned char*>(binned) + desc->off_data;
+    a.elems = desc->n_tasks > 0 ? desc->data_elems : 0;
+    a.b = L.b;
+    a.x = L.x;
+    a.ib = c.ib;
+    a.part = c.tpart;
+    const i64 work = std::max<i64>(p->M, a.elems / (D + 1));
+    const unsigned nb = (unsigned)std::max<i64>(1, std::min<i64>((work + CT_THREADS - 1) / CT_THREADS, (i64)c.nb));
+    k_ct_terms<T, D><<<nb, CT_THREADS, 0, st>>>(s, a);
+    VGGP_LAUNCH_CHECK();
+    const double* outside = desc->n_inside < desc->n ? reinterpret_cast<const double*>(binned) : nullptr;
+    k_ct_terms_final<D><<<1, CT_THREADS, 0, st>>>(s, c.tpart, (int)nb, c.ldf, (double)desc->n, outside,
+                                                  p->family == VGGP_SVGP_MARKOV ? 1 : 0, out);
+    VGGP_LAUNCH_CHECK();
+    return 0;
+}
+int ct_terms_dispatch(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, double* out, cudaStream_t st) {
+    VGGP_DISPATCH_TD(p, ct_terms_impl, p, desc, binned, out, st);
+}
+
+
 extern "C" {
 
 int vggp_abi_version(void) { return VGGP_ABI_VERSION; }
@@ -2548,7 +2860,7 @@ int vggp_workspace_bytes(const vggp_plan* p, int64_t* plan_bytes, int64_t* gbuf_
     if (gbuf_bytes) *gbuf_bytes = total;
     if (scratch_bytes) {
         const size_t tsz = p->obs_dtype == VGGP_F32 ? 4 : 8;
-        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes + p->mo_kbytes + p->co_bytes;
+        size_t sc = p->det_bytes + p->det_fp_elems * sizeof(double) + (size_t)p->pk_cap * tsz * (p->D + 1) + (size_t)p->b0s_raw_bytes + p->mo_bytes + p->mo_kbytes + p->co_bytes + p->ct_bytes;
         if (p->st_x) sc += (size_t)p->st_n * tsz * (p->D + 1) + sizeof(double) * (2 * (size_t)p->M + 2 * (size_t)p->Lsize) + (size_t)total;
         *scratch_bytes = (int64_t)sc;
     }
@@ -2786,6 +3098,7 @@ int vggp_plan_destroy(vggp_plan* p) {
     if (p->det_fp) cudaFree(p->det_fp);
     if (p->mo_buf) cudaFree(p->mo_buf);
     if (p->mo_kbuf) cudaFree(p->mo_kbuf);
+    if (p->ct_buf) cudaFree(p->ct_buf);
     if (p->co_buf) cudaFree(p->co_buf);
     for (auto& e : p->k1_ev) cudaEventDestroy(e);
     for (auto& e : p->k1_gev) if (e) cudaEventDestroy(e);
@@ -2828,6 +3141,7 @@ int vggp_grid_forward(vggp_plan* p, const double* theta, const double* m, const 
     int rc;
     p->last_stream = st;
     p->forwarded = true;
+    p->mo_solved = false;                   // a new theta: the iterate of the last optimal-mean solve no longer belongs to it
     if (p->family == VGGP_SVGP_MARKOV) return svgpm_forward(p, theta, m, L, st);
     if (p->family == VGGP_B1_ASVGP) return b1f_forward(p, theta, m, L, st);
     VGGP_CUDA(cudaMemcpyAsync(p->mws, m, sizeof(double) * p->M, cudaMemcpyDeviceToDevice, st));
@@ -3394,7 +3708,9 @@ int vggp_meanopt_assemble(vggp_plan* p, const vggp_binned_desc* desc, const void
         p->mo_bytes = want;
     }
     p->mo_assembled = false;
+    p->mo_solved = false;
     if (int rc = mo_assemble_dispatch(p, desc, binned, st)) return rc;
+    p->mo_set[0] = desc->n; p->mo_set[1] = desc->n_tasks; p->mo_set[2] = desc->data_elems;
     p->mo_assembled = true;
     return 0;
 }
@@ -3415,11 +3731,53 @@ int vggp_meanopt_solve_pc(vggp_plan* p, int precond, double rtol, int max_iter, 
         return fail(VGGP_E_ARG, "precond must be VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER");
     if (!p->mo_assembled) return fail(VGGP_E_ARG, "vggp_meanopt_solve needs a previous vggp_meanopt_assemble on this plan");
     cudaStream_t st = (cudaStream_t)stream;
+    int rc;
     switch (p->D) {
-        case 1: return mo_solve_impl<1>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
-        case 2: return mo_solve_impl<2>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
-        default: return mo_solve_impl<3>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st);
+        case 1: rc = mo_solve_impl<1>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st); break;
+        case 2: rc = mo_solve_impl<2>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st); break;
+        default: rc = mo_solve_impl<3>(p, precond, rtol, max_iter, m_out, iters_host, relres_host, st); break;
     }
+    p->mo_solved = rc == 0;
+    return rc;
+}
+
+int vggp_logdet_system(vggp_plan* p, int precond, int probe_kind, int n_probes, uint64_t seed_or_first, int max_steps,
+                       double rtol, double* out_host, double* per_probe_host, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !out_host) return fail(VGGP_E_ARG, "null argument");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the collapsed ELBO is built for the B1 and VGGP_SVGP_MARKOV families (3^D-stencil system)");
+    if (precond != VGGP_MEANOPT_JACOBI && precond != VGGP_MEANOPT_KRONECKER)
+        return fail(VGGP_E_ARG, "precond must be VGGP_MEANOPT_JACOBI or VGGP_MEANOPT_KRONECKER");
+    if (probe_kind != VGGP_PROBE_RADEMACHER && probe_kind != VGGP_PROBE_UNIT)
+        return fail(VGGP_E_ARG, "probe_kind must be VGGP_PROBE_RADEMACHER or VGGP_PROBE_UNIT");
+    if (n_probes < 1 || n_probes > VGGP_MAX_PROBES || max_steps < 1 || !(rtol >= 0.0))
+        return fail(VGGP_E_ARG, "1 <= n_probes <= VGGP_MAX_PROBES, max_steps >= 1 and rtol >= 0");
+    if (probe_kind == VGGP_PROBE_UNIT && (seed_or_first >= (uint64_t)p->M || (uint64_t)n_probes > (uint64_t)p->M - seed_or_first))
+        return fail(VGGP_E_ARG, "unit probes e_first .. e_{first + n_probes - 1} must lie below M");
+    if (!p->mo_assembled) return fail(VGGP_E_ARG, "vggp_logdet_system needs a previous vggp_meanopt_assemble on this plan");
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (p->D) {
+        case 1: return ct_logdet_impl<1>(p, precond, probe_kind, n_probes, seed_or_first, max_steps, rtol, out_host, per_probe_host, st);
+        case 2: return ct_logdet_impl<2>(p, precond, probe_kind, n_probes, seed_or_first, max_steps, rtol, out_host, per_probe_host, st);
+        default: return ct_logdet_impl<3>(p, precond, probe_kind, n_probes, seed_or_first, max_steps, rtol, out_host, per_probe_host, st);
+    }
+}
+
+int vggp_collapsed_terms(vggp_plan* p, const vggp_binned_desc* desc, const void* binned, double* out, void* stream) {
+    DeviceGuard dev_guard(p ? p->device : -1);
+    if (!p || !desc || !out) return fail(VGGP_E_ARG, "null argument");
+    if (p->family != VGGP_B1_ASVGP && p->family != VGGP_SVGP_MARKOV)
+        return fail(VGGP_E_UNSUPPORTED, "the collapsed ELBO is built for the B1 and VGGP_SVGP_MARKOV families (3^D-stencil system)");
+    if (desc->D != p->D || desc->n_tasks < 0 || (desc->n_tasks > 0 && !binned) || (desc->n_inside < desc->n && !binned))
+        return fail(VGGP_E_ARG, "binned buffer does not match the plan");
+    if (!p->mo_assembled) return fail(VGGP_E_ARG, "vggp_collapsed_terms needs a previous vggp_meanopt_assemble on this plan");
+    if (!p->mo_solved)
+        return fail(VGGP_E_ARG, "vggp_collapsed_terms needs a vggp_meanopt_solve on the current assembly after the last "
+                                "vggp_grid_forward");
+    if (desc->n != p->mo_set[0] || desc->n_tasks != p->mo_set[1] || desc->data_elems != p->mo_set[2])
+        return fail(VGGP_E_ARG, "vggp_collapsed_terms takes the binned set given to vggp_meanopt_assemble");
+    return ct_terms_dispatch(p, desc, binned, out, (cudaStream_t)stream);
 }
 
 int vggp_covopt_update(vggp_plan* p, int dim, const void* gbuf, double ell_scale, const double* L, double* L_out,

@@ -169,6 +169,40 @@ class GridPlan:
                                                   _stream_ptr(self.device)))
         return m, int(it.value), float(rr.value)
 
+    PROBES = {"rademacher": _lib.PROBE_RADEMACHER, "unit": _lib.PROBE_UNIT}
+
+    def logdet_system(self, n_probes: int, seed: int = 0, preconditioner: str = "kronecker", probes: str = "rademacher",
+                      max_steps: int = 1000, rtol: float = 1e-6, per_probe: bool = False) -> dict:
+        """log det of the assembled optimal-mean system A by preconditioned stochastic Lanczos quadrature
+        (vggp_logdet_system; synchronises).  `probes`: "rademacher" (signs hashed from `seed`) or "unit" (e_seed ..
+        e_{seed + n_probes - 1}: with seed = 0 and n_probes = M the exact value).  Returns {"logdet", "stderr", "logdet_p",
+        "steps", "converged", "probes"} and, with per_probe, the per-probe values (float64 CPU tensor)."""
+        if preconditioner not in self.MEANOPT_PRECONDITIONERS:
+            raise ValueError(f"preconditioner must be one of {sorted(self.MEANOPT_PRECONDITIONERS)}, not {preconditioner!r}")
+        if probes not in self.PROBES:
+            raise ValueError(f"probes must be one of {sorted(self.PROBES)}, not {probes!r}")
+        out = (C.c_double * _lib.LOGDET_FIELDS)()
+        pp = (C.c_double * int(n_probes))() if per_probe and n_probes > 0 else None
+        _lib.check(self.lib.vggp_logdet_system(self.handle, self.MEANOPT_PRECONDITIONERS[preconditioner], self.PROBES[probes],
+                                               int(n_probes), int(seed), int(max_steps), float(rtol), C.cast(out, C.c_void_p),
+                                               C.cast(pp, C.c_void_p) if pp is not None else None,
+                                               _stream_ptr(self.device)))
+        res = {"logdet": out[0], "stderr": out[1], "logdet_p": out[2], "steps": int(out[3]), "converged": int(out[4]),
+               "probes": int(out[5])}
+        if pp is not None:
+            res["per_probe"] = torch.tensor(pp[:], dtype=torch.float64)
+        return res
+
+    def collapsed_terms(self, binned: "BinnedObs") -> torch.Tensor:
+        """{N, sum y^2, b^T x*, tr(F^-1 G), log det Kuu} (float64 device tensor; vggp_collapsed_terms, asynchronous) of the
+        assembled and solved optimal-mean system; `binned` is the set given to meanopt_assemble."""
+        if not isinstance(binned, BinnedObs):
+            raise TypeError("collapsed_terms takes the BinnedObs of GridPlan.bin")
+        out = torch.empty(_lib.CT_FIELDS, dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.vggp_collapsed_terms(self.handle, C.byref(binned.desc), binned.buf.data_ptr(), out.data_ptr(),
+                                                 _stream_ptr(self.device)))
+        return out
+
     def covopt_update(self, dim: int, gbuf: torch.Tensor, ell_scale: float, L: torch.Tensor, change: torch.Tensor):
         """One coordinate update of the optimal Kronecker-factored covariance (vggp_covopt_update; B1 and SVGP_MARKOV):
         block `dim` of the float64 factors `L` (the L of the last grid_forward) is overwritten in place with the Cholesky
